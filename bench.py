@@ -48,6 +48,7 @@ NCU_SEEDVAR_DRAM_BYTES_PER_READ = (222.070016e6 + 21.044992e6) / 746917
 # k_seed (config 2 runs one level of it), per read of its input (same capture: 2 155 000 reads left by the
 # prefilter; 497.53 MB read + 37.23 MB written)
 NCU_SEED_DRAM_BYTES_PER_READ = (497.526784e6 + 37.233920e6) / 2155000
+DUMP_SAMPLE = 1_000_000      # reads whose results --dump-outputs writes: 5 x 4 MB of float32 + 8 MB of indices
 
 
 def make_config():
@@ -165,6 +166,19 @@ def bind_to_gpu_numa_node(local: int):
         return f"node {node} ({len(cpus)} cpus)"
     except Exception as exc:
         return f"unavailable ({type(exc).__name__})"
+
+
+def dump_outputs(out_dir, res):
+    """Writes the per-read results `res` (bdx_result records) as <out_dir>/<field>.npy in float32 (every field is a
+    small integer, exact in float32) for a fixed, seeded sample of DUMP_SAMPLE reads, and <out_dir>/read_index.npy
+    (float64) with the indices of those reads.  The reads come from a seeded generator, so two builds run with the
+    same arguments can be compared file for file."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(res)
+    idx = np.arange(n) if n <= DUMP_SAMPLE else np.sort(np.random.default_rng(SEED).choice(n, DUMP_SAMPLE, replace=False))
+    np.save(os.path.join(out_dir, "read_index.npy"), idx.astype(np.float64))
+    for f in res.dtype.names:
+        np.save(os.path.join(out_dir, f"{f}.npy"), res[f][idx].astype(np.float32))
 
 
 def oracle_rate(cfg, blob, off64, threads):
@@ -426,6 +440,8 @@ def run_ours(args):
     # ---- sanity on the timed results (parity proper lives in tests/) -----------------------
     res = np.frombuffer(d_res.cpu().numpy().tobytes(), dtype=bdx.RESULT_DTYPE)
     matched = int((res["status"] == 0).sum())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res)
 
     if args.no_e2e:
         if rank == 0:
@@ -583,13 +599,12 @@ def run_ours(args):
             for dv in devs:
                 torch.cuda.synchronize(dv)
             t0 = time.perf_counter()
-            steps_pool = max(args.steps, 2 * world)
-            m = pool_pass(steps_pool)
+            m = pool_pass(args.steps)
             for dv in devs:
                 torch.cuda.synchronize(dv)
             dtp = time.perf_counter() - t0
-            assert m == steps_pool * int((res["status"][:nb * B] == 0).sum())
-            pool_line = {"n_gpus": world, "reads_per_sec": steps_pool * nb * B / dtp, "streams_per_device": 2,
+            assert m == args.steps * int((res["status"][:nb * B] == 0).sum())
+            pool_line = {"n_gpus": world, "reads_per_sec": args.steps * nb * B / dtp, "streams_per_device": 2,
                          "batches_in_flight": cap, "api": "bdx_pool_submit_pinned / bdx_pool_fetch_view, ONE host process and "
                          "thread, one pinned copy of the workload on rank 0's NUMA node"}
             pool.close()
@@ -636,17 +651,18 @@ def run_ours(args):
         stream.sync()
         f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         f0.record(ext)
-        for _ in range(3):
+        for _ in range(args.steps):
             stream.classify_device(d_seq.data_ptr(), d_off.data_ptr(), nf, d_res.data_ptr())
         f1.record(ext)
         stream.sync()
-        tf = torch.tensor([f0.elapsed_time(f1) / 3], dtype=torch.float64, device="cuda")
+        tf = torch.tensor([f0.elapsed_time(f1) / args.steps], dtype=torch.float64, device="cuda")
         if world > 1:
             dist.all_reduce(tf, op=dist.ReduceOp.MAX)
         floor = {"reads_per_sec": world * nf / (float(tf.item()) * 1e-3), "reads_per_gpu": nf,
                  "workload": "config2 reads with plant_permille = 0: no read carries a barcode, all of them run the "
                              "full-range automaton (the rate when nothing can be short-cut)"}
-    # ---- BASELINE.json configs 3, 4, 5 at their stated sizes (device-resident, sharded over the ranks) ----
+    # ---- BASELINE.json configs 3, 4, 5 at their stated sizes (device-resident, sharded over the ranks).  Each is timed
+    # as one pass over its stated read count (the whole job is the unit those configs are quoted in), not per --steps ----
     others = None
     if not args.no_configs:
         import bench_configs
@@ -804,7 +820,14 @@ def main():
     ap.add_argument("--config-scale", type=float, default=1.0, help="fraction of the stated read counts (1.0 = 50 M / 50 M / 200 M)")
     ap.add_argument("--parity-seconds", type=float, default=15.0, help="oracle time per config for the parity sample")
     ap.add_argument("--parity-reads", type=int, default=0, help="parity sample size per config (0 = by --parity-seconds)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the CUDA path's per-read results of the last timed step (rank 0's reads; a seeded "
+                         f"sample of {DUMP_SAMPLE} of them) to DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path's results; it does not apply to --impl reference")
     if args.reads % args.e2e_batch:
         args.e2e_batch = args.reads
     if args.impl == "reference":
