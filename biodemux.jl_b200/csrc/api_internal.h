@@ -64,8 +64,30 @@ struct HostSet {
     HostSeedVar sv[2];
 };
 
+// ---- the kernel sequence of a pass (plan.cu) ----
+enum { kStepHammingScan, kStepPrefilter, kStepSeed, kStepSeedVar, kStepSeedDeep, kStepFilter, kStepMarkPending,
+       kStepLiteral };
+enum { kWlNone, kWlWork, kWlWork2 };   // no worklist (every read of the batch), Scratch::worklist, Scratch::worklist2
+// k_literal's reads: all of them over every barcode, those with candidates, Scratch::wl_win, ::wl_full, a worklist
+enum { kLitAll, kLitCand, kLitWin, kLitFull, kLitRest };
+// one launch: kernel (kStep*), k_seed / k_seed_var level, the worklists (kWl*) it takes its reads from and appends the
+// reads it leaves open to, k_literal's reads (kLit*; kLitRest: those of worklist `in`), profiling stage (kSt*)
+struct PlanStep {
+    uint8_t kind, level, in, out, reads, stage;
+};
+struct PassPlan {
+    bool clear_lit = false;   // zero the lengths of k_literal's two read lists before the first step
+    int n = 0;
+    PlanStep step[8];
+};
+// What runs for `pass` of a config, from its parameters alone: the table sizes in P already reflect the device's
+// shared-memory limit (bdx_api.cu).  Made once per config and device; bdx_enqueue_classify walks it.
+PassPlan plan_pass(const DevParams &P, int pass);
+std::string plan_text(const PassPlan &plan);   // "k_prefilter,k_seed@1,...": the steps for bdx_config_describe
+
 struct DeviceTables {
     DevParams P;
+    PassPlan plan[2];
     std::vector<void *> allocs;
     int sm_count = 0;
 };

@@ -15,11 +15,6 @@
 
 using namespace bdx;
 
-namespace bdx {
-size_t filter_smem_bytes_for(const DevSet &S);
-size_t prefilter_smem_bytes_for(const DevSet &S);
-}
-
 // ---------------------------------------------------------------------------
 // errors
 // ---------------------------------------------------------------------------
@@ -112,7 +107,6 @@ extern "C" int bdx_config_create_debug(const bdx_params *p, uint32_t debug, bdx_
     P.algo = p->algorithm;
     P.is_dual = p->is_dual ? 1 : 0;
     P.want_stats = p->want_stats ? 1 : 0;
-    P.filter_ok = cfg->set[0].use_filter && (!p->is_dual || cfg->set[1].use_filter);
     P.two = 2;
     P.debug = (int)debug;
     P.unit_costs = p->match == 0 && p->mismatch == 1 && p->indel == 1 && (!p->has_nindel || p->nindel == 1);
@@ -179,25 +173,26 @@ static cudaError_t upload(DeviceTables *t, const std::vector<T> &v, const T **ou
     return e;
 }
 
-static int get_tables(bdx_config *cfg, int device, DeviceTables **out)
+// sharedMemPerBlockOptin of sm_100 (227 KB); the library runs on no other architecture
+constexpr size_t kSm100SmemOptin = 232448;
+
+// A config's device parameter block without the table pointers, with the stages whose shared memory would exceed
+// `smem_optin` switched off: what plan_pass decides by, on a device (get_tables) or for sm_100 (bdx_config_describe).
+static DevParams host_params(const bdx_config &cfg, size_t smem_optin)
 {
-    std::lock_guard<std::mutex> lk(cfg->mu);
-    auto it = cfg->per_device.find(device);
-    if (it != cfg->per_device.end()) {
-        *out = it->second;
-        return BDX_OK;
-    }
-    CU(cudaSetDevice(device));
-    cudaDeviceProp prop;
-    CU(cudaGetDeviceProperties(&prop, device));
-    if (prop.major < 10)
-        return fail(BDX_ERR_CUDA, "libbdx is built for sm_100a only; device compute capability too low");
-    DeviceTables *t = new DeviceTables();
-    t->P = cfg->base;
-    t->sm_count = prop.multiProcessorCount;
-    for (int s = 0; s < (cfg->base.is_dual ? 2 : 1); s++) {
-        HostSet &hs = cfg->set[s];
-        DevSet &D = t->P.set[s];
+    DevParams P = cfg.base;
+    auto level = [](const HostSet::HostSeedLevel &H, SeedLevel &L) {
+        L.k = H.k;
+        L.q = H.q;
+        L.pow = H.pow;
+        L.log2 = H.log2;
+        L.bm_log2 = H.bm_log2;
+        L.max_hits = H.max_hits;
+        L.n_entries = (int)H.entries.size();
+    };
+    for (int s = 0; s < (P.is_dual ? 2 : 1); s++) {
+        const HostSet &hs = cfg.set[s];
+        DevSet &D = P.set[s];
         D.n_bc = hs.n_bc;
         D.n_bc_pad = hs.n_bc_pad;
         D.max_m = hs.max_m;
@@ -208,57 +203,17 @@ static int get_tables(bdx_config *cfg, int device, DeviceTables **out)
         D.rs = hs.rs;
         D.bs = hs.bs;
         D.be = hs.be;
-        std::vector<uint8_t> cls(hs.class_of, hs.class_of + 256);
-        cudaError_t e = upload(t, hs.bytes, &D.bc_bytes);
-        if (e == cudaSuccess) e = upload(t, hs.off, &D.bc_off);
-        if (e == cudaSuccess) e = upload(t, hs.norm, &D.norm);
-        if (e == cudaSuccess) e = upload(t, hs.peq, &D.peq);
-        if (e == cudaSuccess) e = upload(t, hs.filt_allowed, &D.filt_allowed);
-        if (e == cudaSuccess) e = upload(t, hs.allowed0, &D.allowed0);
-        if (e == cudaSuccess) e = upload(t, cls, &D.class_of);
         D.pf_enabled = hs.pf_enabled;
         D.pf_seed = hs.pf_seed;
         D.pf_pow = hs.pf_pow;
         D.pf_log2 = hs.pf_log2;
         D.pf_bm_log2 = hs.pf_bm_log2;
-        if (e == cudaSuccess) e = upload(t, hs.pf_bitmap, &D.pf_bitmap);
-        if (e == cudaSuccess) e = upload(t, hs.pf_keys, &D.pf_keys);
-        if (e == cudaSuccess) e = upload(t, hs.pf_vals, &D.pf_vals);
-        if (e == cudaSuccess) e = upload(t, hs.bc_cls, &D.bc_cls);
         D.sd_levels = hs.sd_levels;
         D.sd_m = hs.sd_m;
-        for (int l = 0; l < hs.sd_levels; l++) {
-            const HostSet::HostSeedLevel &H = hs.sd[l];
-            SeedLevel &L = D.sd[l];
-            L.k = H.k;
-            L.q = H.q;
-            L.pow = H.pow;
-            L.log2 = H.log2;
-            L.bm_log2 = H.bm_log2;
-            L.max_hits = H.max_hits;
-            L.n_entries = (int)H.entries.size();
-            if (e == cudaSuccess) e = upload(t, H.bstart, &L.bstart);
-            if (e == cudaSuccess) e = upload(t, H.entries, &L.entries);
-            if (e == cudaSuccess) e = upload(t, H.ekeys, &L.ekeys);
-            if (e == cudaSuccess) e = upload(t, H.bitmap, &L.bitmap);
-        }
+        for (int l = 0; l < hs.sd_levels; l++) level(hs.sd[l], D.sd[l]);
         D.sdd_n = hs.sdd_n;
         D.sdd_k = hs.sdd_k;
-        for (int l = 0; l < hs.sdd_n; l++) {
-            const HostSet::HostSeedLevel &H = hs.sdd[l];
-            SeedLevel &L = D.sdd[l];
-            L.k = H.k;
-            L.q = H.q;
-            L.pow = H.pow;
-            L.log2 = H.log2;
-            L.bm_log2 = H.bm_log2;
-            L.max_hits = H.max_hits;
-            L.n_entries = (int)H.entries.size();
-            if (e == cudaSuccess) e = upload(t, H.bstart, &L.bstart);
-            if (e == cudaSuccess) e = upload(t, H.entries, &L.entries);
-            if (e == cudaSuccess) e = upload(t, H.ekeys, &L.ekeys);
-            if (e == cudaSuccess) e = upload(t, H.bitmap, &L.bitmap);
-        }
+        for (int l = 0; l < hs.sdd_n; l++) level(hs.sdd[l], D.sdd[l]);
         D.sv_levels = hs.sv_levels;
         for (int l = 0; l < hs.sv_levels; l++) {
             const HostSet::HostSeedVar &H = hs.sv[l];
@@ -274,9 +229,6 @@ static int get_tables(bdx_config *cfg, int device, DeviceTables **out)
             V.hit_rows = H.hit_rows;
             V.qgram_filter = H.qgram_filter;
             V.sigma_min = H.sigma_min;
-            if (e == cudaSuccess) e = upload(t, H.bstart, &V.bstart);
-            if (e == cudaSuccess) e = upload(t, H.entries, &V.entries);
-            if (e == cudaSuccess) e = upload(t, H.kdepth, &V.kdepth);
         }
         D.hp.enabled = hs.hp_enabled;
         D.hp.m = hs.hp_m;
@@ -288,21 +240,14 @@ static int get_tables(bdx_config *cfg, int device, DeviceTables **out)
             D.hp.seg_q[k] = hs.hp_q[k];
             D.hp.seg_base[k] = hs.hp_base[k];
         }
-        if (e == cudaSuccess) e = upload(t, hs.hp_bstart, &D.hp.bstart);
-        if (e == cudaSuccess) e = upload(t, hs.hp_entries, &D.hp.entries);
-        if (e == cudaSuccess) e = upload(t, hs.hp_bcw, &D.hp.bcw);
-        if (e != cudaSuccess) {
-            free_tables(t);
-            return cuda_fail(e, "uploading barcode tables");
-        }
-        // shared-memory footprints against the device's opt-in limit: the prefilter's hash table and bitmap
-        // (large sets of short barcodes), then the filter kernel's Peq planes
-        if (D.pf_enabled && prefilter_smem_bytes_for(D) > (size_t)prop.sharedMemPerBlockOptin) {
+        // shared-memory footprints against the opt-in limit: the prefilter's hash table and bitmap (large sets of
+        // short barcodes), then the filter kernel's Peq planes
+        if (D.pf_enabled && prefilter_smem_bytes(D) > smem_optin) {
             D.pf_enabled = 0;   // k_prefilter and the k_seed levels behind it are skipped; k_filter takes every read
             D.sd_levels = 0;
             D.sdd_n = 0;
         }
-        if (D.words && filter_smem_bytes_for(D) > (size_t)prop.sharedMemPerBlockOptin) {
+        if (D.words && filter_smem_bytes(D) > smem_optin) {
             D.words = 0;
             D.use_filter = 0;
             D.pf_enabled = 0;
@@ -311,7 +256,63 @@ static int get_tables(bdx_config *cfg, int device, DeviceTables **out)
             D.sv_levels = 0;
         }
     }
-    t->P.filter_ok = t->P.set[0].use_filter && (!t->P.is_dual || t->P.set[1].use_filter);
+    return P;
+}
+
+static int get_tables(bdx_config *cfg, int device, DeviceTables **out)
+{
+    std::lock_guard<std::mutex> lk(cfg->mu);
+    auto it = cfg->per_device.find(device);
+    if (it != cfg->per_device.end()) {
+        *out = it->second;
+        return BDX_OK;
+    }
+    CU(cudaSetDevice(device));
+    cudaDeviceProp prop;
+    CU(cudaGetDeviceProperties(&prop, device));
+    if (prop.major < 10)
+        return fail(BDX_ERR_CUDA, "libbdx is built for sm_100a only; device compute capability too low");
+    DeviceTables *t = new DeviceTables();
+    t->P = host_params(*cfg, prop.sharedMemPerBlockOptin);
+    t->sm_count = prop.multiProcessorCount;
+    const int passes = t->P.is_dual ? 2 : 1;
+    for (int s = 0; s < passes; s++) {
+        const HostSet &hs = cfg->set[s];
+        DevSet &D = t->P.set[s];
+        std::vector<uint8_t> cls(hs.class_of, hs.class_of + 256);
+        cudaError_t e = upload(t, hs.bytes, &D.bc_bytes);
+        if (e == cudaSuccess) e = upload(t, hs.off, &D.bc_off);
+        if (e == cudaSuccess) e = upload(t, hs.norm, &D.norm);
+        if (e == cudaSuccess) e = upload(t, hs.peq, &D.peq);
+        if (e == cudaSuccess) e = upload(t, hs.filt_allowed, &D.filt_allowed);
+        if (e == cudaSuccess) e = upload(t, hs.allowed0, &D.allowed0);
+        if (e == cudaSuccess) e = upload(t, cls, &D.class_of);
+        if (e == cudaSuccess) e = upload(t, hs.pf_bitmap, &D.pf_bitmap);
+        if (e == cudaSuccess) e = upload(t, hs.pf_keys, &D.pf_keys);
+        if (e == cudaSuccess) e = upload(t, hs.pf_vals, &D.pf_vals);
+        if (e == cudaSuccess) e = upload(t, hs.bc_cls, &D.bc_cls);
+        auto level = [&](const HostSet::HostSeedLevel &H, SeedLevel &L) {
+            if (e == cudaSuccess) e = upload(t, H.bstart, &L.bstart);
+            if (e == cudaSuccess) e = upload(t, H.entries, &L.entries);
+            if (e == cudaSuccess) e = upload(t, H.ekeys, &L.ekeys);
+            if (e == cudaSuccess) e = upload(t, H.bitmap, &L.bitmap);
+        };
+        for (int l = 0; l < hs.sd_levels; l++) level(hs.sd[l], D.sd[l]);
+        for (int l = 0; l < hs.sdd_n; l++) level(hs.sdd[l], D.sdd[l]);
+        for (int l = 0; l < hs.sv_levels; l++) {
+            if (e == cudaSuccess) e = upload(t, hs.sv[l].bstart, &D.sv[l].bstart);
+            if (e == cudaSuccess) e = upload(t, hs.sv[l].entries, &D.sv[l].entries);
+            if (e == cudaSuccess) e = upload(t, hs.sv[l].kdepth, &D.sv[l].kdepth);
+        }
+        if (e == cudaSuccess) e = upload(t, hs.hp_bstart, &D.hp.bstart);
+        if (e == cudaSuccess) e = upload(t, hs.hp_entries, &D.hp.entries);
+        if (e == cudaSuccess) e = upload(t, hs.hp_bcw, &D.hp.bcw);
+        if (e != cudaSuccess) {
+            free_tables(t);
+            return cuda_fail(e, "uploading barcode tables");
+        }
+    }
+    for (int pass = 0; pass < passes; pass++) t->plan[pass] = plan_pass(t->P, pass);
     cfg->per_device[device] = t;
     *out = t;
     return BDX_OK;
@@ -517,100 +518,36 @@ int bdx_enqueue_classify(bdx_stream *s, const uint8_t *d_seq, const int32_t *d_o
         return BDX_OK;
     };
     const DevParams &P = s->tab->P;
-    const int passes = P.is_dual ? 2 : 1;
-    for (int pass = 0; pass < passes; pass++) {
-        if (hamming_packed_applies(P, pass)) {
-            // :hamming -- packed pigeonhole scan over every start position, then the literal rules on the candidates
-            if ((rc = staged(kStHamming, [&] { return launch_hamming_scan(P, pass, d_seq, d_off, n, s->sc, s->tab->sm_count, s->st_comp); }))) return rc;
-            if ((rc = staged(kStLiteral, [&] { return launch_literal(P, pass, 1, d_seq, d_off, n, s->sc, s->st_comp); }))) return rc;
-        } else if (exact_hash_applies(P, pass)) {
-            // :exact -- rolling-hash candidate generation, then the literal rules on the candidates
-            if ((rc = staged(kStPrefilter, [&] { return launch_prefilter(P, pass, d_seq, d_off, n, s->sc, s->tab->sm_count, s->d_counters, s->st_comp); }))) return rc;
-            if ((rc = staged(kStLiteral, [&] { return launch_literal(P, pass, 1, d_seq, d_off, n, s->sc, s->st_comp); }))) return rc;
-        } else if (P.set[pass].words > 0) {
-            const bool pre = prefilter_applies(P, pass);
-            CU(cudaMemsetAsync(s->sc.n_lit, 0, 2 * sizeof(int), s->st_comp));   // k_literal's two read lists
-            if (pre) {
-                if ((rc = staged(kStPrefilter, [&] { return launch_prefilter(P, pass, d_seq, d_off, n, s->sc, s->tab->sm_count, s->d_counters, s->st_comp); }))) return rc;
-            }
-            int wl = pre ? 1 : 0;
-            {
-                // seed levels hand the reads they cannot finish from one worklist to the other; without a
-                // prefilter in front (min_delta != 0) the first level takes every read of the batch
-                // barcodes of different lengths / constrained start or end: k_seed_var instead of the levels
-                const int sv_levels = seed_var_levels(P, pass);
-                for (int l = 0; l < sv_levels; l++) {
-                    const int *wl_in = wl == 0 ? nullptr : (wl == 1 ? s->sc.worklist : s->sc.worklist2);
-                    const int *n_in = wl == 0 ? nullptr : (wl == 1 ? s->sc.n_work : s->sc.n_work2);
-                    const bool to2 = wl != 2;
-                    if ((rc = staged(l == 0 ? kStSeed : kStSeedDeep, [&] { return launch_seed_var(P, pass, l, d_seq, d_off, n, s->sc, wl_in, n_in,
-                                   to2 ? s->sc.worklist2 : s->sc.worklist, to2 ? s->sc.n_work2 : s->sc.n_work,
-                                   s->tab->sm_count, s->d_counters, s->st_comp); }))) return rc;
-                    wl = to2 ? 2 : 1;
+    const Scratch &sc = s->sc;
+    const int sm = s->tab->sm_count;
+    unsigned long long *const ctr = s->d_counters;
+    cudaStream_t st = s->st_comp;
+    int *const wl[3] = {nullptr, sc.worklist, sc.worklist2}, *const n_wl[3] = {nullptr, sc.n_work, sc.n_work2};
+    for (int pass = 0; pass < (P.is_dual ? 2 : 1); pass++) {
+        const PassPlan &plan = s->tab->plan[pass];
+        if (plan.clear_lit) CU(cudaMemsetAsync(sc.n_lit, 0, 2 * sizeof(int), st));   // k_literal's two read lists
+        for (int i = 0; i < plan.n; i++) {
+            const PlanStep &t = plan.step[i];
+            int *const in = wl[t.in], *const n_in = n_wl[t.in], *const out = wl[t.out], *const n_out = n_wl[t.out];
+            const int *const list[5] = {nullptr, nullptr, sc.wl_win, sc.wl_full, in};   // k_literal's read list by t.reads
+            const int *const len[5] = {nullptr, nullptr, sc.n_lit, sc.n_lit + 1, n_in};
+            if ((rc = staged(t.stage, [&]() -> cudaError_t {
+                switch (t.kind) {
+                case kStepHammingScan: return launch_hamming_scan(P, pass, d_seq, d_off, n, sc, sm, st);
+                case kStepPrefilter: return launch_prefilter(P, pass, d_seq, d_off, n, sc, sm, ctr, st);
+                case kStepSeed: return launch_seed(P, pass, t.level, d_seq, d_off, n, sc, in, n_in, out, n_out, sm, ctr, st);
+                case kStepSeedVar: return launch_seed_var(P, pass, t.level, d_seq, d_off, n, sc, in, n_in, out, n_out, sm, ctr, st);
+                case kStepSeedDeep: return launch_seed_deep(P, pass, d_seq, d_off, n, sc, in, n_in, out, n_out, sm, ctr, st);
+                case kStepFilter: return launch_filter(P, pass, d_seq, d_off, n, sc, sm, ctr, in, n_in, st);
+                case kStepMarkPending: return launch_mark_pending(P, pass, n, sc, in, n_in, st);
+                case kStepLiteral: return launch_literal(P, pass, t.reads != kLitAll, d_seq, d_off, n, sc, st, list[t.reads], len[t.reads]);
                 }
-                const int levels = sv_levels ? 0 : seed_levels(P, pass);
-                for (int l = 0; l < levels; l++) {
-                    const int *wl_in = wl == 0 ? nullptr : (wl == 1 ? s->sc.worklist : s->sc.worklist2);
-                    const int *n_in = wl == 0 ? nullptr : (wl == 1 ? s->sc.n_work : s->sc.n_work2);
-                    const bool to2 = wl != 2;
-                    if ((rc = staged(kStSeed, [&] { return launch_seed(P, pass, l, d_seq, d_off, n, s->sc, wl_in, n_in, to2 ? s->sc.worklist2 : s->sc.worklist,
-                                   to2 ? s->sc.n_work2 : s->sc.n_work, s->tab->sm_count, s->d_counters, s->st_comp); }))) return rc;
-                    wl = to2 ? 2 : 1;
-                }
-                const int tail = levels > 0 ? seed_var_tail_level(P, pass) : -1;
-                if (tail >= 0) {
-                    // k_seed_var's complete level on what k_seed's levels left: verdicts are final, k_filter sees only
-                    // the reads it hands on (hit-list overflow)
-                    const bool to2 = wl != 2;
-                    if ((rc = staged(kStSeedDeep, [&] { return launch_seed_var(P, pass, tail, d_seq, d_off, n, s->sc, wl == 1 ? s->sc.worklist : s->sc.worklist2,
-                                        wl == 1 ? s->sc.n_work : s->sc.n_work2, to2 ? s->sc.worklist2 : s->sc.worklist,
-                                        to2 ? s->sc.n_work2 : s->sc.n_work, s->tab->sm_count, s->d_counters, s->st_comp); }))) return rc;
-                    wl = to2 ? 2 : 1;
-                }
-                if (levels > 0 && tail < 0 && seed_deep_applies(P, pass)) {
-                    const bool to2 = wl != 2;
-                    if ((rc = staged(kStSeedDeep, [&] { return launch_seed_deep(P, pass, d_seq, d_off, n, s->sc, wl == 1 ? s->sc.worklist : s->sc.worklist2,
-                                        wl == 1 ? s->sc.n_work : s->sc.n_work2, to2 ? s->sc.worklist2 : s->sc.worklist,
-                                        to2 ? s->sc.n_work2 : s->sc.n_work, s->tab->sm_count, s->d_counters, s->st_comp); }))) return rc;
-                    wl = to2 ? 2 : 1;
-                }
-            }
-            if (!P.set[pass].use_filter) {
-                // tiny set: no filter kernel.  What the shortcut stages left goes to k_literal over every barcode.
-                if (wl == 0) {
-                    if ((rc = staged(kStLiteral, [&] { return launch_literal(P, pass, 0, d_seq, d_off, n, s->sc, s->st_comp); }))) return rc;
-                } else {
-                    const int *rest = wl == 1 ? s->sc.worklist : s->sc.worklist2;
-                    const int *n_rest = wl == 1 ? s->sc.n_work : s->sc.n_work2;
-                    if ((rc = staged(kStOther, [&] { return launch_mark_pending(P, pass, n, s->sc, rest, n_rest, s->st_comp); }))) return rc;
-                    // seed winners (windowed) and the scan-everything rest as separate, compacted launches
-                    if ((rc = staged(kStLiteral, [&] { return launch_literal(P, pass, 1, d_seq, d_off, n, s->sc, s->st_comp, s->sc.wl_win, s->sc.n_lit); }))) return rc;
-                    if ((rc = staged(kStLiteral, [&] { return launch_literal(P, pass, 1, d_seq, d_off, n, s->sc, s->st_comp, rest, n_rest); }))) return rc;
-                }
-                continue;
-            }
-            if ((rc = staged(kStFilter, [&] { return launch_filter(P, pass, d_seq, d_off, n, s->sc, s->tab->sm_count, s->d_counters, wl, s->st_comp); }))) return rc;
-            // the exact regime finishes inside the filter kernel; anything else leaves
-            // kBcPending reads with candidate lists for the literal kernel
-            const bool may_finish = P.algo == BDX_SEMIGLOBAL && P.unit_costs && P.set[pass].trim_side == 0 &&
-                                    !P.want_stats;
-            const DevRange &bs = P.set[pass].bs, &be = P.set[pass].be;
-            const bool default_geometry = bs.start_off <= 1 && !bs.start_from_end && bs.end_from_end &&
-                                          bs.end_off >= 0 && be.start_off <= 1 && !be.start_from_end;
-            if (!(may_finish && default_geometry)) {
-                // seed winners (windowed DP) and k_filter's candidate reads as separate, compacted launches:
-                // a warp costs as much as its most expensive lane
-                if (wl != 0 && seed_levels(P, pass) > 0) {
-                    if ((rc = staged(kStLiteral, [&] { return launch_literal(P, pass, 1, d_seq, d_off, n, s->sc, s->st_comp, s->sc.wl_win, s->sc.n_lit); }))) return rc;
-                }
-                if ((rc = staged(kStLiteral, [&] { return launch_literal(P, pass, 1, d_seq, d_off, n, s->sc, s->st_comp, s->sc.wl_full, s->sc.n_lit + 1); }))) return rc;
-            }
-        } else {
-            if ((rc = staged(kStLiteral, [&] { return launch_literal(P, pass, 0, d_seq, d_off, n, s->sc, s->st_comp); }))) return rc;
+                return cudaErrorInvalidValue;
+            }))) return rc;
         }
     }
     StatsDev sd{s->d_stats, s->cfg->lay, s->d_ovf, s->d_n_ovf, (unsigned int)std::min<int64_t>(s->ovf_cap, 0xFFFFFFFFll)};
-    if ((rc = staged(kStFinalize, [&] { return launch_finalize(P, d_off, n, s->sc, d_res, d_det, sd, s->st_comp); }))) return rc;
+    if ((rc = staged(kStFinalize, [&] { return launch_finalize(P, d_off, n, sc, d_res, d_det, sd, st); }))) return rc;
     return BDX_OK;
 }
 
@@ -782,7 +719,10 @@ extern "C" int bdx_config_code_table(const bdx_config *cfg, uint8_t table[256])
 extern "C" int bdx_config_describe(const bdx_config *cfg, int pass, char *buf, int len)
 {
     if (!cfg || pass < 0 || pass > 1 || len < 0 || (len > 0 && !buf)) return fail(BDX_ERR_INVALID, "bad argument");
-    const std::string text = cfg->set[pass].n_bc ? bdx_describe_set(cfg->set[pass]) : std::string();
+    std::string text;
+    if (cfg->set[pass].n_bc)
+        text = bdx_describe_set(cfg->set[pass]) + "plan: steps=" +
+               plan_text(plan_pass(host_params(*cfg, kSm100SmemOptin), pass)) + "\n";
     if (len > 0) {
         const size_t k = std::min(text.size(), (size_t)len - 1);
         memcpy(buf, text.data(), k);

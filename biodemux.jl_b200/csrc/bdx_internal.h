@@ -141,7 +141,6 @@ struct DevParams {
     double max_error_rate, min_delta;
     int match, mismatch, indel, nindel, has_n;
     int algo, is_dual, want_stats;
-    int filter_ok;    // costs allow the unit-cost filter to be a superset (DESIGN.md)
     int unit_costs;   // match 0, mismatch 1, indel 1 (and nindel 1): filter distance is the score
     int two;          // (reserved)
     int debug;        // BDX_DEBUG_* flags of the config (test hooks)
@@ -182,14 +181,22 @@ struct Scratch {
 // threads, smem): the two runtime queries cost microseconds each, which adds up for 4000-read batches.
 cudaError_t blocks_per_sm_cached(const void *kern, int threads, size_t smem, int *per_sm);
 
+// dynamic shared memory of each kernel's launch, from its file's layout arithmetic (the pass plan, plan.cu, holds
+// them against its budgets)
+size_t hamming_scan_smem(const DevSet &S);
+size_t prefilter_smem_bytes(const DevSet &S);
+size_t filter_smem_bytes(const DevSet &S);
+size_t seed_smem(const DevSet &S, const SeedLevel &L);
+size_t deep_smem(const DevSet &S);
+size_t seed_var_smem(const DevSet &S, const SeedVar &V);
+
 // ---- launch wrappers (kernels.cu / filter.cu) ----
 cudaError_t launch_literal(const DevParams &P, int pass, int from_filter, const uint8_t *seq,
                            const int *off, int n, const Scratch &sc, cudaStream_t st, const int *list = nullptr,
                            const int *n_list = nullptr);   // list: compacted read indices (length on the device)
 cudaError_t launch_filter(const DevParams &P, int pass, const uint8_t *seq, const int *off, int n,
-                          const Scratch &sc, int sm_count, unsigned long long *counters, int use_worklist,
-                          cudaStream_t st);   // use_worklist: 0 = all reads, 1 = worklist, 2 = worklist2
-int seed_levels(const DevParams &P, int pass);   // number of k_seed levels that apply (0 = none)
+                          const Scratch &sc, int sm_count, unsigned long long *counters, const int *wl, const int *n_wl,
+                          cudaStream_t st);   // wl: the reads to scan (nullptr: all of them)
 // level `level` over the reads of wl_in; the reads it cannot finish are appended to wl_out
 cudaError_t launch_seed(const DevParams &P, int pass, int level, const uint8_t *seq, const int *off, int n,
                         const Scratch &sc, const int *wl_in, const int *n_in, int *wl_out, int *n_out, int sm_count,
@@ -197,20 +204,14 @@ cudaError_t launch_seed(const DevParams &P, int pass, int level, const uint8_t *
 // reads of a worklist that no kernel resolved: queue them for k_literal over every barcode
 cudaError_t launch_mark_pending(const DevParams &P, int pass, int n, const Scratch &sc, const int *wl, const int *n_wl,
                                 cudaStream_t st);
-int seed_var_levels(const DevParams &P, int pass);     // number of k_seed_var levels that apply (0 = none)
-int seed_var_tail_level(const DevParams &P, int pass); // the complete level, usable behind k_seed's levels (-1 = none)
 cudaError_t launch_seed_var(const DevParams &P, int pass, int level, const uint8_t *seq, const int *off, int n, const Scratch &sc,
                             const int *wl_in, const int *n_in, int *wl_out, int *n_out, int sm_count,
                             unsigned long long *counters, cudaStream_t st);
-bool seed_deep_applies(const DevParams &P, int pass);
 cudaError_t launch_seed_deep(const DevParams &P, int pass, const uint8_t *seq, const int *off, int n, const Scratch &sc,
                              const int *wl_in, const int *n_in, int *wl_out, int *n_out, int sm_count,
                              unsigned long long *counters, cudaStream_t st);
 cudaError_t launch_prefilter(const DevParams &P, int pass, const uint8_t *seq, const int *off, int n,
                              const Scratch &sc, int sm_count, unsigned long long *counters, cudaStream_t st);
-bool prefilter_applies(const DevParams &P, int pass);
-bool exact_hash_applies(const DevParams &P, int pass);
-bool hamming_packed_applies(const DevParams &P, int pass);
 cudaError_t launch_hamming_scan(const DevParams &P, int pass, const uint8_t *seq, const int *off, int n,
                                 const Scratch &sc, int sm_count, cudaStream_t st);
 cudaError_t launch_finalize(const DevParams &P, const int *off, int n, const Scratch &sc,

@@ -344,8 +344,6 @@ k_filter(const __grid_constant__ DevParams P, const int pass, const uint8_t *__r
 // and byte-wise verification on a hit.  Resolved reads get their PassOut here; all other
 // reads are appended to the worklist the bit-parallel kernel then walks.
 // ---------------------------------------------------------------------------------------
-size_t prefilter_smem_bytes_for(const DevSet &S);
-
 constexpr int kPfThreads = 256;
 constexpr int kPfStageBytes = 48 * 1024;   // raw bytes of one group of 256 reads (<= 192 bases each)
 constexpr int kPfMaxCand = 2;              // table hits remembered per read; more => leave it to the DP
@@ -604,7 +602,7 @@ k_prefilter(const __grid_constant__ DevParams P, const int pass, const uint8_t *
                 }
             } else if (g.valid && g.max_start_pos >= n && g.min_end_pos <= g.start_j && ncols >= seed) {
                 // same per-read regime test as k_filter's `fast` (the cost conditions are config-level and
-                // checked by the launcher, prefilter_applies)
+                // checked by the pass plan, plan.cu)
                 // Positions (trimming / stats): every hit of the winning barcode scores 0, so the reference keeps
                 // the first one it meets (early exit for trim 5, no later hit is strictly better otherwise,
                 // classification.jl:419-436, :141-153) -- the leftmost occurrence -- or, trimming 3', the one
@@ -640,7 +638,7 @@ cudaError_t launch_prefilter(const DevParams &P, int pass, const uint8_t *seq, c
                              const Scratch &sc, int sm_count, unsigned long long *counters, cudaStream_t st)
 {
     const DevSet &S = P.set[pass];
-    const size_t smem = prefilter_smem_bytes_for(S);
+    const size_t smem = prefilter_smem_bytes(S);
     auto kern = P.algo == BDX_EXACT ? k_prefilter<1> : (P.algo == BDX_HAMMING ? k_prefilter<2> : k_prefilter<0>);
     int per_sm = 0;
     cudaError_t e = blocks_per_sm_cached((const void *)kern, kPfThreads, smem, &per_sm);
@@ -654,28 +652,7 @@ cudaError_t launch_prefilter(const DevParams &P, int pass, const uint8_t *seq, c
     return cudaGetLastError();
 }
 
-// :exact with a hash table: k_prefilter<1> replaces the Shift-And filter kernel altogether
-bool exact_hash_applies(const DevParams &P, int pass)
-{
-    const DevSet &S = P.set[pass];
-    return P.algo == BDX_EXACT && S.use_filter && S.pf_enabled && P.max_error_rate >= 0.0;
-}
-
-// true when every read of this pass that is in the exact regime may be resolved by k_prefilter
-bool prefilter_applies(const DevParams &P, int pass)
-{
-    const DevSet &S = P.set[pass];
-    if (P.algo == BDX_HAMMING)   // positions are produced, so trim / stats are fine; needs no wildcard rows
-        return S.use_filter && S.pf_enabled && P.min_delta == 0.0 && P.max_error_rate >= 0.0;
-    // :semiglobal -- with trimming / stats the resolved reads also need positions: a verbatim occurrence has
-    // them (k_prefilter), a seed-resolved read gets them from k_literal run on its single winning barcode
-    // Any positive edit costs will do (match = 0): a verbatim occurrence is the only way to score 0, whatever a
-    // mismatch or a gap costs, and score 0 beats every other barcode under the strict "<" of :658.
-    return P.algo == BDX_SEMIGLOBAL && S.words > 0 && S.pf_enabled && P.match == 0 && P.mismatch >= 1 && P.indel >= 1 &&
-           P.min_delta == 0.0 && P.max_error_rate >= 0.0;
-}
-
-static size_t filter_smem_bytes(const DevSet &S)
+size_t filter_smem_bytes(const DevSet &S)
 {
     const size_t n_pad = (size_t)S.n_bc_pad;
     size_t b = (size_t)S.words * S.n_classes * n_pad * 4;
@@ -686,7 +663,7 @@ static size_t filter_smem_bytes(const DevSet &S)
 
 template <int W, int G, int CODING, bool PAIR>
 static cudaError_t launch_wgv(const DevParams &P, int pass, const uint8_t *seq, const int *off, int n,
-                              const Scratch &sc, int sm_count, unsigned long long *counters, int use_worklist,
+                              const Scratch &sc, int sm_count, unsigned long long *counters, const int *wl, const int *n_wl,
                               cudaStream_t st)
 {
     const size_t smem = filter_smem_bytes(P.set[pass]);
@@ -700,25 +677,22 @@ static cudaError_t launch_wgv(const DevParams &P, int pass, const uint8_t *seq, 
     if (blocks > need) blocks = need;
     if (blocks < 1) blocks = 1;
     kern<<<(unsigned)blocks, kFilterWarps * 32, smem, st>>>(P, pass, seq, off, n, sc.pass[pass], sc.pass[0],
-                                                            sc.cand, sc.cand_cnt, counters,
-                                                            use_worklist == 2 ? sc.worklist2 : (use_worklist ? sc.worklist : nullptr),
-                                                            use_worklist == 2 ? sc.n_work2 : (use_worklist ? sc.n_work : nullptr),
-                                                            sc.wl_full, sc.n_lit + 1);
+                                                            sc.cand, sc.cand_cnt, counters, wl, n_wl, sc.wl_full, sc.n_lit + 1);
     return cudaGetLastError();
 }
 
 template <int W, int G>
 static cudaError_t launch_wg(const DevParams &P, int pass, const uint8_t *seq, const int *off, int n,
-                             const Scratch &sc, int sm_count, unsigned long long *counters, int use_worklist,
+                             const Scratch &sc, int sm_count, unsigned long long *counters, const int *wl, const int *n_wl,
                              cudaStream_t st)
 {
     if (P.algo == BDX_EXACT)
-        return launch_wgv<W, G, kShiftAnd, false>(P, pass, seq, off, n, sc, sm_count, counters, use_worklist, st);
-    return launch_wgv<W, G, kMyers, true>(P, pass, seq, off, n, sc, sm_count, counters, use_worklist, st);
+        return launch_wgv<W, G, kShiftAnd, false>(P, pass, seq, off, n, sc, sm_count, counters, wl, n_wl, st);
+    return launch_wgv<W, G, kMyers, true>(P, pass, seq, off, n, sc, sm_count, counters, wl, n_wl, st);
 }
 
 cudaError_t launch_filter(const DevParams &P, int pass, const uint8_t *seq, const int *off, int n,
-                          const Scratch &sc, int sm_count, unsigned long long *counters, int use_worklist,
+                          const Scratch &sc, int sm_count, unsigned long long *counters, const int *wl, const int *n_wl,
                           cudaStream_t st)
 {
     if (n <= 0) return cudaSuccess;
@@ -726,17 +700,15 @@ cudaError_t launch_filter(const DevParams &P, int pass, const uint8_t *seq, cons
     const int groups = S.n_bc_pad / 32;
     const int G = groups >= 4 && groups % 4 == 0 ? 4 : (groups % 3 == 0 ? 3 : (groups % 2 == 0 ? 2 : 1));
 #define BDX_CASE(W_, G_) \
-    if (S.words == W_ && G == G_) return launch_wg<W_, G_>(P, pass, seq, off, n, sc, sm_count, counters, use_worklist, st);
+    if (S.words == W_ && G == G_) return launch_wg<W_, G_>(P, pass, seq, off, n, sc, sm_count, counters, wl, n_wl, st);
     BDX_CASE(1, 1) BDX_CASE(1, 2) BDX_CASE(1, 3) BDX_CASE(1, 4)
     BDX_CASE(2, 1) BDX_CASE(2, 2) BDX_CASE(2, 3) BDX_CASE(2, 4)
 #undef BDX_CASE
     return cudaErrorInvalidValue;
 }
 
-size_t filter_smem_bytes_for(const DevSet &S) { return filter_smem_bytes(S); }
-
 // k_prefilter's dynamic shared memory: read staging + hash table (keys, values) + first-level bitmap
-size_t prefilter_smem_bytes_for(const DevSet &S)
+size_t prefilter_smem_bytes(const DevSet &S)
 {
     return kPfStageBytes + 16 + ((size_t)8 << S.pf_log2) + ((size_t)4 << (S.pf_bm_log2 - 5));
 }

@@ -196,7 +196,7 @@ k_hamming_scan(const __grid_constant__ DevParams P, const int pass, const uint8_
     }
 }
 
-static size_t hamming_scan_smem(const DevSet &S)
+size_t hamming_scan_smem(const DevSet &S)
 {
     const HammingPacked &H = S.hp;
     size_t b = 3 * (size_t)kHpPlane * kHpThreads * 4;
@@ -204,13 +204,6 @@ static size_t hamming_scan_smem(const DevSet &S)
     b += (size_t)((H.n_bstart + 1) & ~1) * 2 + (size_t)((H.n_seg * S.n_bc + 1) & ~1) * 2;
     b += (size_t)kCandMax * kHpThreads * 4 + 256;
     return (b + 15) & ~(size_t)15;
-}
-
-bool hamming_packed_applies(const DevParams &P, int pass)
-{
-    const bool off = false;   // (switched off through BDX_DEBUG_* at config creation: the tables are not built then)
-    const DevSet &S = P.set[pass];
-    return !off && P.algo == BDX_HAMMING && S.hp.enabled && hamming_scan_smem(S) <= 200 * 1024;
 }
 
 cudaError_t launch_hamming_scan(const DevParams &P, int pass, const uint8_t *seq, const int *off, int n,

@@ -345,17 +345,7 @@ static size_t seed_smem(const DevSet &S, const SeedLevel &L, bool tab_smem)
 // the CSR table goes to shared memory while the whole carve-up stays small enough for >= 3 blocks per SM
 static bool seed_tab_in_smem(const DevSet &S, const SeedLevel &L) { return seed_smem(S, L, true) <= 72 * 1024; }
 
-int seed_levels(const DevParams &P, int pass)
-{
-    const bool off = false;   // (switched off through BDX_DEBUG_* at config creation: the tables are not built then)
-    const DevSet &S = P.set[pass];
-    // the exact regime of k_filter (unit costs, uniform length, no wildcard rows: the tables exist only then);
-    // min_delta is handled, trimming / stats go through k_literal for the positions
-    if (off || P.algo != BDX_SEMIGLOBAL || !P.unit_costs || !S.pf_enabled || S.words < 1 || P.max_error_rate < 0.0) return 0;
-    for (int l = 0; l < S.sd_levels; l++)
-        if (seed_smem(S, S.sd[l], seed_tab_in_smem(S, S.sd[l])) > 110 * 1024) return 0;
-    return S.sd_levels;
-}
+size_t seed_smem(const DevSet &S, const SeedLevel &L) { return seed_smem(S, L, seed_tab_in_smem(S, L)); }
 
 cudaError_t launch_seed(const DevParams &P, int pass, int level, const uint8_t *seq, const int *off, int n,
                         const Scratch &sc, const int *wl_in, const int *n_in, int *wl_out, int *n_out, int sm_count,

@@ -263,20 +263,12 @@ k_seed_deep(const __grid_constant__ DevParams P, const int pass, const uint8_t *
     if (lane == 0 && n_done && counters) atomicAdd(counters + 2, (unsigned long long)n_done);
 }
 
-static size_t deep_smem(const DevSet &S)
+size_t deep_smem(const DevSet &S)
 {
     size_t words = (size_t)S.words * S.n_classes * S.n_bc_pad + (size_t)kSeedMaxHits * kSeedThreads;
     for (int t = 0; t < S.sdd_n; t++)
         words += ((size_t)1 << (S.sdd[t].bm_log2 - 5)) + ((size_t)1 << S.sdd[t].log2) + 1 + 2 * (size_t)S.sdd[t].n_entries;
     return words * 4 + (size_t)kSeedMaxWins * kSeedThreads * 2 + 256 + (size_t)kSeedThreads * kSeedSlot + 16;
-}
-
-// the deep level runs after k_seed's levels, for min_delta = 0 (it keeps no runner-up)
-bool seed_deep_applies(const DevParams &P, int pass)
-{
-    const bool off = false;   // (switched off through BDX_DEBUG_* at config creation: the tables are not built then)
-    const DevSet &S = P.set[pass];
-    return !off && S.sdd_n > 0 && seed_levels(P, pass) > 0 && P.min_delta == 0.0 && deep_smem(S) <= 96 * 1024;
 }
 
 cudaError_t launch_seed_deep(const DevParams &P, int pass, const uint8_t *seq, const int *off, int n, const Scratch &sc,

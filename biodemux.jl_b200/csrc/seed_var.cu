@@ -705,13 +705,6 @@ static int sv_slot_cols(const DevSet &S)
     return kSvMaxCols;
 }
 
-static bool sv_default_geometry(const DevSet &S)
-{
-    const DevRange &bs = S.bs, &be = S.be;
-    return bs.start_off <= 1 && !bs.start_from_end && bs.end_from_end && bs.end_off >= 0 && be.start_off <= 1 &&
-           !be.start_from_end;
-}
-
 struct SvLaunch {
     int slot_cols, slot_stride;
     size_t smem;
@@ -731,30 +724,7 @@ static SvLaunch sv_launch_params(const DevSet &S, const SeedVar &V)
     return L;
 }
 
-// Does k_seed_var take this pass?  Score-only :semiglobal passes with unit costs whose set has the tables, when
-// k_seed's levels do not apply (barcodes of different lengths) or would refuse every read (constrained start / end).
-int seed_var_levels(const DevParams &P, int pass)
-{
-    const DevSet &S = P.set[pass];
-    if (P.algo != BDX_SEMIGLOBAL || !P.unit_costs || S.sv_levels < 1 || S.words < 1 || P.max_error_rate < 0.0) return 0;
-    if (S.trim_side != 0 || P.want_stats) return 0;
-    if (seed_levels(P, pass) > 0 && sv_default_geometry(S) && !(P.debug & BDX_DEBUG_PREFER_SEED_VAR)) return 0;
-    for (int l = 0; l < S.sv_levels; l++)
-        if (sv_launch_params(S, S.sv[l]).smem > 160 * 1024) return l;
-    return S.sv_levels;
-}
-
-// The complete level behind k_seed's own levels (uniform-length sets in the default geometry): it takes the reads
-// they could not finish -- best barcode at the allowed distance, or none at all -- instead of k_filter.
-int seed_var_tail_level(const DevParams &P, int pass)
-{
-    const DevSet &S = P.set[pass];
-    if (P.algo != BDX_SEMIGLOBAL || !P.unit_costs || S.sv_levels < 1 || S.words < 1 || P.max_error_rate < 0.0) return -1;
-    if (S.trim_side != 0 || P.want_stats) return -1;
-    const int l = S.sv_levels - 1;
-    if (!S.sv[l].complete || sv_launch_params(S, S.sv[l]).smem > 160 * 1024) return -1;
-    return l;
-}
+size_t seed_var_smem(const DevSet &S, const SeedVar &V) { return sv_launch_params(S, V).smem; }
 
 cudaError_t launch_seed_var(const DevParams &P, int pass, int level, const uint8_t *seq, const int *off, int n, const Scratch &sc,
                             const int *wl_in, const int *n_in, int *wl_out, int *n_out, int sm_count,

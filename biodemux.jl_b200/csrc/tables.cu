@@ -516,7 +516,7 @@ void build_seed_var(const Build &B)
                     build_complete(q_lo, segs, e.chance);
             }
         }
-        // With a complete level behind them (score-only passes: seed_var_tail_level), k_seed's levels only have to
+        // With a complete level behind them (score-only passes, plan.cu), k_seed's levels only have to
         // be cheap, not deep: its second level is dropped when its seeds are short (> 0.02 chance hits per column,
         // e.g. 96 x 24 nt at depth 3: 6-mers, 14 chance hits per read) -- the reads it resolved cost less in the
         // complete level than the level costs on all of its input (config 2: 889 -> 910 M reads/s).  Sets without a

@@ -186,8 +186,11 @@ void bdx_host_free(void *p);
  * thread-safe, no CUDA): n_bytes input bytes -> (n_bytes + 1) / 2 output bytes. */
 int bdx_config_code_table(const bdx_config *cfg, uint8_t table[256]);   /* returns the number of codes incl. 0 */
 /* Diagnostics: a text description (one line per table) of what bdx_config_create built for barcode set `pass`
- * (0 or 1) -- which shortcut stages exist and their level parameters (seed lengths, depths, group sizes).  Writes at
- * most len - 1 bytes and a NUL; returns the full length of the text (0 for an absent second set).  Host data only. */
+ * (0 or 1) -- which shortcut stages exist and their level parameters (seed lengths, depths, group sizes) -- and a
+ * last line `plan: steps=...` naming the kernels the pass launches, in order (k_seed@1 = k_seed's level 1; k_literal
+ * @all / @cand / @win / @full / @rest = the reads it scans).  The plan is computed for sm_100's shared-memory limit
+ * per block (227 KB), the only device the library runs on.  Writes at most len - 1 bytes and a NUL; returns the
+ * full length of the text (0 for an absent second set).  Host data only. */
 int bdx_config_describe(const bdx_config *cfg, int pass, char *buf, int len);
 int bdx_pack_reads4(const bdx_config *cfg, const uint8_t *seq_bytes, int64_t n_bytes, uint8_t *packed_out);
 int bdx_submit_packed4(bdx_stream *s, const uint8_t *packed, const int32_t *offsets, int32_t n_reads, uint64_t tag);
