@@ -30,6 +30,7 @@ DEBUG_NO_QGRAM_FILTER = 256
 EXPORTS = [
     "bdx_last_error", "bdx_abi_version", "bdx_device_count", "bdx_config_create", "bdx_config_create_debug", "bdx_config_destroy",
     "bdx_stream_work_counters", "bdx_config_code_table", "bdx_config_describe", "bdx_pack_reads4", "bdx_submit_packed4", "bdx_submit_packed4_pinned",
+    "bdx_window_spans", "bdx_window_reads", "bdx_submit_windows", "bdx_submit_windows_pinned",
     "bdx_stream_create", "bdx_stream_destroy", "bdx_submit", "bdx_acquire", "bdx_commit",
     "bdx_submit_pinned", "bdx_host_alloc", "bdx_host_free", "bdx_stream_enable_details",
     "bdx_fetch", "bdx_fetch_view", "bdx_classify", "bdx_classify_device", "bdx_stream_sync",
@@ -129,6 +130,10 @@ def load_library():
     L.bdx_pack_reads4.argtypes = [vp, vp, i64, vp]
     L.bdx_submit_packed4.argtypes = [vp, vp, vp, C.c_int32, C.c_uint64]
     L.bdx_submit_packed4_pinned.argtypes = [vp, vp, vp, C.c_int32, C.c_uint64]
+    L.bdx_window_spans.argtypes = [vp, i32, vp]
+    L.bdx_window_reads.argtypes = [vp, vp, vp, i32, vp, vp]
+    L.bdx_submit_windows.argtypes = [vp, vp, vp, vp, i32, C.c_int, u64]
+    L.bdx_submit_windows_pinned.argtypes = [vp, vp, vp, vp, i32, C.c_int, u64]
     L.bdx_config_destroy.argtypes = [vp]
     L.bdx_config_destroy.restype = None
     L.bdx_stream_create.argtypes = [vp, C.c_int, i32, i64, C.POINTER(vp)]
@@ -320,6 +325,26 @@ class Config:
         _check(self.lib.bdx_pack_reads4(self.handle, seq.ctypes.data, seq.size, out.ctypes.data))
         return out
 
+    def window_spans(self, read_len: int):
+        """bdx_window_spans: ((lo1, hi1, lo2, hi2), window length) of a read of ``read_len`` bases."""
+        sp = np.zeros(4, np.int32)
+        n = self.lib.bdx_window_spans(self.handle, int(read_len), sp.ctypes.data)
+        if n < 0:
+            _check(n)
+        return tuple(int(x) for x in sp), int(n)
+
+    def window_reads(self, seq: np.ndarray, off: np.ndarray):
+        """bdx_window_reads: (window bytes, int32 window offsets) of the concatenated reads ``seq`` / ``off``."""
+        seq = np.ascontiguousarray(seq, dtype=np.uint8)
+        off = np.ascontiguousarray(off, dtype=np.int32)
+        n = len(off) - 1
+        win_off = np.zeros(n + 1, np.int32)
+        _check(self.lib.bdx_window_reads(self.handle, None, off.ctypes.data, n, None, win_off.ctypes.data))
+        win = np.zeros(max(int(win_off[-1]), 1), np.uint8)
+        _check(self.lib.bdx_window_reads(self.handle, seq.ctypes.data if seq.size else None, off.ctypes.data, n,
+                                         win.ctypes.data, win_off.ctypes.data))
+        return win[:int(win_off[-1])], win_off
+
     def _set(self, seqs: Sequence[str], lens: Sequence[int], rs, bs, be, trim) -> BarcodeSet:
         raw = [s.encode("latin-1") if isinstance(s, str) else bytes(s) for s in seqs]
         blob = np.frombuffer(b"".join(raw) + b"\0", dtype=np.uint8).copy()
@@ -376,6 +401,14 @@ class Stream:
         """4-bit packed reads (Config.pack4) + the offsets of the unpacked reads."""
         fn = self.lib.bdx_submit_packed4_pinned if pinned else self.lib.bdx_submit_packed4
         _check(fn(self.handle, packed.ctypes.data, off.ctypes.data, len(off) - 1, tag))
+
+    def submit_windows(self, win: np.ndarray, win_off: np.ndarray, off: np.ndarray, packed4: bool = False,
+                       pinned: bool = False, tag: int = 0):
+        """The reads' window bytes (Config.window_reads; packed4: those packed by Config.pack4) + the window offsets
+        + the offsets of the full reads."""
+        fn = self.lib.bdx_submit_windows_pinned if pinned else self.lib.bdx_submit_windows
+        _check(fn(self.handle, win.ctypes.data if win.size else None, win_off.ctypes.data, off.ctypes.data,
+                  len(off) - 1, int(packed4), tag))
 
     def fetch(self, want_details: bool = False, copy: bool = True):
         """Oldest in-flight batch.  copy=False returns views into the stream's pinned result
@@ -596,8 +629,11 @@ class Engine:
     """Config + one stream: what a single reference worker thread would own."""
 
     def __init__(self, cfg: DemuxConfig, device: int = 0, max_reads: int = 4000,
-                 max_bytes: Optional[int] = None, want_stats: Optional[bool] = None, debug: int = 0):
+                 max_bytes: Optional[int] = None, want_stats: Optional[bool] = None, debug: int = 0,
+                 windows: bool = False):
+        """windows: classify_packed sends only the reads' search-window bytes (bdx_submit_windows)."""
         self.cfg = cfg
+        self.windows = windows
         self.config = Config(cfg, want_stats=want_stats, debug=debug)
         self._device = device
         self.stream = Stream(self.config, device=device, max_reads=max_reads, max_bytes=max_bytes)
@@ -622,7 +658,7 @@ class Engine:
             if details != st.details:
                 st.enable_details(details)
         if n <= st.max_reads and (n == 0 or int(off[-1]) <= st.max_bytes):
-            return st.classify(blob, off.astype(np.int32), want_details=want_details)
+            return self._classify(blob, off.astype(np.int32), want_details)
         res = np.zeros(n, RESULT_DTYPE)
         det = np.zeros((2, n), DETAIL_DTYPE) if want_details else None
         a = 0
@@ -631,13 +667,22 @@ class Engine:
             b = min(n, a + st.max_reads)
             b = min(b, int(np.searchsorted(off, off[a] + st.max_bytes, side="right")) - 1)
             b = max(b, a + 1)
-            out = st.classify(blob[off[a]:off[b]], (off[a:b + 1] - off[a]).astype(np.int32), want_details=want_details)
+            out = self._classify(blob[off[a]:off[b]], (off[a:b + 1] - off[a]).astype(np.int32), want_details)
             if want_details:
                 res[a:b], det[:, a:b] = out
             else:
                 res[a:b] = out
             a = b
         return (res, det) if want_details else res
+
+    def _classify(self, blob: np.ndarray, off: np.ndarray, want_details: bool):
+        """One batch that fits the stream: the whole reads (bdx_classify), or their window bytes."""
+        if not self.windows:
+            return self.stream.classify(blob, off, want_details=want_details)
+        win, win_off = self.config.window_reads(blob, off)
+        self.stream.submit_windows(win, win_off, off)
+        out = self.stream.fetch(want_details=want_details)
+        return out[1:] if want_details else out[1]
 
     def demux_stats(self):
         from .stats import stats_from_counters

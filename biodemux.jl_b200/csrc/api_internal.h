@@ -117,6 +117,11 @@ struct Slot {
     bdx_pass_detail *h_det = nullptr;
     uint8_t *d_packed = nullptr;  // 4-bit packed input of the batch (allocated on first packed submit)
     uint8_t *h_packed = nullptr;  // its pinned staging (bdx_submit_packed4 only)
+    // search-window input (windows.cu), allocated on the first windowed submit: the window bytes (packed windows
+    // use d_packed / h_packed, byte windows use h_seq as host staging) and the window stream's offsets
+    uint8_t *d_win = nullptr;
+    int32_t *d_win_off = nullptr;
+    int32_t *h_win_off = nullptr;
     uint8_t *d_seq = nullptr;
     int32_t *d_off = nullptr;
     bdx_result *d_res = nullptr;

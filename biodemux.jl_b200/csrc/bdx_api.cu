@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "api_internal.h"
+#include "literal.cuh"
 
 using namespace bdx;
 
@@ -380,6 +381,9 @@ extern "C" void bdx_stream_destroy(bdx_stream *s)
         cudaFreeHost(sl.h_det);
         cudaFree(sl.d_packed);
         cudaFreeHost(sl.h_packed);
+        cudaFree(sl.d_win);
+        cudaFree(sl.d_win_off);
+        cudaFreeHost(sl.h_win_off);
         cudaFree(sl.d_seq);
         cudaFree(sl.d_off);
         cudaFree(sl.d_res);
@@ -604,20 +608,29 @@ static int enqueue_batch(bdx_stream *s, Slot &sl)
     return bdx_enqueue_classify(s, sl.d_seq, sl.d_off, n, sl.d_res, det);
 }
 
-// h_seq: the batch's sequence bytes, or -- packed -- their 4-bit codes (packed.cu)
-static int launch_slot(bdx_stream *s, Slot &sl, const uint8_t *h_seq, const int32_t *h_off, bool packed = false)
+// h_seq: the batch's sequence bytes, or -- packed -- their 4-bit codes (packed.cu).  h_win_off set: h_seq holds the
+// batch's window bytes (or their codes) with these offsets, h_off those of the full reads (windows.cu).
+static int launch_slot(bdx_stream *s, Slot &sl, const uint8_t *h_seq, const int32_t *h_off, bool packed = false,
+                       const int32_t *h_win_off = nullptr)
 {
     CU(cudaSetDevice(s->device));
     const int32_t n = sl.n;
     const size_t bytes = n ? (size_t)h_off[n] : 0;
+    const bool windows = h_win_off != nullptr;
+    const size_t sent = !n ? 0 : windows ? (size_t)h_win_off[n] : bytes;     // bytes of the stream that travels
+    uint8_t *const d_in = packed ? sl.d_packed : windows ? sl.d_win : sl.d_seq;
     if (n) {
         CU(cudaMemcpyAsync(sl.d_off, h_off, ((size_t)n + 1) * 4, cudaMemcpyHostToDevice, s->st_copy));
-        if (bytes && !packed) CU(cudaMemcpyAsync(sl.d_seq, h_seq, bytes, cudaMemcpyHostToDevice, s->st_copy));
-        if (bytes && packed) CU(cudaMemcpyAsync(sl.d_packed, h_seq, (bytes + 1) / 2, cudaMemcpyHostToDevice, s->st_copy));
+        if (windows) CU(cudaMemcpyAsync(sl.d_win_off, h_win_off, ((size_t)n + 1) * 4, cudaMemcpyHostToDevice, s->st_copy));
+        if (sent) CU(cudaMemcpyAsync(d_in, h_seq, packed ? (sent + 1) / 2 : sent, cudaMemcpyHostToDevice, s->st_copy));
     }
     CU(cudaEventRecord(sl.ev_h2d, s->st_copy));
     CU(cudaStreamWaitEvent(s->st_comp, sl.ev_h2d, 0));
-    if (packed && bytes) {
+    if (windows && bytes) {
+        CU(launch_expand_windows(d_in, packed, sl.d_win_off, sl.d_off, sl.d_seq, n, (long long)bytes, s->tab->P,
+                                 s->cfg->rep_of, s->tab->sm_count, s->st_comp));
+        s->launches++;
+    } else if (packed && bytes) {
         CU(launch_unpack4(sl.d_packed, sl.d_seq, sl.d_off, n, (long long)bytes, s->cfg->rep_of, s->tab->sm_count, s->st_comp));
         s->launches++;
     }
@@ -780,6 +793,110 @@ extern "C" int bdx_submit_packed4(bdx_stream *s, const uint8_t *packed, const in
 extern "C" int bdx_submit_packed4_pinned(bdx_stream *s, const uint8_t *packed, const int32_t *offsets, int32_t n, uint64_t tag)
 {
     return submit_packed(s, packed, offsets, n, tag, true);
+}
+
+// ---- search-window input (windows.cu) ----
+extern "C" int bdx_window_spans(const bdx_config *cfg, int32_t read_len, int32_t spans[4])
+{
+    if (!cfg || !spans || read_len < 0) return fail(BDX_ERR_INVALID, "bad argument");
+    const DevParams P = host_params(*cfg, kSm100SmemOptin);
+    int sp[4];
+    const int len = read_windows(P, read_len, sp);
+    for (int k = 0; k < 4; k++) spans[k] = sp[k];
+    return len;
+}
+
+extern "C" int bdx_window_reads(const bdx_config *cfg, const uint8_t *seq, const int32_t *offsets, int32_t n,
+                                uint8_t *win, int32_t *win_off)
+{
+    if (!cfg || n < 0 || (n > 0 && (!offsets || !win_off || (win && !seq)))) return fail(BDX_ERR_INVALID, "bad argument");
+    if (n == 0) {
+        if (win_off) win_off[0] = 0;
+        return BDX_OK;
+    }
+    if (offsets[0] != 0) return fail(BDX_ERR_INVALID, "offsets[0] must be 0");
+    for (int32_t i = 0; i < n; i++)
+        if (offsets[i + 1] < offsets[i]) return fail(BDX_ERR_INVALID, "offsets must be non-decreasing");
+    const DevParams P = host_params(*cfg, kSm100SmemOptin);
+    int32_t w = 0, last_n = -1, len = 0;
+    int sp[4] = {};
+    win_off[0] = 0;
+    for (int32_t i = 0; i < n; i++) {
+        if (offsets[i + 1] - offsets[i] != last_n)       // the spans follow from the length: runs of equal lengths
+            len = read_windows(P, last_n = offsets[i + 1] - offsets[i], sp);
+        if (win) {
+            for (int k = 0; k < 4; k += 2)               // column c of read i is seq[offsets[i] + c - 1]
+                if (sp[k + 1] >= sp[k]) {
+                    memcpy(win + w, seq + offsets[i] + sp[k] - 1, (size_t)(sp[k + 1] - sp[k] + 1));
+                    w += sp[k + 1] - sp[k] + 1;
+                }
+        } else {
+            w += len;
+        }
+        win_off[i + 1] = w;
+    }
+    return BDX_OK;
+}
+
+static int ensure_window_buffers(bdx_stream *s, bool packed, bool host)
+{
+    int rc = packed ? ensure_packed_buffers(s, host) : host ? ensure_host_staging(s) : BDX_OK;
+    if (rc) return rc;
+    CU(cudaSetDevice(s->device));
+    for (Slot &sl : s->slot) {
+        if (!packed && !sl.d_win) CU(cudaMalloc(&sl.d_win, (size_t)std::max<int64_t>(s->max_bytes, 16)));
+        if (!sl.d_win_off) CU(cudaMalloc(&sl.d_win_off, ((size_t)s->max_reads + 1) * 4));
+        if (host && !sl.h_win_off) CU(cudaHostAlloc(&sl.h_win_off, ((size_t)s->max_reads + 1) * 4, cudaHostAllocDefault));
+    }
+    return BDX_OK;
+}
+
+static int submit_windows(bdx_stream *s, const uint8_t *win, const int32_t *win_off, const int32_t *offsets, int32_t n,
+                          int packed, uint64_t tag, bool pinned)
+{
+    if (!s || (n > 0 && (!offsets || !win_off))) return fail(BDX_ERR_INVALID, "null argument");
+    if (packed && !s->cfg->n_codes) return fail(BDX_ERR_INVALID, "more than 15 distinct barcode bytes: no 4-bit packed input for this config");
+    if (s->max_reads <= 0) return fail(BDX_ERR_STATE, "stream has no staging (max_reads = 0)");
+    if (s->acquired) return fail(BDX_ERR_STATE, "bdx_acquire pending; call bdx_commit");
+    if (s->in_flight >= BDX_MAX_IN_FLIGHT) return fail(BDX_ERR_STATE, "BDX_MAX_IN_FLIGHT batches already in flight; call bdx_fetch");
+    int rc = check_batch(s, offsets, n);
+    if (rc) return rc;
+    // the device trusts win_off: every read's window length is checked against the rule here
+    if (n && win_off[0] != 0) return fail(BDX_ERR_INVALID, "win_offsets[0] must be 0");
+    const DevParams &P = s->tab->P;
+    int32_t last_n = -1, len = 0;
+    for (int32_t i = 0; i < n; i++) {
+        int sp[4];
+        if (offsets[i + 1] - offsets[i] != last_n) len = read_windows(P, last_n = offsets[i + 1] - offsets[i], sp);
+        if (win_off[i + 1] - win_off[i] != len)
+            return fail(BDX_ERR_INVALID, "win_offsets do not match the search windows of the read lengths (first bad read: " +
+                                         std::to_string(i) + ")");
+    }
+    if (n && win_off[n] > 0 && !win) return fail(BDX_ERR_INVALID, "null argument");
+    if ((rc = ensure_window_buffers(s, packed != 0, !pinned))) return rc;
+    Slot &sl = s->slot[s->head];
+    sl.n = n;
+    sl.tag = tag;
+    if (pinned) return launch_slot(s, sl, win, offsets, packed != 0, win_off);
+    uint8_t *const h_in = packed ? sl.h_packed : sl.h_seq;
+    if (n) {
+        memcpy(sl.h_off, offsets, ((size_t)n + 1) * 4);
+        memcpy(sl.h_win_off, win_off, ((size_t)n + 1) * 4);
+        if (win_off[n]) memcpy(h_in, win, packed ? ((size_t)win_off[n] + 1) / 2 : (size_t)win_off[n]);
+    }
+    return launch_slot(s, sl, h_in, sl.h_off, packed != 0, sl.h_win_off);
+}
+
+extern "C" int bdx_submit_windows(bdx_stream *s, const uint8_t *win, const int32_t *win_offsets, const int32_t *offsets,
+                                  int32_t n_reads, int packed4, uint64_t tag)
+{
+    return submit_windows(s, win, win_offsets, offsets, n_reads, packed4, tag, false);
+}
+
+extern "C" int bdx_submit_windows_pinned(bdx_stream *s, const uint8_t *win, const int32_t *win_offsets,
+                                         const int32_t *offsets, int32_t n_reads, int packed4, uint64_t tag)
+{
+    return submit_windows(s, win, win_offsets, offsets, n_reads, packed4, tag, true);
 }
 
 extern "C" int bdx_acquire(bdx_stream *s, uint8_t **seq, int32_t **offsets)

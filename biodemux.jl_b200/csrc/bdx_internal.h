@@ -218,6 +218,10 @@ cudaError_t launch_finalize(const DevParams &P, const int *off, int n, const Scr
                             bdx_result *res, bdx_pass_detail *det, StatsDev stats, cudaStream_t st);
 cudaError_t launch_unpack4(const uint8_t *d_packed, uint8_t *d_seq, const int *d_off, int n_reads, long long max_bytes,
                            const uint8_t rep[16], int sm_count, cudaStream_t st);
+// search-window input (windows.cu): window bytes (or their 4-bit codes) -> the batch's full-length sequence buffer
+cudaError_t launch_expand_windows(const uint8_t *d_win, bool packed, const int *d_win_off, const int *d_off,
+                                  uint8_t *d_seq, int n_reads, long long bytes, const DevParams &P, const uint8_t rep[16],
+                                  int sm_count, cudaStream_t st);
 cudaError_t launch_synth(const DevParams &P, const bdx_synth_spec &spec, int n, uint8_t *seq, int *off,
                          cudaStream_t st);
 cudaError_t run_int_alu_peak(int device, double *ops_per_second);

@@ -10,6 +10,8 @@
 // by 2^20 and barcode length by 256, so no cell exceeds 2^29 = kInf.
 #pragma once
 
+#include <math_constants.h>
+
 #include "bdx_internal.h"
 
 namespace bdx {
@@ -31,7 +33,7 @@ __device__ __forceinline__ int allowed_from(double max_error, int norm)
 }
 
 // resolve(dr, len)  (classification.jl:96-100) with Julia's UnitRange normalisation
-__device__ __forceinline__ void resolve_range(const DevRange &dr, int len, int &first, int &last)
+__host__ __device__ __forceinline__ void resolve_range(const DevRange &dr, int len, int &first, int &last)
 {
     int s = dr.start_from_end ? len + dr.start_off : dr.start_off;
     int e = dr.end_from_end ? len + dr.end_off : dr.end_off;
@@ -46,7 +48,7 @@ struct Geometry {
 };
 
 // match_barcode_pass range prologue (classification.jl:795-807)
-__device__ __forceinline__ Geometry pass_geometry(const DevSet &S, int n)
+__host__ __device__ __forceinline__ Geometry pass_geometry(const DevSet &S, int n)
 {
     int rf, rl, bf, bl, ef, el;
     resolve_range(S.rs, n, rf, rl);
@@ -59,6 +61,37 @@ __device__ __forceinline__ Geometry pass_geometry(const DevSet &S, int n)
     g.min_end_pos = ef;
     g.valid = !(g.start_j > g.end_j || g.start_j > g.max_start_pos || g.end_j < g.min_end_pos);
     return g;
+}
+
+// The columns of a read of length n that a classification can depend on (bdx_submit_windows): per pass that runs,
+// :semiglobal [start_j, end_j] (sg_literal reads no other column); :hamming / :exact [start_j, last + max_m - 1]
+// with last = min(end_j, max_start_pos), the furthest column a start position's comparison reaches.  exact_literal
+// may scan beyond, but an occurrence it finds outside the window gives kInf whatever the bytes are (findprev:
+// every start in [first, last] is tried before any start < first; findnext: every one before any > last).
+// sp = lo1, hi1, lo2, hi2 (1-based, inclusive, hi < lo = empty), sorted and merged when they overlap or touch.
+// Returns the number of window columns.
+__host__ __device__ __forceinline__ int read_windows(const DevParams &P, int n, int sp[4])
+{
+    int lo[2] = {1, 1}, hi[2] = {0, 0};
+    for (int p = 0; p < (P.is_dual ? 2 : 1); p++) {
+        const DevSet &S = P.set[p];
+        const Geometry g = pass_geometry(S, n);
+        if (!g.valid) continue;
+        lo[p] = g.start_j;
+        hi[p] = P.algo == BDX_SEMIGLOBAL ? g.end_j : min(n, min(g.end_j, g.max_start_pos) + S.max_m - 1);
+        if (hi[p] < lo[p]) lo[p] = 1, hi[p] = 0;
+    }
+    const bool e0 = hi[0] < lo[0], e1 = hi[1] < lo[1];
+    if (e0 || (!e1 && lo[1] < lo[0])) {          // the non-empty / leftmost span first
+        int t = lo[0]; lo[0] = lo[1]; lo[1] = t;
+        t = hi[0]; hi[0] = hi[1]; hi[1] = t;
+    }
+    if (hi[1] >= lo[1] && lo[1] <= hi[0] + 1) {  // overlapping or touching: one span
+        hi[0] = max(hi[0], hi[1]);
+        lo[1] = 1, hi[1] = 0;
+    }
+    sp[0] = lo[0], sp[1] = hi[0], sp[2] = lo[1], sp[3] = hi[1];
+    return max(0, hi[0] - lo[0] + 1) + max(0, hi[1] - lo[1] + 1);
 }
 
 // semiglobal_alignment_core (classification.jl:238-445).  q1 / r1 are 1-based

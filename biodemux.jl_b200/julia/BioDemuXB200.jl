@@ -132,17 +132,19 @@ function filename_of(c::DemuxConfig, r::BdxResult)
 end
 
 """
-    gpu_worker_task(input_channel, output_channel, gcfg; device=0, chunk_size=4000, max_read_len=1024)
+    gpu_worker_task(input_channel, output_channel, gcfg; device=0, chunk_size=4000, max_read_len=1024, windows=false)
 
 Drop-in for `BioDemuX.worker_task` (core.jl:226-279).  One bdx_stream per worker task; up to three batches are
 kept in flight so H2D copies overlap the kernels.  The stream's pinned staging holds `chunk_size` reads /
 `chunk_size * max_read_len` sequence bytes per batch: a chunk that does not fit (long reads, or a reader chunk
 larger than the worker's) is split into several batches -- nothing is ever written past the staging buffers --
-and only a single read longer than the whole staging buffer is an error (raise `max_read_len`).  Returns the
-stream's DemuxStats (from the device counters) when `config.summary`, else `nothing`.
+and only a single read longer than the whole staging buffer is an error (raise `max_read_len`).  With
+`windows=true` only the bytes of every read's search windows travel (`bdx_submit_windows`; same results): the gain
+of long reads with short search ranges.  Returns the stream's DemuxStats (from the device counters) when
+`config.summary`, else `nothing`.
 """
 function gpu_worker_task(input_channel::Channel{Chunk}, output_channel::Channel{ResultChunk}, g::GpuConfig;
-                         device::Int=0, chunk_size::Int=4000, max_read_len::Int=1024)
+                         device::Int=0, chunk_size::Int=4000, max_read_len::Int=1024, windows::Bool=false)
     c = g.config
     max_bytes = chunk_size * max_read_len
     sref = Ref{Ptr{Cvoid}}(C_NULL)
@@ -200,6 +202,11 @@ function gpu_worker_task(input_channel::Channel{Chunk}, output_channel::Channel{
                 while length(in_flight) >= 3                 # BDX_MAX_IN_FLIGHT is 4
                     finish_oldest()
                 end
+                if windows
+                    submit_windows(s, g, seqs, rng, chunk.id)
+                    push!(in_flight, (length(pending), rng))
+                    continue
+                end
                 # zero-copy: write straight into the stream's pinned staging (bounds established above)
                 pseq = Ref{Ptr{UInt8}}(C_NULL); poff = Ref{Ptr{Int32}}(C_NULL)
                 check(ccall((:bdx_acquire, libbdx), Cint, (Ptr{Cvoid}, Ref{Ptr{UInt8}}, Ref{Ptr{Int32}}), s, pseq, poff))
@@ -226,6 +233,34 @@ function gpu_worker_task(input_channel::Channel{Chunk}, output_channel::Channel{
     finally
         ccall((:bdx_stream_destroy, libbdx), Cvoid, (Ptr{Cvoid},), s)
     end
+end
+
+"bdx_window_spans: ([lo1, hi1, lo2, hi2], window length) of a read of `len` bases (1-based, inclusive; hi < lo = empty)."
+function window_spans(g::GpuConfig, len::Integer)
+    sp = zeros(Int32, 4)
+    n = ccall((:bdx_window_spans, libbdx), Cint, (Ptr{Cvoid}, Int32, Ptr{Int32}), g.handle, len, sp)
+    n < 0 && error("libbdx: " * bdx_error())
+    return sp, Int(n)
+end
+
+"One batch as the reads' window bytes (bdx_submit_windows; the library copies them to its staging before returning)."
+function submit_windows(s::Ptr{Cvoid}, g::GpuConfig, seqs::Vector{String}, rng::UnitRange{Int}, tag)
+    off = zeros(Int32, length(rng) + 1)
+    woff = zeros(Int32, length(rng) + 1)
+    win = UInt8[]
+    spans = Dict{Int,Tuple{Vector{Int32},Int}}()      # the spans follow from the length alone
+    for (k, i) in enumerate(rng)
+        cu = codeunits(seqs[i])
+        sp, wl = get!(() -> window_spans(g, length(cu)), spans, length(cu))
+        for j in (1, 3)
+            sp[j+1] >= sp[j] && append!(win, view(cu, sp[j]:sp[j+1]))
+        end
+        off[k+1] = off[k] + length(cu)
+        woff[k+1] = woff[k] + wl
+    end
+    check(ccall((:bdx_submit_windows, libbdx), Cint,
+                (Ptr{Cvoid}, Ptr{UInt8}, Ptr{Int32}, Ptr{Int32}, Int32, Cint, UInt64),
+                s, win, woff, off, length(rng), 0, tag))
 end
 
 "Device counters -> DemuxStats (classification.jl:736-767); score keys are round(dist / norm, digits=2)."

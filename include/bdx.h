@@ -198,6 +198,31 @@ int bdx_submit_packed4(bdx_stream *s, const uint8_t *packed, const int32_t *offs
 int bdx_submit_packed4_pinned(bdx_stream *s, const uint8_t *packed, const int32_t *offsets, int32_t n_reads,
                               uint64_t tag);
 
+/* ---- search-window input: only the read columns the passes can look at ------------------------------------------
+ * A classification depends on a read's length and on its bytes in at most two spans of columns, computed from the
+ * length alone: per pass, :semiglobal [start, end] of the resolved search range; :hamming / :exact from its start to
+ * min(end, last barcode start) + longest barcode - 1.  A read's "window bytes" are its bytes in those spans, in
+ * column order.  Sending them instead of the whole read gives identical results, details and DemuxStats; for long
+ * reads with short search ranges it is a small fraction of the bytes.
+ * bdx_window_spans: the spans of a read of read_len bases -- lo1, hi1, lo2, hi2 (1-based, inclusive; hi < lo = empty;
+ * sorted, merged when they overlap or touch) -- and, as the return value, their total length (< 0: error).
+ * bdx_window_reads: the window bytes of a batch (concatenated; win_bytes may be NULL to size the output first) and
+ * their offsets win_offsets (n_reads + 1 entries).  offsets are the full reads'.  Both are host-only, thread-safe and
+ * need no CUDA device. */
+int bdx_window_spans(const bdx_config *cfg, int32_t read_len, int32_t spans[4]);
+int bdx_window_reads(const bdx_config *cfg, const uint8_t *seq_bytes, const int32_t *offsets, int32_t n_reads,
+                     uint8_t *win_bytes, int32_t *win_offsets);
+/* Queue one batch given as window bytes: win / win_offsets as bdx_window_reads makes them, offsets those of the FULL
+ * reads exactly as for bdx_submit (max_bytes bounds the full bytes: the device rebuilds them).  packed4 != 0: win is
+ * the window stream packed by bdx_pack_reads4 (nibble k = window byte k; win_offsets still count unpacked bytes;
+ * BDX_ERR_INVALID when the config has more than 15 distinct barcode bytes).  Before anything is enqueued every
+ * read's window length is checked against its length: a mismatch is BDX_ERR_INVALID.  Fetch as usual. */
+int bdx_submit_windows(bdx_stream *s, const uint8_t *win, const int32_t *win_offsets, const int32_t *offsets,
+                       int32_t n_reads, int packed4, uint64_t tag);
+/* like bdx_submit_pinned: win / win_offsets / offsets are page-locked and stay untouched until the batch is fetched */
+int bdx_submit_windows_pinned(bdx_stream *s, const uint8_t *win, const int32_t *win_offsets, const int32_t *offsets,
+                              int32_t n_reads, int packed4, uint64_t tag);
+
 /* Per-pass details are copied back only when enabled (default: on iff want_stats). */
 int bdx_stream_enable_details(bdx_stream *s, int on);
 
