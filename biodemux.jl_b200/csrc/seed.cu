@@ -42,6 +42,14 @@
 
 namespace bdx {
 
+// the reference's acceptance of a barcode at distance d (classification.jl:254, :658, :696): the DP allows d
+// (floor(fl(thr * norm))) and the score passes (fl(d / norm) <= thr).  Near the threshold either check can fail
+// while the other passes.
+__device__ __forceinline__ bool seed_accepts(int d, int norm, double max_error_rate)
+{
+    return d <= allowed_from(max_error_rate, norm) && __ddiv_rn((double)d, (double)norm) <= max_error_rate;
+}
+
 // TAB_SMEM: the CSR bucket table (bstart / entries / ekeys) is copied to shared memory; large sets read it
 // from global memory instead (it is touched only on first-level bitmap hits).
 template <bool TAB_SMEM, int W>      // W: 32-bit words per barcode row vector (1: up to 32 nt, 2: up to 64)
@@ -263,12 +271,14 @@ k_seed(const __grid_constant__ DevParams P, const int pass, const int level, con
                     bool decided = true, ambiguous = false;
                     if (with_delta) {
                         // delta = second-best score - best score (:711).  Every barcode within K edits is known
-                        // exactly; an unseen runner-up is more than K edits away (or not acceptable at all)
-                        const int allowed0 = S.allowed0[0];
+                        // exactly; an unseen runner-up is more than K edits away.  A runner-up counts only if the
+                        // reference accepts it (:696): both checks pass, as for the best.  With one common length
+                        // both are monotone in the distance, so when the nearest one fails, every farther one
+                        // fails too and sub_min stays Inf
                         if (second_d <= K) {
                             const double sc2 = __ddiv_rn((double)second_d, (double)norm);
-                            ambiguous = __dsub_rn(sc2, sc) < P.min_delta;
-                        } else if (K + 1 <= allowed0) {
+                            ambiguous = seed_accepts(second_d, norm, P.max_error_rate) && __dsub_rn(sc2, sc) < P.min_delta;
+                        } else if (seed_accepts(K + 1, norm, P.max_error_rate)) {
                             const double sc2 = __ddiv_rn((double)(K + 1), (double)norm);
                             decided = !(__dsub_rn(sc2, sc) < P.min_delta);      // safe whatever the runner-up is
                         }

@@ -631,6 +631,12 @@ int bdx_build_set(const bdx_params &p, const bdx_barcode_set &in, HostSet &hs, u
         // hamming: m (:567, :607)
         hs.norm[b] = (p.algorithm == BDX_SEMIGLOBAL && p.has_nindel) ? in.lengths_no_n[b] : m;
         if (hs.norm[b] < 0) return bdx_fail(BDX_ERR_INVALID, std::string(name) + ": negative lengths_no_n");
+        // floor(Int, max_error_rate * norm) (classification.jl:254, :567) raises InexactError unless the product is a
+        // number whose floor fits Int64: refused here for every barcode, as the reference would fail on its first read
+        volatile double prod = p.max_error_rate * (double)hs.norm[b];
+        if (p.algorithm != BDX_EXACT && !(prod >= -9223372036854775808.0 && prod < 9223372036854775808.0))
+            return bdx_fail(BDX_ERR_INVALID, std::string(name) + ": max_error_rate * length outside Int64 (the reference "
+                                                             "raises InexactError on floor(Int, max_error_rate * length))");
     }
     int min_m = hs.max_m;
     for (int b = 0; b < hs.n_bc; b++) min_m = std::min(min_m, hs.off[b + 1] - hs.off[b]);

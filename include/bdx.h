@@ -128,7 +128,10 @@ int bdx_device_count(void);
 /* Copies everything it needs; the caller keeps ownership of its buffers.
  * Validation mirrors the reference (trim_side in {0,3,5}); additionally rejects
  * what the device encoding cannot express: empty barcodes, zero gap costs
- * (Julia raises DivideError), |cost| > 2^20, more than 65535 barcodes per set. */
+ * (Julia raises DivideError), for :semiglobal and :hamming a max_error_rate
+ * whose product with a barcode's length is infinite or outside Int64 (Julia
+ * raises InexactError on floor(Int, max_error_rate * length)),
+ * |cost| > 2^20, more than 65535 barcodes per set. */
 int bdx_config_create(const bdx_params *params, bdx_config **out);
 void bdx_config_destroy(bdx_config *cfg);
 

@@ -30,8 +30,9 @@ def run_cuda(cfg, reads, want_stats=False, details=True, debug=0):
     return out, None, counters, layout
 
 
-def compare(cfg, reads, want_stats=False, label=""):
-    res, det, counters, layout = run_cuda(cfg, reads, want_stats=want_stats)
+def compare(cfg, reads, want_stats=False, label="", debug=0):
+    """debug: BDX_DEBUG_* flags of the CUDA run (single pipeline stages switched off)."""
+    res, det, counters, layout = run_cuda(cfg, reads, want_stats=want_stats, debug=debug)
     ref = orc.Oracle(cfg, want_stats=want_stats).classify_reads(reads)
     n = len(reads)
     for f in ("status", "bc1", "bc2", "keep_start", "keep_end"):
