@@ -24,44 +24,27 @@ std::string &bdx_error_text();
     } while (0)
 
 // ---- configuration ----
+// The host vectors of one barcode set's tables (tables.cu), each uploaded per device into the DevSet pointer that
+// get_tables (bdx_api.cu) pairs it with.  The set's scalars -- sizes, seed lengths, depths, which stages exist -- are
+// kept only in its DevSet, bdx_config::base.set[s].  A level that is not built has empty vectors.
 struct HostSet {
-    int n_bc = 0, n_bc_pad = 0, max_m = 0, trim_side = 0, words = 0, n_classes = 1, use_filter = 0;
-    DevRange rs{}, bs{}, be{};
-    std::vector<uint8_t> bytes;
+    int min_m = 0;                       // shortest barcode
+    std::vector<uint8_t> bytes, class_of, bc_cls;
     std::vector<int> off, norm, filt_allowed, allowed0;
     std::vector<uint32_t> peq;
-    uint8_t class_of[256];
-    // perfect-occurrence prefilter
-    int pf_enabled = 0, pf_seed = 0, pf_log2 = 0, pf_bm_log2 = 0;
-    std::vector<uint32_t> pf_bitmap;
-    uint32_t pf_pow = 0;
-    std::vector<uint32_t> pf_keys, pf_vals;
-    std::vector<uint8_t> bc_cls;
-    // :semiglobal depth-limited seeds
-    // :hamming packed scan (hamming.cu)
-    int hp_enabled = 0, hp_m = 0, hp_allowed = 0, hp_n_seg = 0;
-    int hp_off[8] = {}, hp_q[8] = {}, hp_base[8] = {};
-    std::vector<uint16_t> hp_bstart, hp_entries;
-    std::vector<uint2> hp_bcw;
+    std::vector<uint32_t> pf_bitmap, pf_keys, pf_vals;   // perfect-occurrence prefilter
     struct HostSeedLevel {
-        int k = 0, q = 0, log2 = 0, bm_log2 = 0, max_hits = 0;
-        uint32_t pow = 0;
         std::vector<uint32_t> bstart, entries, ekeys, bitmap;
     };
-    int sd_levels = 0, sd_m = 0;
-    HostSeedLevel sd[2];
-    int sdd_n = 0, sdd_k = 0;      // deepest level (seed_deep.cu): one table per seed length
-    HostSeedLevel sdd[2];
-    // variable lengths / constrained geometries (seed_var.cu)
+    HostSeedLevel sd[2], sdd[2];         // k_seed levels (seed.cu), k_seed_deep tables (seed_deep.cu)
     struct HostSeedVar {
-        int q = 0, q2 = 0, complete = 0, group_reads = 0, hit_rows = 0, qgram_filter = 0;
-        double sigma_min = 0.0;
         std::vector<uint16_t> bstart;
         std::vector<uint32_t> entries;
         std::vector<uint8_t> kdepth;
     };
-    int sv_levels = 0;
-    HostSeedVar sv[2];
+    HostSeedVar sv[2];                   // k_seed_var levels (seed_var.cu)
+    std::vector<uint16_t> hp_bstart, hp_entries;   // k_hamming_scan (hamming.cu)
+    std::vector<uint2> hp_bcw;
 };
 
 // ---- the kernel sequence of a pass (plan.cu) ----
@@ -98,16 +81,18 @@ struct bdx_config {
     int n_codes = 0;     // codes incl. 0; 0 = more than 15 distinct barcode bytes, packed input unavailable
     uint8_t code_of[256] = {};
     uint8_t rep_of[16] = {};
-    DevParams base{};  // device pointers unset
+    DevParams base{};  // every scalar of the config and its sets; device pointers unset
     HostSet set[2];
     bdx_stats_layout lay{};
     std::mutex mu;
     std::map<int, DeviceTables *> per_device;
 };
 
-// Validates one barcode set and builds its host-side tables (tables.cu).  debug: BDX_DEBUG_* switches.
-int bdx_build_set(const bdx_params &p, const bdx_barcode_set &in, HostSet &hs, uint32_t debug, const char *name);
-std::string bdx_describe_set(const HostSet &hs);   // tables.cu: text description for bdx_config_describe
+// Validates one barcode set and builds its tables (tables.cu): the scalars into D, the vectors into hs.
+// debug: BDX_DEBUG_* switches.
+int bdx_build_set(const bdx_params &p, const bdx_barcode_set &in, HostSet &hs, DevSet &D, uint32_t debug,
+                  const char *name);
+std::string bdx_describe_set(const HostSet &hs, const DevSet &D);   // tables.cu: text for bdx_config_describe
 
 // ---- streams ----
 struct Slot {

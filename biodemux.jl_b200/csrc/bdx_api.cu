@@ -69,8 +69,9 @@ extern "C" int bdx_config_create_debug(const bdx_params *p, uint32_t debug, bdx_
     bdx_config *cfg = new (std::nothrow) bdx_config();
     if (!cfg) return fail(BDX_ERR_NOMEM, "out of memory");
     cfg->debug = debug;
-    int rc = bdx_build_set(*p, p->set1, cfg->set[0], debug, "set1");
-    if (rc == BDX_OK && p->is_dual) rc = bdx_build_set(*p, p->set2, cfg->set[1], debug, "set2");
+    DevParams &P = cfg->base;
+    int rc = bdx_build_set(*p, p->set1, cfg->set[0], P.set[0], debug, "set1");
+    if (rc == BDX_OK && p->is_dual) rc = bdx_build_set(*p, p->set2, cfg->set[1], P.set[1], debug, "set2");
     if (rc != BDX_OK) {
         delete cfg;
         return rc;
@@ -97,7 +98,6 @@ extern "C" int bdx_config_create_debug(const bdx_params *p, uint32_t debug, bdx_
                 break;
             }
     }
-    DevParams &P = cfg->base;
     P.max_error_rate = p->max_error_rate;
     P.min_delta = p->min_delta;
     P.match = (int)p->match;
@@ -114,11 +114,11 @@ extern "C" int bdx_config_create_debug(const bdx_params *p, uint32_t debug, bdx_
 
     // stats layout (classification.jl:736-758)
     bdx_stats_layout &L = cfg->lay;
-    const int b1 = cfg->set[0].n_bc, b2 = p->is_dual ? cfg->set[1].n_bc : 0;
-    const int max_m = std::max(cfg->set[0].max_m, p->is_dual ? cfg->set[1].max_m : 0);
+    const int b1 = P.set[0].n_bc, b2 = p->is_dual ? P.set[1].n_bc : 0;
+    const int max_m = std::max(P.set[0].max_m, p->is_dual ? P.set[1].max_m : 0);
     int max_allowed = 0;
     for (int s = 0; s < (p->is_dual ? 2 : 1); s++)
-        for (int b = 0; b < cfg->set[s].n_bc; b++) max_allowed = std::max(max_allowed, cfg->set[s].allowed0[b]);
+        for (int b = 0; b < P.set[s].n_bc; b++) max_allowed = std::max(max_allowed, cfg->set[s].allowed0[b]);
     L.b1 = b1;
     L.b2 = b2;
     L.pos_bias = max_m;
@@ -182,65 +182,8 @@ constexpr size_t kSm100SmemOptin = 232448;
 static DevParams host_params(const bdx_config &cfg, size_t smem_optin)
 {
     DevParams P = cfg.base;
-    auto level = [](const HostSet::HostSeedLevel &H, SeedLevel &L) {
-        L.k = H.k;
-        L.q = H.q;
-        L.pow = H.pow;
-        L.log2 = H.log2;
-        L.bm_log2 = H.bm_log2;
-        L.max_hits = H.max_hits;
-        L.n_entries = (int)H.entries.size();
-    };
     for (int s = 0; s < (P.is_dual ? 2 : 1); s++) {
-        const HostSet &hs = cfg.set[s];
         DevSet &D = P.set[s];
-        D.n_bc = hs.n_bc;
-        D.n_bc_pad = hs.n_bc_pad;
-        D.max_m = hs.max_m;
-        D.trim_side = hs.trim_side;
-        D.words = hs.words;
-        D.use_filter = hs.use_filter;
-        D.n_classes = hs.n_classes;
-        D.rs = hs.rs;
-        D.bs = hs.bs;
-        D.be = hs.be;
-        D.pf_enabled = hs.pf_enabled;
-        D.pf_seed = hs.pf_seed;
-        D.pf_pow = hs.pf_pow;
-        D.pf_log2 = hs.pf_log2;
-        D.pf_bm_log2 = hs.pf_bm_log2;
-        D.sd_levels = hs.sd_levels;
-        D.sd_m = hs.sd_m;
-        for (int l = 0; l < hs.sd_levels; l++) level(hs.sd[l], D.sd[l]);
-        D.sdd_n = hs.sdd_n;
-        D.sdd_k = hs.sdd_k;
-        for (int l = 0; l < hs.sdd_n; l++) level(hs.sdd[l], D.sdd[l]);
-        D.sv_levels = hs.sv_levels;
-        for (int l = 0; l < hs.sv_levels; l++) {
-            const HostSet::HostSeedVar &H = hs.sv[l];
-            SeedVar &V = D.sv[l];
-            V.enabled = 1;
-            V.q = H.q;
-            V.q2 = H.q2;
-            V.bstart2 = (1 << (2 * H.q)) + 1;
-            V.n_bstart = (int)H.bstart.size();
-            V.n_entries = (int)H.entries.size();
-            V.complete = H.complete;
-            V.group_reads = H.group_reads;
-            V.hit_rows = H.hit_rows;
-            V.qgram_filter = H.qgram_filter;
-            V.sigma_min = H.sigma_min;
-        }
-        D.hp.enabled = hs.hp_enabled;
-        D.hp.m = hs.hp_m;
-        D.hp.allowed = hs.hp_allowed;
-        D.hp.n_seg = hs.hp_n_seg;
-        D.hp.n_bstart = (int)hs.hp_bstart.size();
-        for (int k = 0; k < 8; k++) {
-            D.hp.seg_off[k] = hs.hp_off[k];
-            D.hp.seg_q[k] = hs.hp_q[k];
-            D.hp.seg_base[k] = hs.hp_base[k];
-        }
         // shared-memory footprints against the opt-in limit: the prefilter's hash table and bitmap (large sets of
         // short barcodes), then the filter kernel's Peq planes
         if (D.pf_enabled && prefilter_smem_bytes(D) > smem_optin) {
@@ -277,41 +220,46 @@ static int get_tables(bdx_config *cfg, int device, DeviceTables **out)
     t->P = host_params(*cfg, prop.sharedMemPerBlockOptin);
     t->sm_count = prop.multiProcessorCount;
     const int passes = t->P.is_dual ? 2 : 1;
+    // every table of a set, paired with the DevSet pointer its device copy goes to; a level that was not built has
+    // empty vectors and keeps a null pointer.  Nothing is uploaded after the first error.
+    cudaError_t e = cudaSuccess;
+    auto up = [&](const auto &v, auto &dev) {
+        if (e == cudaSuccess) e = upload(t, v, &dev);
+    };
     for (int s = 0; s < passes; s++) {
         const HostSet &hs = cfg->set[s];
         DevSet &D = t->P.set[s];
-        std::vector<uint8_t> cls(hs.class_of, hs.class_of + 256);
-        cudaError_t e = upload(t, hs.bytes, &D.bc_bytes);
-        if (e == cudaSuccess) e = upload(t, hs.off, &D.bc_off);
-        if (e == cudaSuccess) e = upload(t, hs.norm, &D.norm);
-        if (e == cudaSuccess) e = upload(t, hs.peq, &D.peq);
-        if (e == cudaSuccess) e = upload(t, hs.filt_allowed, &D.filt_allowed);
-        if (e == cudaSuccess) e = upload(t, hs.allowed0, &D.allowed0);
-        if (e == cudaSuccess) e = upload(t, cls, &D.class_of);
-        if (e == cudaSuccess) e = upload(t, hs.pf_bitmap, &D.pf_bitmap);
-        if (e == cudaSuccess) e = upload(t, hs.pf_keys, &D.pf_keys);
-        if (e == cudaSuccess) e = upload(t, hs.pf_vals, &D.pf_vals);
-        if (e == cudaSuccess) e = upload(t, hs.bc_cls, &D.bc_cls);
+        up(hs.bytes, D.bc_bytes);
+        up(hs.off, D.bc_off);
+        up(hs.norm, D.norm);
+        up(hs.peq, D.peq);
+        up(hs.filt_allowed, D.filt_allowed);
+        up(hs.allowed0, D.allowed0);
+        up(hs.class_of, D.class_of);
+        up(hs.pf_bitmap, D.pf_bitmap);
+        up(hs.pf_keys, D.pf_keys);
+        up(hs.pf_vals, D.pf_vals);
+        up(hs.bc_cls, D.bc_cls);
         auto level = [&](const HostSet::HostSeedLevel &H, SeedLevel &L) {
-            if (e == cudaSuccess) e = upload(t, H.bstart, &L.bstart);
-            if (e == cudaSuccess) e = upload(t, H.entries, &L.entries);
-            if (e == cudaSuccess) e = upload(t, H.ekeys, &L.ekeys);
-            if (e == cudaSuccess) e = upload(t, H.bitmap, &L.bitmap);
+            up(H.bstart, L.bstart);
+            up(H.entries, L.entries);
+            up(H.ekeys, L.ekeys);
+            up(H.bitmap, L.bitmap);
         };
-        for (int l = 0; l < hs.sd_levels; l++) level(hs.sd[l], D.sd[l]);
-        for (int l = 0; l < hs.sdd_n; l++) level(hs.sdd[l], D.sdd[l]);
-        for (int l = 0; l < hs.sv_levels; l++) {
-            if (e == cudaSuccess) e = upload(t, hs.sv[l].bstart, &D.sv[l].bstart);
-            if (e == cudaSuccess) e = upload(t, hs.sv[l].entries, &D.sv[l].entries);
-            if (e == cudaSuccess) e = upload(t, hs.sv[l].kdepth, &D.sv[l].kdepth);
+        for (int l = 0; l < 2; l++) level(hs.sd[l], D.sd[l]);
+        for (int l = 0; l < 2; l++) level(hs.sdd[l], D.sdd[l]);
+        for (int l = 0; l < 2; l++) {
+            up(hs.sv[l].bstart, D.sv[l].bstart);
+            up(hs.sv[l].entries, D.sv[l].entries);
+            up(hs.sv[l].kdepth, D.sv[l].kdepth);
         }
-        if (e == cudaSuccess) e = upload(t, hs.hp_bstart, &D.hp.bstart);
-        if (e == cudaSuccess) e = upload(t, hs.hp_entries, &D.hp.entries);
-        if (e == cudaSuccess) e = upload(t, hs.hp_bcw, &D.hp.bcw);
-        if (e != cudaSuccess) {
-            free_tables(t);
-            return cuda_fail(e, "uploading barcode tables");
-        }
+        up(hs.hp_bstart, D.hp.bstart);
+        up(hs.hp_entries, D.hp.entries);
+        up(hs.hp_bcw, D.hp.bcw);
+    }
+    if (e != cudaSuccess) {
+        free_tables(t);
+        return cuda_fail(e, "uploading barcode tables");
     }
     for (int pass = 0; pass < passes; pass++) t->plan[pass] = plan_pass(t->P, pass);
     cfg->per_device[device] = t;
@@ -733,8 +681,8 @@ extern "C" int bdx_config_describe(const bdx_config *cfg, int pass, char *buf, i
 {
     if (!cfg || pass < 0 || pass > 1 || len < 0 || (len > 0 && !buf)) return fail(BDX_ERR_INVALID, "bad argument");
     std::string text;
-    if (cfg->set[pass].n_bc)
-        text = bdx_describe_set(cfg->set[pass]) + "plan: steps=" +
+    if (cfg->base.set[pass].n_bc)
+        text = bdx_describe_set(cfg->set[pass], cfg->base.set[pass]) + "plan: steps=" +
                plan_text(plan_pass(host_params(*cfg, kSm100SmemOptin), pass)) + "\n";
     if (len > 0) {
         const size_t k = std::min(text.size(), (size_t)len - 1);

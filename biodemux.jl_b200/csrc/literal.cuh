@@ -24,9 +24,15 @@ struct Costs {
 // floor(Int, max_error * normalization_length)  (classification.jl:254, :567) as an
 // IEEE double multiply (no contraction), clamped to +-2^28 which is beyond any
 // reachable cell value and therefore indistinguishable from the unclamped Int64.
-__device__ __forceinline__ int allowed_from(double max_error, int norm)
+// The host (allowed0, tables.cu) must get the same value as every kernel.
+__host__ __device__ __forceinline__ int allowed_from(double max_error, int norm)
 {
+#ifdef __CUDA_ARCH__
     double x = floor(__dmul_rn(max_error, (double)norm));
+#else
+    volatile double prod = max_error * (double)norm;   // stored as a double: no fused multiply-add on the host
+    double x = floor(prod);
+#endif
     if (!(x < 268435456.0)) return 268435456;  // also catches NaN/Inf
     if (x < -268435456.0) return -268435456;
     return (int)x;

@@ -1,7 +1,8 @@
 // tables.cu -- host-side barcode tables of a bdx_config (built once per config, uploaded per device by
 // bdx_api.cu): the byte -> class map and the Peq match masks of the bit-parallel kernels, the hash table of
 // the perfect-occurrence prefilter, the seed tables of k_seed / k_seed_deep / k_seed_var and the bit planes of
-// the packed Hamming scan.  Pure host code.
+// the packed Hamming scan.  Pure host code.  Each builder writes its stage's scalars into the set's DevSet (the
+// config's base parameter block) and its vectors into the HostSet.
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
@@ -9,6 +10,7 @@
 #include <string>
 
 #include "api_internal.h"
+#include "literal.cuh"
 
 using namespace bdx;
 
@@ -24,62 +26,48 @@ static int narrow_range(const bdx_range &in, DevRange &out, const char *name)
     return BDX_OK;
 }
 
-static int host_allowed(double max_error, int norm)
-{
-    // floor(Int, max_error * normalization_length), classification.jl:254 (same clamp as the device)
-    volatile double prod = max_error * (double)norm;
-    double x = std::floor(prod);
-    if (!(x < 268435456.0)) return 268435456;
-    if (x < -268435456.0) return -268435456;
-    return (int)x;
-}
-
 namespace {
 
-// what the builders below share
-struct Build {
-    const bdx_params &p;
-    HostSet &hs;
-    uint32_t debug;
-    bool sg;          // :semiglobal
-    bool benign;      // costs for which the unit-cost filter is a superset filter (DESIGN.md)
-    int min_m;        // shortest barcode
-};
+// kPfBase^(q-1): the weight of a q-mer's first byte in its polynomial hash
+uint32_t hash_pow(int q)
+{
+    uint32_t pw = 1;
+    for (int i = 1; i < q; i++) pw *= kPfBase;
+    return pw;
+}
 
 // byte classes, Peq match masks and candidate thresholds of the bit-parallel kernels (filter.cu)
-void build_filter_tables(const Build &B)
+void build_filter_tables(const bdx_params &p, HostSet &hs, DevSet &D, uint32_t debug)
 {
-    const bdx_params &p = B.p;
-    HostSet &hs = B.hs;
-    const bool sg = B.sg, benign = B.benign;
-    const int min_m = B.min_m;
-    (void)p; (void)sg; (void)benign; (void)min_m;
+    const bool sg = p.algorithm == BDX_SEMIGLOBAL;
+    // costs for which the unit-cost filter is a superset filter (DESIGN.md)
+    const bool benign = p.match >= 0 && p.mismatch >= 1 && p.indel >= 1 && (!p.has_nindel || p.nindel >= p.indel);
     // ---- bit-parallel filter tables (semiglobal only) ----
-    const int groups = (hs.n_bc + 31) / 32;
+    const int groups = (D.n_bc + 31) / 32;
     int gpad = groups;
     if (groups > 4) {
         const int m3 = (groups + 2) / 3 * 3, m4 = (groups + 3) / 4 * 4;
         gpad = m4 <= m3 ? m4 : m3;
     }
-    hs.n_bc_pad = gpad * 32;
-    memset(hs.class_of, 0, sizeof(hs.class_of));
-    hs.n_classes = 1;
+    D.n_bc_pad = gpad * 32;
+    hs.class_of.assign(256, 0);
+    D.n_classes = 1;
     for (uint8_t c : hs.bytes)
-        if (!hs.class_of[c]) hs.class_of[c] = (uint8_t)hs.n_classes++;
-    hs.words = hs.max_m <= 32 ? 1 : (hs.max_m <= 32 * kMaxFilterWords ? 2 : 0);
+        if (!hs.class_of[c]) hs.class_of[c] = (uint8_t)D.n_classes++;
+    D.words = D.max_m <= 32 ? 1 : (D.max_m <= 32 * kMaxFilterWords ? 2 : 0);
     // The unit-cost filter is also a superset filter for :hamming (Hamming distance >= edit
     // distance; a barcode N is a wildcard there, classification.jl:597) and :exact (distance 0).
     // Tiny sets are cheaper to scan with the literal kernel than to spread over 32 lanes: they get the tables
     // (for the thread-per-read prefilter / seed kernels) but not the filter kernel.
-    if ((sg && !benign) || (B.debug & BDX_DEBUG_NO_FILTER) || hs.n_classes > 64) hs.words = 0;
-    hs.use_filter = hs.words > 0 && hs.n_bc >= 8;
+    if ((sg && !benign) || (debug & BDX_DEBUG_NO_FILTER) || D.n_classes > 64) D.words = 0;
+    D.use_filter = D.words > 0 && D.n_bc >= 8;
 
-    hs.allowed0.assign(hs.n_bc_pad, -1);
-    hs.filt_allowed.assign(hs.n_bc_pad, -1);
+    hs.allowed0.assign(D.n_bc_pad, -1);
+    hs.filt_allowed.assign(D.n_bc_pad, -1);
     int64_t min_cost = std::min(p.mismatch, p.indel);
     if (p.has_nindel) min_cost = std::min(min_cost, p.nindel);
-    for (int b = 0; b < hs.n_bc; b++) {
-        hs.allowed0[b] = host_allowed(p.max_error_rate, hs.norm[b]);
+    for (int b = 0; b < D.n_bc; b++) {
+        hs.allowed0[b] = allowed_from(p.max_error_rate, hs.norm[b]);
         if (p.algorithm == BDX_EXACT)
             hs.filt_allowed[b] = p.max_error_rate >= 0.0 ? 0 : -1;          // score 0.0 <= thr (:658, :696)
         else if (p.algorithm == BDX_HAMMING)
@@ -87,14 +75,14 @@ void build_filter_tables(const Build &B)
         else if (benign)
             hs.filt_allowed[b] = hs.allowed0[b] < 0 ? -1 : (int)(hs.allowed0[b] / min_cost);
     }
-    if (hs.words) {
-        const int W = hs.words;
-        const size_t plane = (size_t)hs.n_classes * hs.n_bc_pad;
+    if (D.words) {
+        const int W = D.words;
+        const size_t plane = (size_t)D.n_classes * D.n_bc_pad;
         hs.peq.assign((size_t)W * plane, 0u);
-        for (int b = 0; b < hs.n_bc_pad; b++) {
-            const int m = b < hs.n_bc ? hs.off[b + 1] - hs.off[b] : 0;
+        for (int b = 0; b < D.n_bc_pad; b++) {
+            const int m = b < D.n_bc ? hs.off[b + 1] - hs.off[b] : 0;
             const int first_row_bit = W * 32 - m;  // bit of barcode row 1; lower bits are phantom rows
-            for (int c = 0; c < hs.n_classes; c++) {
+            for (int c = 0; c < D.n_classes; c++) {
                 uint64_t v = first_row_bit >= 64 ? ~0ull : ((1ull << first_row_bit) - 1);  // phantom rows match
                 if (W == 1) v &= 0xFFFFFFFFull;
                 for (int i = 0; i < m; i++) {
@@ -103,45 +91,39 @@ void build_filter_tables(const Build &B)
                     const bool is_n = q == (uint8_t)'N' && ((sg && p.has_nindel) || p.algorithm == BDX_HAMMING);
                     if (is_n || (c != 0 && hs.class_of[q] == c)) v |= 1ull << (first_row_bit + i);
                 }
-                hs.peq[0 * plane + (size_t)c * hs.n_bc_pad + b] = (uint32_t)v;
-                if (W == 2) hs.peq[1 * plane + (size_t)c * hs.n_bc_pad + b] = (uint32_t)(v >> 32);
+                hs.peq[0 * plane + (size_t)c * D.n_bc_pad + b] = (uint32_t)v;
+                if (W == 2) hs.peq[1 * plane + (size_t)c * D.n_bc_pad + b] = (uint32_t)(v >> 32);
             }
         }
     }
 }
 
 // hash table of whole-barcode prefixes: k_prefilter (filter.cu)
-void build_prefilter(const Build &B)
+void build_prefilter(const bdx_params &p, HostSet &hs, DevSet &D, uint32_t debug)
 {
-    const bdx_params &p = B.p;
-    HostSet &hs = B.hs;
-    const bool sg = B.sg, benign = B.benign;
-    const int min_m = B.min_m;
-    (void)p; (void)sg; (void)benign; (void)min_m;
     // ---- perfect-occurrence prefilter table (semiglobal, no wildcard rows) ----
     hs.bc_cls.resize(hs.bytes.size());
     for (size_t k = 0; k < hs.bytes.size(); k++) hs.bc_cls[k] = hs.class_of[hs.bytes[k]];
+    const bool sg = p.algorithm == BDX_SEMIGLOBAL;
     const bool ex = p.algorithm == BDX_EXACT;   // :exact keeps duplicates (each index is a candidate)
     // :hamming treats every barcode N as a wildcard (classification.jl:597): no table then
     const bool hm = p.algorithm == BDX_HAMMING &&
                     std::find(hs.bytes.begin(), hs.bytes.end(), (uint8_t)'N') == hs.bytes.end();
-    if (hs.words && ((sg && !p.has_nindel) || ex || hm) && min_m >= kPfMinSeed && !(B.debug & BDX_DEBUG_NO_PREFILTER)) {
-        const int seed = std::min(min_m, kPfMaxSeed);
-        hs.pf_seed = seed;
-        uint32_t pw = 1;
-        for (int i = 1; i < seed; i++) pw *= kPfBase;
-        hs.pf_pow = pw;
+    if (D.words && ((sg && !p.has_nindel) || ex || hm) && hs.min_m >= kPfMinSeed && !(debug & BDX_DEBUG_NO_PREFILTER)) {
+        const int seed = std::min(hs.min_m, kPfMaxSeed);
+        D.pf_seed = seed;
+        D.pf_pow = hash_pow(seed);
         int lg = 4;
-        while ((1 << lg) < 2 * hs.n_bc) lg++;
-        hs.pf_log2 = lg;
+        while ((1 << lg) < 2 * D.n_bc) lg++;
+        D.pf_log2 = lg;
         const uint32_t size = 1u << lg;
         hs.pf_keys.assign(size, 0u);
         hs.pf_vals.assign(size, kPfEmpty);
         int bl = 13;                                    // >= 512 bits per barcode, 8 KB .. 32 KB
-        while (bl < 18 && (1 << bl) < 512 * hs.n_bc) bl++;
-        hs.pf_bm_log2 = bl;
+        while (bl < 18 && (1 << bl) < 512 * D.n_bc) bl++;
+        D.pf_bm_log2 = bl;
         hs.pf_bitmap.assign((size_t)1 << (bl - 5), 0u);
-        for (int b = 0; b < hs.n_bc; b++) {            // ascending: the lowest index of identical sequences stays
+        for (int b = 0; b < D.n_bc; b++) {            // ascending: the lowest index of identical sequences stays
             const int m = hs.off[b + 1] - hs.off[b];
             uint32_t h = 0;
             for (int i = 0; i < seed; i++) h = h * kPfBase + (uint32_t)hs.bytes[hs.off[b] + i];
@@ -164,164 +146,150 @@ void build_prefilter(const Build &B)
                 hs.pf_vals[slot] = ((uint32_t)m << 16) | (uint32_t)b;
             }
         }
-        hs.pf_enabled = 1;
+        D.pf_enabled = 1;
     }
 }
 
-// pigeonhole seed levels of k_seed (seed.cu)
-void build_seed_levels(const Build &B)
+// a hashed seed table of k_seed / k_seed_deep: the q-mer at each offset in `offs` of every barcode (class codes),
+// a first-level bitmap and CSR buckets of (barcode index << 8) | offset with the q-mer's hash
+void build_hashed_level(const HostSet &hs, int n_bc, int q, const std::vector<int> &offs, SeedLevel &L,
+                        HostSet::HostSeedLevel &H)
 {
-    const bdx_params &p = B.p;
-    HostSet &hs = B.hs;
-    const bool sg = B.sg, benign = B.benign;
-    const int min_m = B.min_m;
-    (void)p; (void)sg; (void)benign; (void)min_m;
+    L.q = q;
+    L.pow = hash_pow(q);
+    const size_t n_entries = (size_t)n_bc * offs.size();
+    int lg = 8;
+    while (lg < 14 && (size_t)(1 << lg) < n_entries) lg++;
+    L.log2 = lg;
+    int bl = 13;                                // ~64 bits per entry: 4 KB for 96 barcodes
+    while (bl < 18 && ((size_t)1 << bl) < 64 * n_entries) bl++;
+    L.bm_log2 = bl;
+    H.bitmap.assign((size_t)1 << (bl - 5), 0u);
+    std::vector<std::vector<std::pair<uint32_t, uint32_t>>> buckets((size_t)1 << lg);
+    for (int b = 0; b < n_bc; b++)
+        for (int o : offs) {
+            uint32_t h = 0;
+            for (int k = 0; k < q; k++) h = h * kPfBase + (uint32_t)hs.bc_cls[hs.off[b] + o + k];
+            const uint32_t bit = pf_bit(h, bl);
+            H.bitmap[bit >> 5] |= 1u << (bit & 31);
+            buckets[pf_slot(h, lg)].emplace_back(((uint32_t)b << 8) | (uint32_t)o, h);
+        }
+    H.bstart.assign(((size_t)1 << lg) + 1, 0u);
+    for (size_t k = 0; k < buckets.size(); k++) {
+        H.bstart[k + 1] = H.bstart[k] + (uint32_t)buckets[k].size();
+        for (auto &pr : buckets[k]) {
+            H.entries.push_back(pr.first);
+            H.ekeys.push_back(pr.second);
+        }
+    }
+    L.n_entries = (int)H.entries.size();
+}
+
+// pigeonhole seed levels of k_seed (seed.cu)
+void build_seed_levels(const bdx_params &p, HostSet &hs, DevSet &D, uint32_t debug)
+{
     // ---- :semiglobal depth-limited seeds (seed.cu): uniform barcode length, no wildcard rows ----
-    if (hs.pf_enabled && sg && hs.words >= 1 && min_m == hs.max_m && hs.allowed0[0] >= 1 && hs.n_bc < (1 << 14) &&
-        !(B.debug & BDX_DEBUG_NO_SEEDS)) {
-        const int m = hs.max_m, allowed = hs.allowed0[0];
-        const double alpha = std::max(2, hs.n_classes - 1);
+    if (D.pf_enabled && p.algorithm == BDX_SEMIGLOBAL && D.words >= 1 && hs.min_m == D.max_m && hs.allowed0[0] >= 1 &&
+        D.n_bc < (1 << 14) && !(debug & BDX_DEBUG_NO_SEEDS)) {
+        const int m = D.max_m, allowed = hs.allowed0[0];
+        const double alpha = std::max(2, D.n_classes - 1);
         // chance hits per read column of level k: entries / alphabet^q with q = min(12, m / (k + 1))
         auto q_of = [&](int k) { return std::min(12, m / (k + 1)); };
-        auto rate_of = [&](int k) { return (double)hs.n_bc * (k + 1) / std::pow(alpha, q_of(k)); };
+        auto rate_of = [&](int k) { return (double)D.n_bc * (k + 1) / std::pow(alpha, q_of(k)); };
         // deepest level whose seeds are long enough to be selective (q >= 6, <= 0.12 chance hits per column)
         int K = 0;
         for (int k = 1; k <= std::min(allowed, 7); k++)   // hit records keep the diagonal span in 3 bits
             if (q_of(k) >= 6 && rate_of(k) <= 0.12) K = k;
         // a shallower level with far fewer chance hits in front of it pays when the deep one has many
         int K0 = 0;
-        if (K >= 2 && rate_of(K) > 0.02 && !(B.debug & BDX_DEBUG_ONE_SEED_LEVEL))
+        if (K >= 2 && rate_of(K) > 0.02 && !(debug & BDX_DEBUG_ONE_SEED_LEVEL))
             for (int k = 1; k < K; k++)
                 if (rate_of(k) <= 0.01) K0 = k;
-        hs.sd_m = m;
+        D.sd_m = m;
         for (int K_l : {K0, K}) {
             if (K_l < 1) continue;
-            HostSet::HostSeedLevel &L = hs.sd[hs.sd_levels++];
-            const int seg = m / (K_l + 1), q = std::min(12, seg);
+            const int l = D.sd_levels++, seg = m / (K_l + 1);
+            SeedLevel &L = D.sd[l];
             L.k = K_l;
-            L.q = q;
             // rows of k_seed's per-read hit list: three times the chance hits expected on 150 columns + two records
             // per true segment + slack.  (A fixed 28 rows cost 14 KB of shared memory per block -- one resident
             // block per SM less for 96 barcodes, whose lists never hold more than a handful.)
             L.max_hits = std::max(12, std::min(28, (int)std::ceil(3.0 * 150.0 * rate_of(K_l)) + 2 * (K_l + 1) + 4));
-            uint32_t pw = 1;
-            for (int i = 1; i < q; i++) pw *= kPfBase;
-            L.pow = pw;
-            const size_t n_entries = (size_t)hs.n_bc * (K_l + 1);
-            int lg = 8;
-            while (lg < 14 && (size_t)(1 << lg) < n_entries) lg++;
-            L.log2 = lg;
-            int bl = 13;                                // ~64 bits per entry: 4 KB for 96 barcodes
-            while (bl < 18 && ((size_t)1 << bl) < 64 * n_entries) bl++;
-            L.bm_log2 = bl;
-            L.bitmap.assign((size_t)1 << (bl - 5), 0u);
-            std::vector<std::vector<std::pair<uint32_t, uint32_t>>> buckets((size_t)1 << lg);
-            for (int b = 0; b < hs.n_bc; b++)
-                for (int i = 0; i <= K_l; i++) {
-                    const int o = i * seg;
-                    uint32_t h = 0;
-                    for (int k = 0; k < q; k++) h = h * kPfBase + (uint32_t)hs.bc_cls[hs.off[b] + o + k];
-                    const uint32_t bit = pf_bit(h, bl);
-                    L.bitmap[bit >> 5] |= 1u << (bit & 31);
-                    buckets[pf_slot(h, lg)].emplace_back(((uint32_t)b << 8) | (uint32_t)o, h);
-                }
-            L.bstart.assign(((size_t)1 << lg) + 1, 0u);
-            for (size_t k = 0; k < buckets.size(); k++) {
-                L.bstart[k + 1] = L.bstart[k] + (uint32_t)buckets[k].size();
-                for (auto &pr : buckets[k]) {
-                    L.entries.push_back(pr.first);
-                    L.ekeys.push_back(pr.second);
-                }
-            }
+            std::vector<int> offs;
+            for (int i = 0; i <= K_l; i++) offs.push_back(i * seg);
+            build_hashed_level(hs, D.n_bc, q_of(K_l), offs, L, hs.sd[l]);
         }
     }
 }
 
 // the deepest level of k_seed_deep (seed_deep.cu)
-void build_seed_deep(const Build &B)
+void build_seed_deep(HostSet &hs, DevSet &D, uint32_t debug)
 {
-    const bdx_params &p = B.p;
-    HostSet &hs = B.hs;
-    const bool sg = B.sg, benign = B.benign;
-    const int min_m = B.min_m;
-    (void)p; (void)sg; (void)benign; (void)min_m;
     // ---- deepest seed level (seed_deep.cu): depth beyond the regular levels, each segment hashed with its own
     // length.  Measured on B200: with 0.75 chance hits per column (96 x 24 nt at depth 4) it is slower than the
     // bit-parallel kernel it would replace (17 vs 11.5 ms per 10 M-read step), so it is used while the hits
     // stay rare (<= 0.25 per column) -- small sets, e.g. one adapter, whose alternative is k_literal ----
-    if (hs.sd_levels > 0 && !(B.debug & BDX_DEBUG_NO_SEED_DEEP)) {
-        const int m = hs.max_m, allowed = hs.allowed0[0];
-        const double alpha = std::max(2, hs.n_classes - 1);
+    if (D.sd_levels > 0 && !(debug & BDX_DEBUG_NO_SEED_DEEP)) {
+        const int m = D.max_m, allowed = hs.allowed0[0];
+        const double alpha = std::max(2, D.n_classes - 1);
         const double deep_rate = 0.25;      // chance hits per column the deep level accepts (measured, see above)
         int KD = 0;
-        for (int k = hs.sd[hs.sd_levels - 1].k + 1; k <= std::min(allowed, 7); k++) {
+        for (int k = D.sd[D.sd_levels - 1].k + 1; k <= std::min(allowed, 7); k++) {
             const int n_seg = k + 1, base_len = m / n_seg, extra = m % n_seg;
             if (base_len < 4) break;
             double rate = 0.0;
-            for (int i = 0; i < n_seg; i++) rate += hs.n_bc / std::pow(alpha, std::min(base_len + (i < extra ? 1 : 0), 8));
+            for (int i = 0; i < n_seg; i++) rate += D.n_bc / std::pow(alpha, std::min(base_len + (i < extra ? 1 : 0), 8));
             if (rate <= deep_rate) KD = k;
         }
         if (KD > 0) {
             const int n_seg = KD + 1, base_len = m / n_seg, extra = m % n_seg;
             const int q_long = std::min(base_len + 1, 8), q_short = std::min(base_len, 8);
-            hs.sdd_k = KD;
+            D.sdd_k = KD;
             // table 0: the longer seeds (if any segment is longer and that changes the seed length), table 1 / 0: the rest
-            struct Seg { int off, q; };
-            std::vector<Seg> segs[2];
+            std::vector<int> offs[2];
             int o = 0;
             for (int i = 0; i < n_seg; i++) {
                 const int len = base_len + (i < extra ? 1 : 0);
-                const int q = std::min(len, 8);
-                segs[(q == q_long && q_long != q_short) ? 0 : 1].push_back(Seg{o, q});
+                offs[(std::min(len, 8) == q_long && q_long != q_short) ? 0 : 1].push_back(o);
                 o += len;
             }
             for (int t = 0; t < 2; t++) {
-                if (segs[t].empty()) continue;
-                HostSet::HostSeedLevel &L = hs.sdd[hs.sdd_n++];
-                const int q = segs[t][0].q;
-                L.k = KD;
-                L.q = q;
-                uint32_t pw = 1;
-                for (int i = 1; i < q; i++) pw *= kPfBase;
-                L.pow = pw;
-                const size_t n_entries = (size_t)hs.n_bc * segs[t].size();
-                int lg = 8;
-                while (lg < 14 && (size_t)(1 << lg) < n_entries) lg++;
-                L.log2 = lg;
-                int bl = 13;
-                while (bl < 18 && ((size_t)1 << bl) < 64 * n_entries) bl++;
-                L.bm_log2 = bl;
-                L.bitmap.assign((size_t)1 << (bl - 5), 0u);
-                std::vector<std::vector<std::pair<uint32_t, uint32_t>>> buckets((size_t)1 << lg);
-                for (int b = 0; b < hs.n_bc; b++)
-                    for (const Seg &sg2 : segs[t]) {
-                        uint32_t h = 0;
-                        for (int k = 0; k < q; k++) h = h * kPfBase + (uint32_t)hs.bc_cls[hs.off[b] + sg2.off + k];
-                        const uint32_t bit = pf_bit(h, bl);
-                        L.bitmap[bit >> 5] |= 1u << (bit & 31);
-                        buckets[pf_slot(h, lg)].emplace_back(((uint32_t)b << 8) | (uint32_t)sg2.off, h);
-                    }
-                L.bstart.assign(((size_t)1 << lg) + 1, 0u);
-                for (size_t k = 0; k < buckets.size(); k++) {
-                    L.bstart[k + 1] = L.bstart[k] + (uint32_t)buckets[k].size();
-                    for (auto &pr : buckets[k]) {
-                        L.entries.push_back(pr.first);
-                        L.ekeys.push_back(pr.second);
-                    }
-                }
+                if (offs[t].empty()) continue;
+                const int l = D.sdd_n++;
+                D.sdd[l].k = KD;
+                build_hashed_level(hs, D.n_bc, t == 0 ? q_long : q_short, offs[t], D.sdd[l], hs.sdd[l]);
             }
         }
     }
 }
 
-// levels of k_seed_var (seed_var.cu)
-void build_seed_var(const Build &B)
+// a segment of barcode b at offset o whose first q bases are a k_seed_var seed
+struct VarSeg { int b, o, q; };
+
+// appends one direct-address table of k_seed_var to H: 4^q + 1 CSR row starts over the 2-bit codes of the segments
+// with seed length q, absolute indices into H.entries of (barcode index << 8) | offset.  false: a bucket holds more
+// than 255 entries (the scan keeps bucket sizes in a byte)
+bool append_direct_table(const HostSet &hs, int q, const std::vector<VarSeg> &segs, HostSet::HostSeedVar &H)
 {
-    const bdx_params &p = B.p;
-    HostSet &hs = B.hs;
-    const bool sg = B.sg, benign = B.benign;
-    const int min_m = B.min_m;
-    (void)p; (void)sg; (void)benign; (void)min_m;
+    std::vector<std::vector<uint32_t>> buckets((size_t)1 << (2 * q));
+    for (const VarSeg &s : segs) {
+        if (s.q != q) continue;
+        uint32_t code = 0;
+        for (int k = 0; k < q; k++) code |= ((uint32_t)(hs.bc_cls[hs.off[s.b] + s.o + k] - 1) & 3u) << (2 * k);
+        buckets[code].push_back(((uint32_t)s.b << 8) | (uint32_t)s.o);
+    }
+    for (const std::vector<uint32_t> &bk : buckets) {
+        if (bk.size() > 255) return false;
+        H.bstart.push_back((uint16_t)H.entries.size());
+        H.entries.insert(H.entries.end(), bk.begin(), bk.end());
+    }
+    H.bstart.push_back((uint16_t)H.entries.size());
+    return true;
+}
+
+// levels of k_seed_var (seed_var.cu)
+void build_seed_var(const bdx_params &p, HostSet &hs, DevSet &D, uint32_t debug)
+{
     // ---- seed-and-verify for sets of different lengths and constrained start / end geometries (seed_var.cu):
     // K_b + 1 disjoint segments per barcode, K_b = min(m_b / q - 1, allowed_b), their first q bases in a
     // direct-address table.  Level 1: q = the shortest seed whose CHANCE hits on admissible diagonals (estimated
@@ -329,23 +297,11 @@ void build_seed_var(const Build &B)
     // Level 2 (reads level 1 could not decide): the longest seed that is COMPLETE (K_b = allowed_b for every
     // barcode, so the candidates are a superset and every verdict is final), used while verifying its chance
     // hits costs less than half the lane-per-barcode automaton over the whole range ----
-    if (sg && hs.words >= 1 && !p.has_nindel && hs.n_classes - 1 <= 4 && hs.n_bc < (1 << 14) && hs.max_m <= 64 &&
-        p.max_error_rate >= 0.0 && !(B.debug & BDX_DEBUG_NO_SEEDS)) {
-        auto resolve = [](const DevRange &dr, int len, int &first, int &last) {      // classification.jl:96-100
-            const int s = dr.start_from_end ? len + dr.start_off : dr.start_off;
-            const int e = dr.end_from_end ? len + dr.end_off : dr.end_off;
-            first = std::max(1, s);
-            last = std::min(len, e);
-            if (last < first) last = first - 1;
-        };
-        const int n_nom = 150;
-        int rf, rl, bf, bl, ef, el;
-        resolve(hs.rs, n_nom, rf, rl);
-        resolve(hs.bs, n_nom, bf, bl);
-        resolve(hs.be, n_nom, ef, el);
-        const int start_j = std::max(rf, std::max(bf, 1)), end_j = std::min(rl, std::min(el, n_nom));
-        const int L = std::max(end_j - start_j + 1, 1), sbase = start_j - 1;
-        const int min_end_rel = ef - sbase, max_start_rel = bl - sbase;
+    if (p.algorithm == BDX_SEMIGLOBAL && D.words >= 1 && !p.has_nindel && D.n_classes - 1 <= 4 && D.n_bc < (1 << 14) &&
+        D.max_m <= 64 && p.max_error_rate >= 0.0 && !(debug & BDX_DEBUG_NO_SEEDS)) {
+        const Geometry g = pass_geometry(D, 150);
+        const int L = std::max(g.end_j - g.start_j + 1, 1), sbase = g.start_j - 1;
+        const int min_end_rel = g.min_end_pos - sbase, max_start_rel = g.max_start_pos - sbase;
         struct Est { double chance, steps; size_t n_entries; bool complete; };
         // admissible diagonals of barcode b at depth K (seed_var.cu, scan)
         auto n_diag = [&](int m, int a0, int K) {
@@ -354,7 +310,7 @@ void build_seed_var(const Build &B)
         };
         auto estimate = [&](int q) {
             Est e{0.0, 0.0, 0, true};
-            for (int b = 0; b < hs.n_bc; b++) {
+            for (int b = 0; b < D.n_bc; b++) {
                 const int m = hs.off[b + 1] - hs.off[b], a0 = hs.allowed0[b];
                 const int K = std::min(m / q - 1, a0);
                 const double c = (double)(K + 1) * n_diag(m, a0, K) / std::pow(4.0, q);
@@ -369,24 +325,24 @@ void build_seed_var(const Build &B)
         // + a handful of true ones -- fill to about 70 %; denser levels take fewer reads per group instead.
         // The 3-gram filter between the hit test and the list pays when most hits can fail it ((m - 2) - 3 K >= 4
         // for most barcodes); about one chance hit in seven passes it then (measured: one in ten for 24 nt, K = 4).
-        auto size_groups = [&](HostSet::HostSeedVar &V, double chance) {
+        auto size_groups = [&](SeedVar &V, const std::vector<uint8_t> &kdepth, double chance) {
             int strong = 0;
-            for (int b = 0; b < hs.n_bc; b++)
-                strong += (hs.off[b + 1] - hs.off[b] - 2) - 3 * (int)V.kdepth[(size_t)b] >= 4;
-            V.qgram_filter = hs.max_m <= 32 && 2 * strong >= hs.n_bc && !(B.debug & BDX_DEBUG_NO_QGRAM_FILTER);
+            for (int b = 0; b < D.n_bc; b++)
+                strong += (hs.off[b + 1] - hs.off[b] - 2) - 3 * (int)kdepth[(size_t)b] >= 4;
+            V.qgram_filter = D.max_m <= 32 && 2 * strong >= D.n_bc && !(debug & BDX_DEBUG_NO_QGRAM_FILTER);
             // mode 1 tests inside the scan (only survivors reach the list), mode 2 over the finished list: with few
             // admissible diagonals per barcode (constrained start / end) the scan's lanes rarely hold a hit at the
             // same time and the test would run for two or three lanes of a warp
             if (V.qgram_filter) {
                 double adm = 0.0, all = 0.0;
-                for (int b = 0; b < hs.n_bc; b++) {
-                    const int m = hs.off[b + 1] - hs.off[b], K = V.kdepth[(size_t)b];
+                for (int b = 0; b < D.n_bc; b++) {
+                    const int m = hs.off[b + 1] - hs.off[b], K = kdepth[(size_t)b];
                     adm += (double)(K + 1) * n_diag(m, hs.allowed0[b], K);
                     all += (double)(K + 1) * L;
                 }
                 V.qgram_filter = adm >= 0.5 * all ? 1 : 2;
             }
-            const double pass = V.qgram_filter == 1 ? (0.15 * strong + (hs.n_bc - strong)) / hs.n_bc : 1.0;
+            const double pass = V.qgram_filter == 1 ? (0.15 * strong + (D.n_bc - strong)) / D.n_bc : 1.0;
             const double per_read = chance * pass + 6.0;
             // shared memory per read (staged range, its bit planes, candidates, bookkeeping) kept to ~20 KB per block:
             // five or six blocks per SM hide the scan's shuffle and shared-memory latencies, three do not
@@ -399,59 +355,63 @@ void build_seed_var(const Build &B)
             V.group_reads = R;
             V.hit_rows = std::max(8, std::min(40, rows_for(R)));
             // a constrained start is re-checked by sg_literal, whose DP column (max_m + 2 entries per thread) reuses the list
-            const bool can_bound_start = !(hs.bs.end_from_end && hs.bs.end_off >= 0);
-            if (can_bound_start) V.hit_rows = std::max(V.hit_rows, hs.max_m + 2);
+            const bool can_bound_start = !(D.bs.end_from_end && D.bs.end_off >= 0);
+            if (can_bound_start) V.hit_rows = std::max(V.hit_rows, D.max_m + 2);
+        };
+        // the next level: the tables of the segments (seed length q, and q + 1 in a second table if any segment has
+        // it), barcode b's seeds complete for kdepth[b] edits.  A level whose table refuses its bucket sizes is not
+        // kept: its vectors are cleared and its SeedVar stays zero.
+        auto add_level = [&](int q, const std::vector<VarSeg> &segs, std::vector<uint8_t> kdepth, double chance) {
+            HostSet::HostSeedVar &H = hs.sv[D.sv_levels];
+            bool two = false;
+            for (const VarSeg &s : segs) two = two || s.q != q;
+            for (int t = 0; t < (two ? 2 : 1); t++)
+                if (!append_direct_table(hs, q + t, segs, H)) {
+                    H = HostSet::HostSeedVar();
+                    return;
+                }
+            SeedVar &V = D.sv[D.sv_levels++];
+            V.enabled = 1;
+            V.q = q;
+            V.q2 = two ? q + 1 : 0;
+            V.bstart2 = (1 << (2 * q)) + 1;
+            V.n_bstart = (int)H.bstart.size();
+            V.n_entries = (int)H.entries.size();
+            V.complete = 1;
+            V.sigma_min = 1e300;
+            for (int b = 0; b < D.n_bc; b++) {
+                if (kdepth[(size_t)b] < hs.allowed0[b]) V.complete = 0;
+                V.sigma_min = std::min(V.sigma_min, (double)(kdepth[(size_t)b] + 1) / (double)hs.norm[b]);
+            }
+            size_groups(V, kdepth, chance);
+            H.kdepth = std::move(kdepth);
         };
         // level with ONE seed length q: K_b + 1 segments of m_b / (K_b + 1) >= q bases, K_b = min(m_b / q - 1, allowed_b)
         auto build = [&](int q, double chance) {
-            HostSet::HostSeedVar &V = hs.sv[hs.sv_levels++];
-            V.q = q;
-            V.q2 = 0;
-            V.kdepth.assign((size_t)hs.n_bc, 0);
-            std::vector<std::vector<uint32_t>> buckets((size_t)1 << (2 * q));
-            V.sigma_min = 1e300;
-            V.complete = 1;
-            for (int b = 0; b < hs.n_bc; b++) {
-                const int m = hs.off[b + 1] - hs.off[b], a0 = hs.allowed0[b];
-                const int K = std::min(m / q - 1, a0);
-                V.kdepth[(size_t)b] = (uint8_t)K;
-                if (K < a0) V.complete = 0;
-                V.sigma_min = std::min(V.sigma_min, (double)(K + 1) / (double)hs.norm[b]);
+            std::vector<VarSeg> segs;
+            std::vector<uint8_t> kdepth((size_t)D.n_bc);
+            for (int b = 0; b < D.n_bc; b++) {
+                const int m = hs.off[b + 1] - hs.off[b], K = std::min(m / q - 1, hs.allowed0[b]);
+                kdepth[(size_t)b] = (uint8_t)K;
                 const int seg = m / (K + 1);                       // >= q: the segments are disjoint
-                for (int i = 0; i <= K; i++) {
-                    const int o = i * seg;
-                    uint32_t code = 0;
-                    for (int k = 0; k < q; k++) code |= ((uint32_t)(hs.bc_cls[hs.off[b] + o + k] - 1) & 3u) << (2 * k);
-                    buckets[code].push_back(((uint32_t)b << 8) | (uint32_t)o);
-                }
+                for (int i = 0; i <= K; i++) segs.push_back(VarSeg{b, i * seg, q});
             }
-            V.bstart.assign(buckets.size() + 1, 0);
-            for (size_t k = 0; k < buckets.size(); k++) {
-                if (buckets[k].size() > 255) {                     // the scan keeps bucket sizes in a byte
-                    V = HostSet::HostSeedVar();
-                    hs.sv_levels--;
-                    return;
-                }
-                V.bstart[k + 1] = (uint16_t)(V.bstart[k] + buckets[k].size());
-                V.entries.insert(V.entries.end(), buckets[k].begin(), buckets[k].end());
-            }
-            size_groups(V, chance);
+            add_level(q, segs, std::move(kdepth), chance);
         };
         // COMPLETE level (K_b = allowed_b): barcode b is cut into allowed_b + 1 segments of m_b / (allowed_b + 1) bases,
         // the first m_b % (allowed_b + 1) of them one base longer; every segment is a seed of its own length, kept
         // in one of two tables (q and q + 1: e.g. 24 nt at depth 4 = four 5-mers and one 4-mer, 2.5 x fewer chance
         // hits than five 4-mers)
-        struct Seg { int b, o, q; };
-        auto complete_segments = [&](int q_lo, std::vector<Seg> &segs) {
+        auto complete_segments = [&](int q_lo, std::vector<VarSeg> &segs) {
             Est e{0.0, 0.0, 0, true};
-            for (int b = 0; b < hs.n_bc; b++) {
+            for (int b = 0; b < D.n_bc; b++) {
                 const int m = hs.off[b + 1] - hs.off[b], a0 = hs.allowed0[b];
                 const int n_seg = a0 + 1, base = m / n_seg, extra = m % n_seg;
                 int o = 0;
                 for (int i = 0; i < n_seg; i++) {
                     const int len = base + (i < extra ? 1 : 0);
                     const int q = (len > q_lo && q_lo < 8) ? q_lo + 1 : q_lo;
-                    segs.push_back(Seg{b, o, q});
+                    segs.push_back(VarSeg{b, o, q});
                     const double c = (double)n_diag(m, a0, a0) / std::pow(4.0, q);
                     e.chance += c;
                     e.steps += c * (m + 2 * a0);
@@ -461,59 +421,24 @@ void build_seed_var(const Build &B)
             e.n_entries = segs.size();
             return e;
         };
-        auto build_complete = [&](int q_lo, const std::vector<Seg> &segs, double chance) {
-            HostSet::HostSeedVar &V = hs.sv[hs.sv_levels++];
-            bool two = false;
-            for (const Seg &sg2 : segs) two = two || sg2.q != q_lo;
-            V.q = q_lo;
-            V.q2 = two ? q_lo + 1 : 0;
-            V.kdepth.assign((size_t)hs.n_bc, 0);
-            V.sigma_min = 1e300;
-            V.complete = 1;
-            for (int b = 0; b < hs.n_bc; b++) {
-                V.kdepth[(size_t)b] = (uint8_t)hs.allowed0[b];
-                V.sigma_min = std::min(V.sigma_min, (double)(hs.allowed0[b] + 1) / (double)hs.norm[b]);
-            }
-            for (int t = 0; t < (two ? 2 : 1); t++) {
-                const int q = t ? q_lo + 1 : q_lo;
-                std::vector<std::vector<uint32_t>> buckets((size_t)1 << (2 * q));
-                for (const Seg &sg2 : segs) {
-                    if (sg2.q != q) continue;
-                    uint32_t code = 0;
-                    for (int k = 0; k < q; k++) code |= ((uint32_t)(hs.bc_cls[hs.off[sg2.b] + sg2.o + k] - 1) & 3u) << (2 * k);
-                    buckets[code].push_back(((uint32_t)sg2.b << 8) | (uint32_t)sg2.o);
-                }
-                for (size_t k = 0; k < buckets.size(); k++) {
-                    if (buckets[k].size() > 255) {                 // the scan keeps bucket sizes in a byte
-                        V = HostSet::HostSeedVar();
-                        hs.sv_levels--;
-                        return;
-                    }
-                    V.bstart.push_back((uint16_t)V.entries.size());
-                    V.entries.insert(V.entries.end(), buckets[k].begin(), buckets[k].end());
-                }
-                V.bstart.push_back((uint16_t)V.entries.size());
-            }
-            size_groups(V, chance);
-        };
         int q1 = 0;
         for (int q = 4; q <= 8 && !q1; q++) {
-            if (min_m < q) break;
+            if (hs.min_m < q) break;
             const Est e = estimate(q);
             if (e.chance <= 24.0 && e.n_entries <= 65535) {
                 build(q, e.chance);
-                if (hs.sv_levels > 0) q1 = q;
+                if (D.sv_levels > 0) q1 = q;
             }
         }
-        if (q1 && !hs.sv[0].complete && !(B.debug & BDX_DEBUG_ONE_SEED_LEVEL)) {
+        if (q1 && !D.sv[0].complete && !(debug & BDX_DEBUG_ONE_SEED_LEVEL)) {
             int q_lo = 8;
-            for (int b = 0; b < hs.n_bc; b++) q_lo = std::min(q_lo, (hs.off[b + 1] - hs.off[b]) / (hs.allowed0[b] + 1));
+            for (int b = 0; b < D.n_bc; b++) q_lo = std::min(q_lo, (hs.off[b + 1] - hs.off[b]) / (hs.allowed0[b] + 1));
             if (q_lo >= 3) {
-                std::vector<Seg> segs;
+                std::vector<VarSeg> segs;
                 const Est e = complete_segments(q_lo, segs);
-                const double automaton_steps = (double)hs.n_bc * L;
+                const double automaton_steps = (double)D.n_bc * L;
                 if (e.n_entries <= 65535 && e.steps < 0.5 * automaton_steps && e.chance <= 200.0)
-                    build_complete(q_lo, segs, e.chance);
+                    add_level(q_lo, segs, std::vector<uint8_t>(hs.allowed0.begin(), hs.allowed0.begin() + D.n_bc), e.chance);
             }
         }
         // With a complete level behind them (score-only passes, plan.cu), k_seed's levels only have to
@@ -521,70 +446,67 @@ void build_seed_var(const Build &B)
         // e.g. 96 x 24 nt at depth 3: 6-mers, 14 chance hits per read) -- the reads it resolved cost less in the
         // complete level than the level costs on all of its input (config 2: 889 -> 910 M reads/s).  Sets without a
         // complete level keep it: there its reads would fall to the lane-per-barcode automaton (config 5: 38 -> 24).
-        if (hs.sv_levels > 0 && hs.sv[hs.sv_levels - 1].complete && hs.sd_levels == 2 && hs.trim_side == 0 && !p.want_stats) {
-            const HostSet::HostSeedLevel &D = hs.sd[1];
-            const double rate = (double)hs.n_bc * (D.k + 1) / std::pow((double)std::max(2, hs.n_classes - 1), D.q);
+        if (D.sv_levels > 0 && D.sv[D.sv_levels - 1].complete && D.sd_levels == 2 && D.trim_side == 0 && !p.want_stats) {
+            const SeedLevel &L2 = D.sd[1];
+            const double rate = (double)D.n_bc * (L2.k + 1) / std::pow((double)std::max(2, D.n_classes - 1), L2.q);
             if (rate > 0.02) {
+                D.sd[1] = SeedLevel();
                 hs.sd[1] = HostSet::HostSeedLevel();
-                hs.sd_levels = 1;
+                D.sd_levels = 1;
             }
         }
     }
 }
 
 // bit planes and direct-address seed tables of k_hamming_scan (hamming.cu)
-void build_hamming_packed(const Build &B)
+void build_hamming_packed(const bdx_params &p, HostSet &hs, DevSet &D, uint32_t debug)
 {
-    const bdx_params &p = B.p;
-    HostSet &hs = B.hs;
-    const bool sg = B.sg, benign = B.benign;
-    const int min_m = B.min_m;
-    (void)p; (void)sg; (void)benign; (void)min_m;
     // ---- :hamming on packed words (hamming.cu): uniform length <= 32, <= 4 distinct barcode bytes, no 'N' ----
-    if (!(B.debug & BDX_DEBUG_NO_HAMMING_PACKED) && p.algorithm == BDX_HAMMING && min_m == hs.max_m && hs.max_m <= 32 && hs.n_classes - 1 <= 4 && hs.n_bc <= 65535 &&
+    if (!(debug & BDX_DEBUG_NO_HAMMING_PACKED) && p.algorithm == BDX_HAMMING && hs.min_m == D.max_m && D.max_m <= 32 && D.n_classes - 1 <= 4 && D.n_bc <= 65535 &&
         hs.allowed0[0] >= 0 && hs.allowed0[0] <= 7 && p.max_error_rate >= 0.0 &&
         std::find(hs.bytes.begin(), hs.bytes.end(), (uint8_t)'N') == hs.bytes.end()) {
-        const int m = hs.max_m, n_seg = hs.allowed0[0] + 1;
+        const int m = D.max_m, n_seg = hs.allowed0[0] + 1;
         const int seg_len = m / n_seg, extra = m % n_seg;      // the first `extra` segments are one base longer
         if (seg_len >= 2) {
-            hs.hp_m = m;
-            hs.hp_allowed = hs.allowed0[0];
-            hs.hp_n_seg = n_seg;
+            HammingPacked &H = D.hp;
+            H.m = m;
+            H.allowed = hs.allowed0[0];
+            H.n_seg = n_seg;
             int o = 0, base = 0;
             for (int i = 0; i < n_seg; i++) {
                 const int len = seg_len + (i < extra ? 1 : 0);
-                hs.hp_off[i] = o;
-                hs.hp_q[i] = std::min(len, 6);                  // direct-address table of 4^q buckets
-                hs.hp_base[i] = base;
-                base += (1 << (2 * hs.hp_q[i])) + 1;
+                H.seg_off[i] = o;
+                H.seg_q[i] = std::min(len, 6);                  // direct-address table of 4^q buckets
+                H.seg_base[i] = base;
+                base += (1 << (2 * H.seg_q[i])) + 1;
                 o += len;
             }
             auto code_of = [&](int b, int pos) { return (uint32_t)(hs.bc_cls[hs.off[b] + pos] - 1) & 3u; };
             hs.hp_bstart.assign((size_t)base, 0);
-            hs.hp_entries.assign((size_t)n_seg * hs.n_bc, 0);
+            hs.hp_entries.assign((size_t)n_seg * D.n_bc, 0);
             for (int i = 0; i < n_seg; i++) {
-                const int nb = 1 << (2 * hs.hp_q[i]);
+                const int nb = 1 << (2 * H.seg_q[i]);
                 std::vector<std::vector<uint16_t>> buckets((size_t)nb);
-                for (int b = 0; b < hs.n_bc; b++) {
+                for (int b = 0; b < D.n_bc; b++) {
                     uint32_t gram = 0;           // bit plane 0 of the q bases, then bit plane 1
-                    for (int k = 0; k < hs.hp_q[i]; k++) {
-                        const uint32_t c = code_of(b, hs.hp_off[i] + k);
+                    for (int k = 0; k < H.seg_q[i]; k++) {
+                        const uint32_t c = code_of(b, H.seg_off[i] + k);
                         gram |= (c & 1u) << k;
-                        gram |= (c >> 1) << (hs.hp_q[i] + k);
+                        gram |= (c >> 1) << (H.seg_q[i] + k);
                     }
                     buckets[gram].push_back((uint16_t)b);
                 }
                 uint16_t run = 0;
-                size_t w = (size_t)i * hs.n_bc;
+                size_t w = (size_t)i * D.n_bc;
                 for (int gidx = 0; gidx < nb; gidx++) {
-                    hs.hp_bstart[(size_t)hs.hp_base[i] + gidx] = run;
+                    hs.hp_bstart[(size_t)H.seg_base[i] + gidx] = run;
                     for (uint16_t b : buckets[(size_t)gidx]) hs.hp_entries[w++] = b;
                     run = (uint16_t)(run + buckets[(size_t)gidx].size());
                 }
-                hs.hp_bstart[(size_t)hs.hp_base[i] + nb] = run;
+                hs.hp_bstart[(size_t)H.seg_base[i] + nb] = run;
             }
-            hs.hp_bcw.resize((size_t)hs.n_bc);
-            for (int b = 0; b < hs.n_bc; b++) {
+            hs.hp_bcw.resize((size_t)D.n_bc);
+            for (int b = 0; b < D.n_bc; b++) {
                 uint32_t w0 = 0, w1 = 0;         // the two bit planes, base k in bit k
                 for (int k = 0; k < m; k++) {
                     w0 |= (code_of(b, k) & 1u) << k;
@@ -592,14 +514,15 @@ void build_hamming_packed(const Build &B)
                 }
                 hs.hp_bcw[(size_t)b] = make_uint2(w0, w1);
             }
-            hs.hp_enabled = 1;
+            H.n_bstart = base;
+            H.enabled = 1;
         }
     }
 }
 
 }  // namespace
 
-int bdx_build_set(const bdx_params &p, const bdx_barcode_set &in, HostSet &hs, uint32_t debug, const char *name)
+int bdx_build_set(const bdx_params &p, const bdx_barcode_set &in, HostSet &hs, DevSet &D, uint32_t debug, const char *name)
 {
     if (in.n_barcodes <= 0 || !in.bytes || !in.offsets)
         return bdx_fail(BDX_ERR_INVALID, std::string(name) + ": empty barcode set");
@@ -608,24 +531,26 @@ int bdx_build_set(const bdx_params &p, const bdx_barcode_set &in, HostSet &hs, u
         return bdx_fail(BDX_ERR_INVALID, "trim_side must be 3 or 5");  // core.jl:308-313
     if (p.has_nindel && !in.lengths_no_n)
         return bdx_fail(BDX_ERR_INVALID, std::string(name) + ": lengths_no_n required with nindel");
-    hs.n_bc = in.n_barcodes;
-    hs.trim_side = in.trim_side;
+    D.n_bc = in.n_barcodes;
+    D.trim_side = in.trim_side;
     int rc;
-    if ((rc = narrow_range(in.ref_search_range, hs.rs, name))) return rc;
-    if ((rc = narrow_range(in.barcode_start_range, hs.bs, name))) return rc;
-    if ((rc = narrow_range(in.barcode_end_range, hs.be, name))) return rc;
+    if ((rc = narrow_range(in.ref_search_range, D.rs, name))) return rc;
+    if ((rc = narrow_range(in.barcode_start_range, D.bs, name))) return rc;
+    if ((rc = narrow_range(in.barcode_end_range, D.be, name))) return rc;
     if (in.offsets[0] != 0) return bdx_fail(BDX_ERR_INVALID, std::string(name) + ": offsets[0] must be 0");
     hs.off.assign(in.offsets, in.offsets + in.n_barcodes + 1);
-    hs.max_m = 0;
-    for (int b = 0; b < hs.n_bc; b++) {
+    D.max_m = 0;
+    hs.min_m = kMaxBarcodeLen;
+    for (int b = 0; b < D.n_bc; b++) {
         const int m = hs.off[b + 1] - hs.off[b];
         if (m <= 0) return bdx_fail(BDX_ERR_INVALID, std::string(name) + ": empty barcode (not supported)");
         if (m > kMaxBarcodeLen) return bdx_fail(BDX_ERR_INVALID, std::string(name) + ": barcode longer than 256");
-        hs.max_m = std::max(hs.max_m, m);
+        D.max_m = std::max(D.max_m, m);
+        hs.min_m = std::min(hs.min_m, m);
     }
-    hs.bytes.assign(in.bytes, in.bytes + hs.off[hs.n_bc]);
-    hs.norm.resize(hs.n_bc);
-    for (int b = 0; b < hs.n_bc; b++) {
+    hs.bytes.assign(in.bytes, in.bytes + hs.off[D.n_bc]);
+    hs.norm.resize(D.n_bc);
+    for (int b = 0; b < D.n_bc; b++) {
         const int m = hs.off[b + 1] - hs.off[b];
         // semiglobal: m, or bc_lengths_no_N under NScoring (classification.jl:460, :476, :647);
         // hamming: m (:567, :607)
@@ -638,59 +563,52 @@ int bdx_build_set(const bdx_params &p, const bdx_barcode_set &in, HostSet &hs, u
             return bdx_fail(BDX_ERR_INVALID, std::string(name) + ": max_error_rate * length outside Int64 (the reference "
                                                              "raises InexactError on floor(Int, max_error_rate * length))");
     }
-    int min_m = hs.max_m;
-    for (int b = 0; b < hs.n_bc; b++) min_m = std::min(min_m, hs.off[b + 1] - hs.off[b]);
-    const bool benign = p.match >= 0 && p.mismatch >= 1 && p.indel >= 1 && (!p.has_nindel || p.nindel >= p.indel);
-    const Build B{p, hs, debug, p.algorithm == BDX_SEMIGLOBAL, benign, min_m};
-    build_filter_tables(B);
-    build_prefilter(B);
-    build_seed_levels(B);
-    build_seed_deep(B);
-    build_seed_var(B);
-    build_hamming_packed(B);
+    build_filter_tables(p, hs, D, debug);
+    build_prefilter(p, hs, D, debug);
+    build_seed_levels(p, hs, D, debug);
+    build_seed_deep(hs, D, debug);
+    build_seed_var(p, hs, D, debug);
+    build_hamming_packed(p, hs, D, debug);
     return BDX_OK;
 }
 
 // Text description of the tables built for one barcode set (bdx_config_describe): which shortcut stages exist and
 // with which parameters.  Host data only.
-std::string bdx_describe_set(const HostSet &hs)
+std::string bdx_describe_set(const HostSet &hs, const DevSet &D)
 {
     char line[256];
     std::string out;
-    int min_m = hs.max_m;
-    for (int b = 0; b < hs.n_bc; b++) min_m = std::min(min_m, hs.off[b + 1] - hs.off[b]);
-    snprintf(line, sizeof line, "set: barcodes=%d length=%d..%d classes=%d words=%d filter=%d\n", hs.n_bc, hs.n_bc ? min_m : 0,
-             hs.max_m, hs.n_classes - 1, hs.words, hs.use_filter);
+    snprintf(line, sizeof line, "set: barcodes=%d length=%d..%d classes=%d words=%d filter=%d\n", D.n_bc, hs.min_m, D.max_m,
+             D.n_classes - 1, D.words, D.use_filter);
     out += line;
-    if (hs.pf_enabled) {
-        snprintf(line, sizeof line, "prefilter: seed=%d log2=%d bitmap_log2=%d\n", hs.pf_seed, hs.pf_log2, hs.pf_bm_log2);
+    if (D.pf_enabled) {
+        snprintf(line, sizeof line, "prefilter: seed=%d log2=%d bitmap_log2=%d\n", D.pf_seed, D.pf_log2, D.pf_bm_log2);
         out += line;
     }
-    for (int l = 0; l < hs.sd_levels; l++) {
-        snprintf(line, sizeof line, "k_seed level %d: K=%d q=%d entries=%zu max_hits=%d\n", l + 1, hs.sd[l].k, hs.sd[l].q,
-                 hs.sd[l].entries.size(), hs.sd[l].max_hits);
+    for (int l = 0; l < D.sd_levels; l++) {
+        snprintf(line, sizeof line, "k_seed level %d: K=%d q=%d entries=%d max_hits=%d\n", l + 1, D.sd[l].k, D.sd[l].q,
+                 D.sd[l].n_entries, D.sd[l].max_hits);
         out += line;
     }
-    for (int l = 0; l < hs.sdd_n; l++) {
-        snprintf(line, sizeof line, "k_seed_deep table %d: K=%d q=%d entries=%zu\n", l + 1, hs.sdd_k, hs.sdd[l].q, hs.sdd[l].entries.size());
+    for (int l = 0; l < D.sdd_n; l++) {
+        snprintf(line, sizeof line, "k_seed_deep table %d: K=%d q=%d entries=%d\n", l + 1, D.sdd_k, D.sdd[l].q, D.sdd[l].n_entries);
         out += line;
     }
-    for (int l = 0; l < hs.sv_levels; l++) {
-        const HostSet::HostSeedVar &V = hs.sv[l];
+    for (int l = 0; l < D.sv_levels; l++) {
+        const SeedVar &V = D.sv[l];
         int k_lo = 255, k_hi = 0;
-        for (uint8_t k : V.kdepth) {
+        for (uint8_t k : hs.sv[l].kdepth) {
             k_lo = std::min<int>(k_lo, k);
             k_hi = std::max<int>(k_hi, k);
         }
-        snprintf(line, sizeof line, "k_seed_var level %d: q=%d q2=%d K=%d..%d complete=%d entries=%zu group_reads=%d hit_rows=%d qgram_filter=%d\n",
-                 l + 1, V.q, V.q2, V.kdepth.empty() ? 0 : k_lo, k_hi, V.complete, V.entries.size(), V.group_reads, V.hit_rows,
+        snprintf(line, sizeof line, "k_seed_var level %d: q=%d q2=%d K=%d..%d complete=%d entries=%d group_reads=%d hit_rows=%d qgram_filter=%d\n",
+                 l + 1, V.q, V.q2, hs.sv[l].kdepth.empty() ? 0 : k_lo, k_hi, V.complete, V.n_entries, V.group_reads, V.hit_rows,
                  V.qgram_filter);
         out += line;
     }
-    if (hs.hp_enabled) {
-        snprintf(line, sizeof line, "k_hamming_scan: m=%d allowed=%d segments=%d\n", hs.hp_m, hs.hp_allowed, hs.hp_n_seg);
+    if (D.hp.enabled) {
+        snprintf(line, sizeof line, "k_hamming_scan: m=%d allowed=%d segments=%d\n", D.hp.m, D.hp.allowed, D.hp.n_seg);
         out += line;
     }
     return out;
 }
-
