@@ -91,16 +91,17 @@ struct DevSet {
     const int *filt_allowed;      // [n_bc_pad] unit-cost candidate threshold, -1 = padding
     const int *allowed0;          // [n_bc_pad] floor(max_error_rate * norm) at the initial threshold
     const uint8_t *class_of;      // [256] byte -> class
-    // perfect-occurrence prefilter (filter.cu): open-addressing table of barcode hashes
+    // perfect-occurrence prefilter (filter.cu): open-addressing table of barcode q-mer hashes
     int pf_enabled;               // 0 = off (N wildcard rows, barcodes shorter than kPfMinSeed, ...)
-    int pf_seed;                  // hashed prefix length = min(shortest barcode, kPfMaxSeed)
+    int pf_seed;                  // hashed q-mer length q = min(shortest barcode, kPfMaxSeed)
     uint32_t pf_pow;              // kPfBase^(pf_seed-1)
     int pf_log2;                  // table size = 1 << pf_log2
     int pf_bm_log2;               // bitmap of 1 << pf_bm_log2 bits indexed by the top hash bits
-    int pad2;
-    const uint32_t *pf_bitmap;    // "some barcode prefix has this hash" (first-level reject)
-    const uint32_t *pf_keys;      // [size] hash of the first pf_seed class codes
-    const uint32_t *pf_vals;      // [size] (len << 16) | barcode index (lowest of identical sequences); kPfEmpty
+    int pf_stride;                // k_prefilter<0> hashes every pf_stride-th column; the table holds the q-mers at
+                                  // offsets 0 .. pf_stride - 1 of every barcode (1: prefixes, every column)
+    const uint32_t *pf_bitmap;    // "some barcode q-mer has this hash" (first-level reject)
+    const uint32_t *pf_keys;      // [size] hash of the entry's q-mer
+    const uint32_t *pf_vals;      // [size] pf_val(barcode, offset, length) (lowest index of identical sequences); kPfEmpty
     const uint8_t *bc_cls;        // barcode bytes mapped through class_of (same offsets as bc_bytes)
     // :semiglobal depth-limited seeds (seed.cu, k_seed): for uniform-length sets, every alignment
     // with <= k edits leaves one of k + 1 disjoint barcode segments intact.  Up to two levels: a
@@ -136,6 +137,22 @@ __host__ __device__ inline uint32_t pf_bit(uint32_t h, int log2bits)
 {
     return (h * kPfMix2) >> (32 - log2bits);
 }
+// hash of a q-mer of a sampled table (pf_stride > 1): its bytes as three little-endian words, the bytes from q on
+// zeroed.  k_prefilter<0> reads each sampled q-mer as three words from shared memory; per-column tables keep the
+// polynomial hash, which rolls.
+__host__ __device__ inline uint32_t pf_words_hash(uint32_t x0, uint32_t x1, uint32_t x2)
+{
+    return x0 * kPfBase + x1 * kPfMix + x2 * kPfMix2;
+}
+// pf_vals entry: barcode index (< 65535, so never kPfEmpty), offset of the q-mer in the barcode (< 256) and the
+// barcode's length (1 .. 256)
+__host__ __device__ inline uint32_t pf_val(int b, int o, int m)
+{
+    return (uint32_t)b | ((uint32_t)o << 16) | ((uint32_t)(m - 1) << 24);
+}
+__host__ __device__ inline int pf_val_bc(uint32_t v) { return (int)(v & 0xFFFFu); }
+__host__ __device__ inline int pf_val_off(uint32_t v) { return (int)((v >> 16) & 0xFFu); }
+__host__ __device__ inline int pf_val_len(uint32_t v) { return (int)(v >> 24) + 1; }
 
 struct DevParams {
     double max_error_rate, min_delta;
@@ -185,6 +202,7 @@ cudaError_t blocks_per_sm_cached(const void *kern, int threads, size_t smem, int
 // them against its budgets)
 size_t hamming_scan_smem(const DevSet &S);
 size_t prefilter_smem_bytes(const DevSet &S);
+int prefilter_blocks_per_sm(size_t smem);   // k_prefilter's resident blocks on sm_100 by shared memory alone
 size_t filter_smem_bytes(const DevSet &S);
 size_t seed_smem(const DevSet &S, const SeedLevel &L);
 size_t deep_smem(const DevSet &S);

@@ -339,33 +339,35 @@ k_filter(const __grid_constant__ DevParams P, const int pass, const uint8_t *__r
 // inside the search range scores 0, the running threshold drops to 0 and no later barcode can be accepted
 // (score < min_score is strict, classification.jl:658); an earlier barcode wins only with a
 // score of 0 itself, i.e. if IT occurs verbatim.  So the answer for such a read is the
-// lowest-index barcode with a verbatim occurrence: found with a rolling polynomial hash of
-// a seed-length window at every column, a table of barcode-prefix hashes in shared memory,
-// and byte-wise verification on a hit.  Resolved reads get their PassOut here; all other
-// reads are appended to the worklist the bit-parallel kernel then walks.
+// lowest-index barcode with a verbatim occurrence: found by hashing the q-mers of sampled
+// columns (every pf_stride-th column; pf_stride = 1: a rolling hash over every column) against
+// a table of barcode q-mer hashes in shared memory, and byte-wise verification on a hit.
+// Resolved reads get their PassOut here; all other reads are appended to the worklist the
+// bit-parallel kernel then walks.
 // ---------------------------------------------------------------------------------------
 constexpr int kPfThreads = 256;
 constexpr int kPfStageBytes = 48 * 1024;   // raw bytes of one group of 256 reads (<= 192 bases each)
 constexpr int kPfMaxCand = 2;              // table hits remembered per read; more => leave it to the DP
 
-// Rolling-hash scan of one read's search range.  Table hits are only RECORDED in the loop
+// Hash scan of one read's search range.  Table hits are only RECORDED in the loop
 // and verified byte by byte afterwards, when all lanes of the warp verify together (doing
 // it inside the loop serialises the lanes: each finds its hit at a different column).
-// Returns the lowest barcode index with a verified verbatim occurrence, 0x7FFFFFFF if none,
-// or -1 if there were more table hits than kPfMaxCand (the caller then leaves the read to
-// the bit-parallel kernel, which is always correct).
-template <typename BytePtr>
+// Every table entry (barcode b, offset o) that the q-mer at column w hashes to names the
+// candidate start w - o.  Returns the lowest barcode index with a verified verbatim occurrence,
+// 0x7FFFFFFF if none, or -1 if there were more table hits than kPfMaxCand (the caller then
+// leaves the read to the bit-parallel kernel, which is always correct).  found_w: the start
+// of the chosen occurrence of that barcode, leftmost or (want_rightmost) rightmost.
+// SAMPLED: the table may be a sampled one (k_prefilter<0>); otherwise pf_stride is 1.  STAGED: c0 points into the
+// shared-memory stage.
+template <bool SAMPLED, bool STAGED, typename BytePtr>
 __device__ __forceinline__ int pf_scan(BytePtr c0, int ncols, const DevSet &S, const uint32_t *keys_s,
                                        const uint32_t *vals_s, const uint32_t *bitmap_s, bool want_rightmost,
                                        int &found_w)
 {
     const int seed = S.pf_seed;
-    const uint32_t pw = S.pf_pow;
+    const int stride = S.pf_stride;
     const int bm_log2 = S.pf_bm_log2;
     const uint32_t size_mask = (1u << S.pf_log2) - 1u;
-    uint32_t h = 0;
-    for (int i = 0; i < seed; i++) h = h * kPfBase + (uint32_t)c0[i];
-    const int nwin = ncols - seed + 1;
     // The loop only REMEMBERS the (few) columns whose hash passes the first-level bitmap; the table is probed
     // after the loop, when the lanes of a warp probe together.  Probing inside the loop ran the probe for one lane
     // at a time -- each lane passes the bitmap at a different column -- and cost a fifth of the kernel's
@@ -373,25 +375,71 @@ __device__ __forceinline__ int pf_scan(BytePtr c0, int ncols, const DevSet &S, c
     constexpr int kRec = 4;
     int rw0 = 0, rw1 = 0, rw2 = 0, rw3 = 0, n_rec = 0;
     uint32_t rh0 = 0, rh1 = 0, rh2 = 0, rh3 = 0;
-    auto probe = [&](int w) {
-        const uint32_t bit = pf_bit(h, bm_log2);
-        if ((bitmap_s[bit >> 5] >> (bit & 31)) & 1u) {       // rare: some barcode prefix hashes here
-            if (n_rec == 0) { rw0 = w; rh0 = h; }
-            else if (n_rec == 1) { rw1 = w; rh1 = h; }
-            else if (n_rec == 2) { rw2 = w; rh2 = h; }
-            else if (n_rec == 3) { rw3 = w; rh3 = h; }
-            n_rec++;
-        }
+    auto record = [&](int w, uint32_t h) {
+        if (n_rec == 0) { rw0 = w; rh0 = h; }
+        else if (n_rec == 1) { rw1 = w; rh1 = h; }
+        else if (n_rec == 2) { rw2 = w; rh2 = h; }
+        else if (n_rec == 3) { rw3 = w; rh3 = h; }
+        n_rec++;
     };
-    const auto *c_in = c0 + seed;
+    auto passes = [&](uint32_t h) {                          // rare: some barcode q-mer hashes here
+        const uint32_t bit = pf_bit(h, bm_log2);
+        return (bitmap_s[bit >> 5] >> (bit & 31)) & 1u;
+    };
+    if (!SAMPLED || stride == 1) {
+        const uint32_t pw = S.pf_pow;
+        uint32_t h = 0;
+        for (int i = 0; i < seed; i++) h = h * kPfBase + (uint32_t)c0[i];
+        const int nwin = ncols - seed + 1;
+        const auto *c_in = c0 + seed;
 #pragma unroll 4
-    for (int w = 0; w < nwin - 1; w++) {
-        probe(w);
-        h = (h - (uint32_t)c0[w] * pw) * kPfBase + (uint32_t)c_in[w];
+        for (int w = 0; w < nwin - 1; w++) {
+            if (passes(h)) record(w, h);
+            h = (h - (uint32_t)c0[w] * pw) * kPfBase + (uint32_t)c_in[w];
+        }
+        if (nwin > 0 && passes(h)) record(nwin - 1, h);
+    } else {
+        // sampled columns are several columns apart: each q-mer (kPfMinSeed <= q <= kPfMaxSeed) is read as three
+        // little-endian words, bytes q.. masked off (pf_words_hash).  From the stage: the four aligned words around
+        // it, funnel-shifted (the stage has 16 bytes of slack behind the last read); from global memory: byte by byte.
+        const uint32_t m1 = seed >= 8 ? 0xFFFFFFFFu : (1u << (8 * (seed - 4))) - 1u;
+        const uint32_t m2 = seed >= 12 ? 0xFFFFFFFFu : (seed <= 8 ? 0u : (1u << (8 * (seed - 8))) - 1u);
+        auto qmer_hash = [&](int w) {
+            const auto *c = c0 + w;
+            uint32_t x0, x1, x2;
+            if constexpr (STAGED) {
+                const uint32_t mis = (uint32_t)reinterpret_cast<uintptr_t>(c) & 3u;
+                const uint32_t *a = reinterpret_cast<const uint32_t *>(c - mis);
+                const uint32_t y0 = a[0], y1 = a[1], y2 = a[2], y3 = a[3];
+                x0 = __funnelshift_r(y0, y1, 8 * mis);
+                x1 = __funnelshift_r(y1, y2, 8 * mis);
+                x2 = __funnelshift_r(y2, y3, 8 * mis);
+            } else {
+                x0 = (uint32_t)c[0] | (uint32_t)c[1] << 8 | (uint32_t)c[2] << 16 | (uint32_t)c[3] << 24;
+                x1 = x2 = 0u;
+#pragma unroll
+                for (int i = 4; i < kPfMaxSeed; i++)
+                    if (i < seed) (i < 8 ? x1 : x2) |= (uint32_t)c[i] << (8 * (i % 4));
+            }
+            return pf_words_hash(x0, x1 & m1, x2 & m2);
+        };
+        // the bitmap passes of up to 32 probes are collected as bits and recorded (hash recomputed) afterwards:
+        // recording inside the loop made ptxas move the record registers at every probe
+        const int n_probes = (ncols - seed) / stride + 1;
+        for (int k0 = 0; k0 < n_probes; k0 += 32) {
+            const int k1 = min(n_probes, k0 + 32);
+            uint32_t pass_bits = 0;
+            for (int k = k0; k < k1; k++) pass_bits |= passes(qmer_hash(k * stride)) << (k - k0);
+            while (pass_bits) {
+                const int k = k0 + __ffs(pass_bits) - 1;
+                pass_bits &= pass_bits - 1;
+                record(k * stride, qmer_hash(k * stride));
+            }
+        }
     }
-    if (nwin > 0) probe(nwin - 1);
     if (n_rec > kRec) return -1;                              // more bitmap hits than remembered: leave it to the DP
-    int cb[kPfMaxCand], cw[kPfMaxCand], nc = 0;
+    static_assert(kPfMaxCand == 2, "candidates are kept in scalars");
+    int cb0 = 0, cs0 = 0, cb1 = 0, cs1 = 0, nc = 0;     // (barcode, start); an indexed array went to local memory
 #pragma unroll
     for (int k = 0; k < kRec; k++) {
         if (k >= n_rec) continue;
@@ -401,11 +449,10 @@ __device__ __forceinline__ int pf_scan(BytePtr c0, int ncols, const DevSet &S, c
         for (;;) {
             const uint32_t v = vals_s[slot];
             if (v == kPfEmpty) break;
-            if (keys_s[slot] == hk && w + (int)(v >> 16) <= ncols) {
-                if (nc < kPfMaxCand) {
-                    cb[nc] = (int)(v & 0xFFFFu);
-                    cw[nc] = w;
-                }
+            const int s = w - pf_val_off(v);                  // candidate start
+            if (keys_s[slot] == hk && s >= 0 && s + pf_val_len(v) <= ncols) {
+                if (nc == 0) { cb0 = pf_val_bc(v); cs0 = s; }
+                else if (nc == 1) { cb1 = pf_val_bc(v); cs1 = s; }
                 nc++;
             }
             slot = (slot + 1) & size_mask;
@@ -416,18 +463,20 @@ __device__ __forceinline__ int pf_scan(BytePtr c0, int ncols, const DevSet &S, c
     found_w = -1;
 #pragma unroll
     for (int k = 0; k < kPfMaxCand; k++) {
-        // candidates are in column order: a later occurrence of the SAME barcode replaces the
-        // position only when the rightmost one is wanted (trim_side == 3, classification.jl:613-619)
-        if (k < nc && (cb[k] < found || (cb[k] == found && want_rightmost))) {
-            const int b = cb[k];
+        // another occurrence of the SAME barcode replaces the position only when it starts further left, or further
+        // right when the rightmost one is wanted (trim_side == 3, classification.jl:613-619).  Starts are compared,
+        // not scan order: a barcode with an internal repeat can yield two candidates at one sampled column.
+        const int cb = k == 0 ? cb0 : cb1, cs = k == 0 ? cs0 : cs1;
+        if (k < nc && (cb < found || (cb == found && (want_rightmost ? cs > found_w : cs < found_w)))) {
+            const int b = cb;
             const uint8_t *q = S.bc_bytes + S.bc_off[b];
             const int len = S.bc_off[b + 1] - S.bc_off[b];
             bool same = true;
             for (int i = 0; i < len; i++)
-                if (q[i] != c0[cw[k] + i]) { same = false; break; }
+                if (q[i] != c0[cs + i]) { same = false; break; }
             if (same) {
                 found = b;
-                found_w = cw[k];
+                found_w = cs;
             }
         }
     }
@@ -461,8 +510,8 @@ __device__ __forceinline__ int pf_scan_exact(BytePtr c0, int n_starts, int cols_
             for (;;) {
                 const uint32_t v = vals_s[slot];
                 if (v == kPfEmpty) break;
-                if (keys_s[slot] == h && w + (int)(v >> 16) <= cols_left && nc != kCandOverflow) {
-                    const uint16_t b = (uint16_t)(v & 0xFFFFu);
+                if (keys_s[slot] == h && w + pf_val_len(v) <= cols_left && nc != kCandOverflow) {
+                    const uint16_t b = (uint16_t)pf_val_bc(v);
                     int pos = 0;                                   // sorted insert, skip duplicates
                     while (pos < nc && list[pos] < b) pos++;
                     if (pos == nc || list[pos] != b) {
@@ -584,10 +633,10 @@ k_prefilter(const __grid_constant__ DevParams P, const int pass, const uint8_t *
                     int found, w = -1;
                     const bool right = S.trim_side == 3;
                     if (staged)
-                        found = pf_scan(stage + skew + (base - blk_base) + g.start_j - 1, cols, S, keys_s, vals_s,
+                        found = pf_scan<false, true>(stage + skew + (base - blk_base) + g.start_j - 1, cols, S, keys_s, vals_s,
                                         bitmap_s, right, w);
                     else
-                        found = pf_scan(seq + base + g.start_j - 1, cols, S, keys_s, vals_s, bitmap_s, right, w);
+                        found = pf_scan<false, false>(seq + base + g.start_j - 1, cols, S, keys_s, vals_s, bitmap_s, right, w);
                     if (found >= 0 && found != 0x7FFFFFFF) {
                         const int m = S.bc_off[found + 1] - S.bc_off[found];
                         const int s1 = g.start_j + w;                       // 1-based start
@@ -610,10 +659,10 @@ k_prefilter(const __grid_constant__ DevParams P, const int pass, const uint8_t *
                 const bool need_tb = S.trim_side != 0 || P.want_stats;
                 int found, w;
                 if (staged)
-                    found = pf_scan(stage + skew + (base - blk_base) + g.start_j - 1, ncols, S, keys_s, vals_s,
+                    found = pf_scan<true, true>(stage + skew + (base - blk_base) + g.start_j - 1, ncols, S, keys_s, vals_s,
                                     bitmap_s, S.trim_side == 3, w);
                 else
-                    found = pf_scan(seq + base + g.start_j - 1, ncols, S, keys_s, vals_s, bitmap_s, S.trim_side == 3, w);
+                    found = pf_scan<true, false>(seq + base + g.start_j - 1, ncols, S, keys_s, vals_s, bitmap_s, S.trim_side == 3, w);
                 if (found >= 0 && found != 0x7FFFFFFF) {
                     const int s1 = g.start_j + w, len = S.bc_off[found + 1] - S.bc_off[found];
                     out[read] = PassOut{found + 1, 0, need_tb ? s1 : -1, need_tb ? s1 + len - 1 : -1};
@@ -711,6 +760,12 @@ cudaError_t launch_filter(const DevParams &P, int pass, const uint8_t *seq, cons
 size_t prefilter_smem_bytes(const DevSet &S)
 {
     return kPfStageBytes + 16 + ((size_t)8 << S.pf_log2) + ((size_t)4 << (S.pf_bm_log2 - 5));
+}
+
+// sm_100: 228 KB of shared memory and 2048 threads an SM, 1 KB of it reserved per block
+int prefilter_blocks_per_sm(size_t smem)
+{
+    return (int)std::min<size_t>(2048 / kPfThreads, (size_t)228 * 1024 / (smem + 1024));
 }
 
 }  // namespace bdx

@@ -98,7 +98,7 @@ void build_filter_tables(const bdx_params &p, HostSet &hs, DevSet &D, uint32_t d
     }
 }
 
-// hash table of whole-barcode prefixes: k_prefilter (filter.cu)
+// hash table of barcode q-mers: k_prefilter (filter.cu)
 void build_prefilter(const bdx_params &p, HostSet &hs, DevSet &D, uint32_t debug)
 {
     // ---- perfect-occurrence prefilter table (semiglobal, no wildcard rows) ----
@@ -113,37 +113,69 @@ void build_prefilter(const bdx_params &p, HostSet &hs, DevSet &D, uint32_t debug
         const int seed = std::min(hs.min_m, kPfMaxSeed);
         D.pf_seed = seed;
         D.pf_pow = hash_pow(seed);
-        int lg = 4;
-        while ((1 << lg) < 2 * D.n_bc) lg++;
-        D.pf_log2 = lg;
-        const uint32_t size = 1u << lg;
-        hs.pf_keys.assign(size, 0u);
-        hs.pf_vals.assign(size, kPfEmpty);
         int bl = 13;                                    // >= 512 bits per barcode, 8 KB .. 32 KB
         while (bl < 18 && (1 << bl) < 512 * D.n_bc) bl++;
         D.pf_bm_log2 = bl;
+        // Table slots for `stride` q-mers per barcode.  The per-column scans probe it at every bitmap pass: load
+        // <= 1/2.  A sampled table is probed about 150 / stride times per read: load <= 3/4 keeps it small.
+        auto log2_for = [&](int stride) {
+            const int n = D.n_bc * stride;
+            int lg = 4;
+            while (stride == 1 ? (1 << lg) < 2 * n : 3 * (1 << lg) < 4 * n) lg++;
+            return lg;
+        };
+        // :semiglobal (k_prefilter<0>) samples every stride-th column, stride <= min_m - q + 1: a verbatim
+        // occurrence of a barcode starting at column s holds exactly one sampled column P in [s, s + stride - 1],
+        // and the q-mer at P is the barcode's q-mer at offset P - s.  The largest stride whose table keeps
+        // k_prefilter at the resident blocks of the prefix table; the bitmap keeps its bits per barcode, so the
+        // chance passes per read (columns probed x entries / bits) stay those of the per-column scan.  A sampled
+        // probe costs about what three columns of the rolling scan cost: below stride 4 the rolling scan stays
+        // (measured on B200: stride 2 made config 5s's k_prefilter 25 % slower).
+        constexpr int kMinStride = 4;
+        D.pf_stride = 1;
+        D.pf_log2 = log2_for(1);
+        const int blocks = std::max(1, prefilter_blocks_per_sm(prefilter_smem_bytes(D)));
+        for (int s = sg ? hs.min_m - seed + 1 : 1; s >= kMinStride; s--) {
+            D.pf_log2 = log2_for(s);
+            if (prefilter_blocks_per_sm(prefilter_smem_bytes(D)) >= blocks) {
+                D.pf_stride = s;
+                break;
+            }
+        }
+        if (D.pf_stride == 1) D.pf_log2 = log2_for(1);
+        const int lg = D.pf_log2, stride = D.pf_stride;
+        const uint32_t size = 1u << lg;
+        hs.pf_keys.assign(size, 0u);
+        hs.pf_vals.assign(size, kPfEmpty);
         hs.pf_bitmap.assign((size_t)1 << (bl - 5), 0u);
         for (int b = 0; b < D.n_bc; b++) {            // ascending: the lowest index of identical sequences stays
             const int m = hs.off[b + 1] - hs.off[b];
-            uint32_t h = 0;
-            for (int i = 0; i < seed; i++) h = h * kPfBase + (uint32_t)hs.bytes[hs.off[b] + i];
-            const uint32_t bit = pf_bit(h, bl);
-            hs.pf_bitmap[bit >> 5] |= 1u << (bit & 31);
-            uint32_t slot = pf_slot(h, lg);
-            bool dup = false;
-            while (hs.pf_vals[slot] != kPfEmpty) {
-                const uint32_t v = hs.pf_vals[slot];
-                const int ob = (int)(v & 0xFFFFu);
-                if (!ex && (int)(v >> 16) == m &&
-                    memcmp(&hs.bytes[hs.off[ob]], &hs.bytes[hs.off[b]], (size_t)m) == 0) {
-                    dup = true;
-                    break;
+            for (int o = 0; o < stride; o++) {
+                const uint8_t *qm = &hs.bytes[hs.off[b] + o];
+                uint32_t h = 0, x[3] = {0u, 0u, 0u};
+                for (int i = 0; i < seed; i++) {
+                    h = h * kPfBase + (uint32_t)qm[i];
+                    x[i / 4] |= (uint32_t)qm[i] << (8 * (i % 4));
                 }
-                slot = (slot + 1) & (size - 1);
-            }
-            if (!dup) {
-                hs.pf_keys[slot] = h;
-                hs.pf_vals[slot] = ((uint32_t)m << 16) | (uint32_t)b;
+                if (stride > 1) h = pf_words_hash(x[0], x[1], x[2]);
+                const uint32_t bit = pf_bit(h, bl);
+                hs.pf_bitmap[bit >> 5] |= 1u << (bit & 31);
+                uint32_t slot = pf_slot(h, lg);
+                bool dup = false;
+                while (hs.pf_vals[slot] != kPfEmpty) {
+                    const uint32_t v = hs.pf_vals[slot];
+                    const int ob = pf_val_bc(v);
+                    if (!ex && pf_val_len(v) == m && pf_val_off(v) == o &&
+                        memcmp(&hs.bytes[hs.off[ob]], &hs.bytes[hs.off[b]], (size_t)m) == 0) {
+                        dup = true;
+                        break;
+                    }
+                    slot = (slot + 1) & (size - 1);
+                }
+                if (!dup) {
+                    hs.pf_keys[slot] = h;
+                    hs.pf_vals[slot] = pf_val(b, o, m);
+                }
             }
         }
         D.pf_enabled = 1;
@@ -582,7 +614,8 @@ std::string bdx_describe_set(const HostSet &hs, const DevSet &D)
              D.n_classes - 1, D.words, D.use_filter);
     out += line;
     if (D.pf_enabled) {
-        snprintf(line, sizeof line, "prefilter: seed=%d log2=%d bitmap_log2=%d\n", D.pf_seed, D.pf_log2, D.pf_bm_log2);
+        snprintf(line, sizeof line, "prefilter: seed=%d stride=%d log2=%d bitmap_log2=%d\n", D.pf_seed, D.pf_stride,
+                 D.pf_log2, D.pf_bm_log2);
         out += line;
     }
     for (int l = 0; l < D.sd_levels; l++) {
