@@ -96,7 +96,7 @@ std::string bdx_describe_set(const HostSet &hs, const DevSet &D);   // tables.cu
 
 // ---- streams ----
 struct Slot {
-    uint8_t *h_seq = nullptr;
+    uint8_t *h_seq = nullptr;     // pinned input staging, allocated on the first batch that is not pinned already
     int32_t *h_off = nullptr;
     bdx_result *h_res = nullptr;
     bdx_pass_detail *h_det = nullptr;
@@ -141,7 +141,6 @@ struct bdx_stream {
     bool details = false;
     cudaStream_t st_copy = nullptr, st_comp = nullptr, st_d2h = nullptr;
     Slot slot[BDX_MAX_IN_FLIGHT];
-    bool host_staging = false;  // pinned h_seq / h_off are allocated on first use
     int head = 0;      // next slot to submit into
     int tail = 0;      // oldest in-flight slot
     int in_flight = 0;

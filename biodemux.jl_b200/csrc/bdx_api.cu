@@ -280,24 +280,29 @@ void bdx_stream_drop_graphs(bdx_stream *s)
         }
 }
 
+static void free_scratch(Scratch &sc)
+{
+    cudaFree(sc.pass[0]);
+    cudaFree(sc.pass[1]);
+    cudaFree(sc.cand);
+    cudaFree(sc.cand_cnt);
+    cudaFree(sc.worklist);
+    cudaFree(sc.n_work);
+    cudaFree(sc.worklist2);
+    cudaFree(sc.n_work2);
+    cudaFree(sc.wl_win);
+    cudaFree(sc.wl_full);
+    cudaFree(sc.n_lit);
+    sc = Scratch{};
+}
+
 static int ensure_scratch(bdx_stream *s, int64_t n)
 {
     if (n <= s->sc_cap) return BDX_OK;
     // in-order on the compute stream: earlier kernels still own the old buffers
     CU(cudaStreamSynchronize(s->st_comp));
     bdx_stream_drop_graphs(s);      // captured launches hold the old scratch pointers
-    cudaFree(s->sc.pass[0]);
-    cudaFree(s->sc.pass[1]);
-    cudaFree(s->sc.cand);
-    cudaFree(s->sc.cand_cnt);
-    cudaFree(s->sc.worklist);
-    cudaFree(s->sc.n_work);
-    cudaFree(s->sc.worklist2);
-    cudaFree(s->sc.n_work2);
-    cudaFree(s->sc.wl_win);
-    cudaFree(s->sc.wl_full);
-    cudaFree(s->sc.n_lit);
-    s->sc = Scratch{};
+    free_scratch(s->sc);
     s->sc_cap = 0;
     const int64_t cap = n + n / 8 + 1024;
     CU(cudaMalloc(&s->sc.pass[0], cap * sizeof(PassOut)));
@@ -315,6 +320,28 @@ static int ensure_scratch(bdx_stream *s, int64_t n)
     return BDX_OK;
 }
 
+// every buffer, event and graph of a slot: whatever stream_create_impl or ensure_input_buffers allocated
+static void free_slot(Slot &sl)
+{
+    cudaFreeHost(sl.h_seq);
+    cudaFreeHost(sl.h_off);
+    cudaFreeHost(sl.h_res);
+    cudaFreeHost(sl.h_det);
+    cudaFree(sl.d_packed);
+    cudaFreeHost(sl.h_packed);
+    cudaFree(sl.d_win);
+    cudaFree(sl.d_win_off);
+    cudaFreeHost(sl.h_win_off);
+    cudaFree(sl.d_seq);
+    cudaFree(sl.d_off);
+    cudaFree(sl.d_res);
+    cudaFree(sl.d_det);
+    if (sl.ev_h2d) cudaEventDestroy(sl.ev_h2d);
+    if (sl.ev_kern) cudaEventDestroy(sl.ev_kern);
+    if (sl.ev_done) cudaEventDestroy(sl.ev_done);
+    if (sl.graph) cudaGraphExecDestroy(sl.graph);
+}
+
 extern "C" void bdx_stream_destroy(bdx_stream *s)
 {
     if (!s) return;
@@ -322,36 +349,8 @@ extern "C" void bdx_stream_destroy(bdx_stream *s)
     if (s->st_comp) cudaStreamSynchronize(s->st_comp);
     if (s->st_copy) cudaStreamSynchronize(s->st_copy);
     if (s->st_d2h) cudaStreamSynchronize(s->st_d2h);
-    for (Slot &sl : s->slot) {
-        cudaFreeHost(sl.h_seq);
-        cudaFreeHost(sl.h_off);
-        cudaFreeHost(sl.h_res);
-        cudaFreeHost(sl.h_det);
-        cudaFree(sl.d_packed);
-        cudaFreeHost(sl.h_packed);
-        cudaFree(sl.d_win);
-        cudaFree(sl.d_win_off);
-        cudaFreeHost(sl.h_win_off);
-        cudaFree(sl.d_seq);
-        cudaFree(sl.d_off);
-        cudaFree(sl.d_res);
-        cudaFree(sl.d_det);
-        if (sl.ev_h2d) cudaEventDestroy(sl.ev_h2d);
-        if (sl.ev_kern) cudaEventDestroy(sl.ev_kern);
-        if (sl.ev_done) cudaEventDestroy(sl.ev_done);
-        if (sl.graph) cudaGraphExecDestroy(sl.graph);
-    }
-    cudaFree(s->sc.pass[0]);
-    cudaFree(s->sc.pass[1]);
-    cudaFree(s->sc.cand);
-    cudaFree(s->sc.cand_cnt);
-    cudaFree(s->sc.worklist);
-    cudaFree(s->sc.n_work);
-    cudaFree(s->sc.worklist2);
-    cudaFree(s->sc.n_work2);
-    cudaFree(s->sc.wl_win);
-    cudaFree(s->sc.wl_full);
-    cudaFree(s->sc.n_lit);
+    for (Slot &sl : s->slot) free_slot(sl);
+    free_scratch(s->sc);
     cudaFree(s->d_stats);
     cudaFree(s->d_ovf);
     cudaFree(s->d_n_ovf);
@@ -556,29 +555,43 @@ static int enqueue_batch(bdx_stream *s, Slot &sl)
     return bdx_enqueue_classify(s, sl.d_seq, sl.d_off, n, sl.d_res, det);
 }
 
-// h_seq: the batch's sequence bytes, or -- packed -- their 4-bit codes (packed.cu).  h_win_off set: h_seq holds the
-// batch's window bytes (or their codes) with these offsets, h_off those of the full reads (windows.cu).
-static int launch_slot(bdx_stream *s, Slot &sl, const uint8_t *h_seq, const int32_t *h_off, bool packed = false,
-                       const int32_t *h_win_off = nullptr)
+// ---- host batches: every bdx_submit* form and bdx_acquire / bdx_commit ----
+// A batch as the caller hands it over: seq holds the reads' bytes, or -- packed -- their 4-bit codes (packed.cu);
+// windowed, only the bytes (or codes) of the reads' search windows, at offsets win_off (windows.cu).  off: the
+// offsets of the full reads.  pinned: the buffers are page-locked and go to the device as they are; otherwise the
+// batch is first copied into the slot's pinned staging.
+struct BatchInput {
+    const uint8_t *seq;
+    const int32_t *off;
+    const int32_t *win_off;
+    bool windows, packed, pinned;
+};
+
+// bytes of the batch's input stream, the one that travels to the device
+static size_t sent_bytes(const BatchInput &in, int32_t n)
 {
-    CU(cudaSetDevice(s->device));
+    if (!n) return 0;
+    const size_t b = (size_t)(in.windows ? in.win_off[n] : in.off[n]);
+    return in.packed ? (b + 1) / 2 : b;
+}
+
+static int launch_slot(bdx_stream *s, Slot &sl, const BatchInput &in)
+{
     const int32_t n = sl.n;
-    const size_t bytes = n ? (size_t)h_off[n] : 0;
-    const bool windows = h_win_off != nullptr;
-    const size_t sent = !n ? 0 : windows ? (size_t)h_win_off[n] : bytes;     // bytes of the stream that travels
-    uint8_t *const d_in = packed ? sl.d_packed : windows ? sl.d_win : sl.d_seq;
+    const size_t bytes = n ? (size_t)in.off[n] : 0, sent = sent_bytes(in, n);
+    uint8_t *const d_in = in.packed ? sl.d_packed : in.windows ? sl.d_win : sl.d_seq;
     if (n) {
-        CU(cudaMemcpyAsync(sl.d_off, h_off, ((size_t)n + 1) * 4, cudaMemcpyHostToDevice, s->st_copy));
-        if (windows) CU(cudaMemcpyAsync(sl.d_win_off, h_win_off, ((size_t)n + 1) * 4, cudaMemcpyHostToDevice, s->st_copy));
-        if (sent) CU(cudaMemcpyAsync(d_in, h_seq, packed ? (sent + 1) / 2 : sent, cudaMemcpyHostToDevice, s->st_copy));
+        CU(cudaMemcpyAsync(sl.d_off, in.off, ((size_t)n + 1) * 4, cudaMemcpyHostToDevice, s->st_copy));
+        if (in.windows) CU(cudaMemcpyAsync(sl.d_win_off, in.win_off, ((size_t)n + 1) * 4, cudaMemcpyHostToDevice, s->st_copy));
+        if (sent) CU(cudaMemcpyAsync(d_in, in.seq, sent, cudaMemcpyHostToDevice, s->st_copy));
     }
     CU(cudaEventRecord(sl.ev_h2d, s->st_copy));
     CU(cudaStreamWaitEvent(s->st_comp, sl.ev_h2d, 0));
-    if (windows && bytes) {
-        CU(launch_expand_windows(d_in, packed, sl.d_win_off, sl.d_off, sl.d_seq, n, (long long)bytes, s->tab->P,
+    if (in.windows && bytes) {
+        CU(launch_expand_windows(d_in, in.packed, sl.d_win_off, sl.d_off, sl.d_seq, n, (long long)bytes, s->tab->P,
                                  s->cfg->rep_of, s->tab->sm_count, s->st_comp));
         s->launches++;
-    } else if (packed && bytes) {
+    } else if (in.packed && bytes) {
         CU(launch_unpack4(sl.d_packed, sl.d_seq, sl.d_off, n, (long long)bytes, s->cfg->rep_of, s->tab->sm_count, s->st_comp));
         s->launches++;
     }
@@ -599,71 +612,116 @@ static int launch_slot(bdx_stream *s, Slot &sl, const uint8_t *h_seq, const int3
     return BDX_OK;
 }
 
-// pinned input staging (only bdx_submit / bdx_acquire need it; bdx_submit_pinned does not)
-static int ensure_host_staging(bdx_stream *s)
+// The input buffers of every slot that a batch form needs beyond those each stream has, allocated lazily on the
+// form's first batch: the device copy of packed codes or of window bytes (packed windows expand from d_packed) and
+// the window offsets; staged (the caller's buffers are not pinned): the pinned host staging of each.
+static int ensure_input_buffers(bdx_stream *s, bool packed, bool windows, bool staged)
 {
-    if (s->host_staging) return BDX_OK;
-    CU(cudaSetDevice(s->device));
+    const size_t seq_cap = (size_t)std::max<int64_t>(s->max_bytes, 16), code_cap = seq_cap / 2 + 32;
+    const size_t off_cap = ((size_t)s->max_reads + 1) * 4;
     for (Slot &sl : s->slot) {
-        if (!sl.h_seq) CU(cudaHostAlloc(&sl.h_seq, (size_t)std::max<int64_t>(s->max_bytes, 16), cudaHostAllocDefault));
-        if (!sl.h_off) CU(cudaHostAlloc(&sl.h_off, ((size_t)s->max_reads + 1) * 4, cudaHostAllocDefault));
+        if (packed && !sl.d_packed) CU(cudaMalloc(&sl.d_packed, code_cap));
+        if (windows && !packed && !sl.d_win) CU(cudaMalloc(&sl.d_win, seq_cap));
+        if (windows && !sl.d_win_off) CU(cudaMalloc(&sl.d_win_off, off_cap));
+        if (!staged) continue;
+        if (packed && !sl.h_packed) CU(cudaHostAlloc(&sl.h_packed, code_cap, cudaHostAllocDefault));
+        if (!packed && !sl.h_seq) CU(cudaHostAlloc(&sl.h_seq, seq_cap, cudaHostAllocDefault));
+        if (!sl.h_off) CU(cudaHostAlloc(&sl.h_off, off_cap, cudaHostAllocDefault));
+        if (windows && !sl.h_win_off) CU(cudaHostAlloc(&sl.h_win_off, off_cap, cudaHostAllocDefault));
     }
-    s->host_staging = true;
+    return BDX_OK;
+}
+
+// Whether the stream can take a new batch now; `pending` is the refusal while a bdx_acquire awaits its bdx_commit.
+static int check_stream(const bdx_stream *s, const char *pending)
+{
+    if (s->max_reads <= 0) return fail(BDX_ERR_STATE, "stream has no staging (max_reads = 0)");
+    if (s->acquired) return fail(BDX_ERR_STATE, pending);
+    if (s->in_flight >= BDX_MAX_IN_FLIGHT) return fail(BDX_ERR_STATE, "BDX_MAX_IN_FLIGHT batches already in flight; call bdx_fetch");
     return BDX_OK;
 }
 
 // Validates a host batch before anything is enqueued: sizes against the stream's staging, offsets non-decreasing
 // (a decreasing pair would be a negative read length on the device).  One branch-free pass over the offsets also
 // yields the longest read, which tells the DemuxStats overflow list how much room the batch can need.
-static int check_batch(bdx_stream *s, const int32_t *offsets, int32_t n)
+static int check_batch(const bdx_stream *s, const int32_t *offsets, int32_t n, int32_t *max_len)
 {
     if (n < 0) return fail(BDX_ERR_INVALID, "negative n_reads");
     if (n > s->max_reads) return fail(BDX_ERR_TOO_LARGE, "batch exceeds max_reads of the stream");
     if (n && offsets[0] != 0) return fail(BDX_ERR_INVALID, "offsets[0] must be 0");
     if (n && (offsets[n] < 0 || (int64_t)offsets[n] > s->max_bytes))
         return fail(BDX_ERR_TOO_LARGE, "batch exceeds max_bytes of the stream");
-    int32_t min_len = 0, max_len = 0;
+    int32_t min_len = 0;
+    *max_len = 0;
     for (int32_t i = 0; i < n; i++) {
         const int32_t len = offsets[i + 1] - offsets[i];
         min_len = std::min(min_len, len);
-        max_len = std::max(max_len, len);
+        *max_len = std::max(*max_len, len);
     }
     if (min_len < 0) return fail(BDX_ERR_INVALID, "offsets must be non-decreasing");
-    return bdx_stats_reserve_overflow(s, n, max_len);
+    return BDX_OK;
+}
+
+// The device trusts win_off: every read's window length is checked against the rule here.
+static int check_windows(const bdx_stream *s, const BatchInput &in, int32_t n)
+{
+    if (n && in.win_off[0] != 0) return fail(BDX_ERR_INVALID, "win_offsets[0] must be 0");
+    int32_t last_n = -1, len = 0;
+    for (int32_t i = 0; i < n; i++) {
+        int sp[4];
+        if (in.off[i + 1] - in.off[i] != last_n) len = read_windows(s->tab->P, last_n = in.off[i + 1] - in.off[i], sp);
+        if (in.win_off[i + 1] - in.win_off[i] != len)
+            return fail(BDX_ERR_INVALID, "win_offsets do not match the search windows of the read lengths (first bad read: " +
+                                         std::to_string(i) + ")");
+    }
+    if (n && in.win_off[n] > 0 && !in.seq) return fail(BDX_ERR_INVALID, "null argument");
+    return BDX_OK;
+}
+
+// A batch from its validation on (bdx_commit starts here): checks, then DemuxStats overflow room -- so a refused
+// batch leaves the stream as it was -- then the form's buffers, the copy into pinned staging and the launch.
+static int stage_batch(bdx_stream *s, const BatchInput &in, int32_t n, uint64_t tag)
+{
+    int32_t max_len = 0;
+    int rc = check_batch(s, in.off, n, &max_len);
+    if (!rc && in.windows) rc = check_windows(s, in, n);
+    if (!rc) rc = bdx_stats_reserve_overflow(s, n, max_len);
+    if (rc) return rc;
+    s->acquired = false;            // a committed bdx_acquire: its staging now holds this batch
+    CU(cudaSetDevice(s->device));
+    if ((rc = ensure_input_buffers(s, in.packed, in.windows, !in.pinned))) return rc;
+    Slot &sl = s->slot[s->head];
+    sl.n = n;
+    sl.tag = tag;
+    if (in.pinned) return launch_slot(s, sl, in);
+    uint8_t *const h_in = in.packed ? sl.h_packed : sl.h_seq;
+    if (n) {
+        memcpy(sl.h_off, in.off, ((size_t)n + 1) * 4);
+        if (in.windows) memcpy(sl.h_win_off, in.win_off, ((size_t)n + 1) * 4);
+        if (const size_t b = sent_bytes(in, n)) memcpy(h_in, in.seq, b);
+    }
+    return launch_slot(s, sl, {h_in, sl.h_off, sl.h_win_off, in.windows, in.packed, true});
+}
+
+static const char kNoPackedInput[] = "more than 15 distinct barcode bytes: no 4-bit packed input for this config";
+
+static int submit_batch(bdx_stream *s, const BatchInput &in, int32_t n, uint64_t tag)
+{
+    if (!s || (n > 0 && (!in.off || (in.windows ? !in.win_off : !in.seq)))) return fail(BDX_ERR_INVALID, "null argument");
+    if (in.packed && !s->cfg->n_codes) return fail(BDX_ERR_INVALID, kNoPackedInput);
+    const int rc = check_stream(s, "bdx_acquire pending; call bdx_commit");
+    return rc ? rc : stage_batch(s, in, n, tag);
 }
 
 extern "C" int bdx_submit(bdx_stream *s, const uint8_t *seq, const int32_t *offsets, int32_t n, uint64_t tag)
 {
-    if (!s || (n > 0 && (!seq || !offsets))) return fail(BDX_ERR_INVALID, "null argument");
-    if (s->max_reads <= 0) return fail(BDX_ERR_STATE, "stream has no staging (max_reads = 0)");
-    if (s->acquired) return fail(BDX_ERR_STATE, "bdx_acquire pending; call bdx_commit");
-    if (s->in_flight >= BDX_MAX_IN_FLIGHT) return fail(BDX_ERR_STATE, "BDX_MAX_IN_FLIGHT batches already in flight; call bdx_fetch");
-    int rc = check_batch(s, offsets, n);
-    if (rc) return rc;
-    if ((rc = ensure_host_staging(s))) return rc;
-    Slot &sl = s->slot[s->head];
-    if (n) {
-        memcpy(sl.h_off, offsets, ((size_t)n + 1) * 4);
-        memcpy(sl.h_seq, seq, (size_t)offsets[n]);
-    }
-    sl.n = n;
-    sl.tag = tag;
-    return launch_slot(s, sl, sl.h_seq, sl.h_off);
+    return submit_batch(s, {seq, offsets, nullptr, false, false, false}, n, tag);
 }
 
 extern "C" int bdx_submit_pinned(bdx_stream *s, const uint8_t *seq, const int32_t *offsets, int32_t n,
                                  uint64_t tag)
 {
-    if (!s || (n > 0 && (!seq || !offsets))) return fail(BDX_ERR_INVALID, "null argument");
-    if (s->max_reads <= 0) return fail(BDX_ERR_STATE, "stream has no staging (max_reads = 0)");
-    if (s->acquired) return fail(BDX_ERR_STATE, "bdx_acquire pending; call bdx_commit");
-    if (s->in_flight >= BDX_MAX_IN_FLIGHT) return fail(BDX_ERR_STATE, "BDX_MAX_IN_FLIGHT batches already in flight; call bdx_fetch");
-    int rc = check_batch(s, offsets, n);
-    if (rc) return rc;
-    Slot &sl = s->slot[s->head];
-    sl.n = n;
-    sl.tag = tag;
-    return launch_slot(s, sl, seq, offsets);
+    return submit_batch(s, {seq, offsets, nullptr, false, false, true}, n, tag);
 }
 
 // ---- 4-bit packed input ----
@@ -672,7 +730,7 @@ void bdx_pack4_bytes(const uint8_t code[256], const uint8_t *in, int64_t n, uint
 extern "C" int bdx_config_code_table(const bdx_config *cfg, uint8_t table[256])
 {
     if (!cfg || !table) return fail(BDX_ERR_INVALID, "null argument");
-    if (!cfg->n_codes) return fail(BDX_ERR_INVALID, "more than 15 distinct barcode bytes: no 4-bit packed input for this config");
+    if (!cfg->n_codes) return fail(BDX_ERR_INVALID, kNoPackedInput);
     memcpy(table, cfg->code_of, 256);
     return cfg->n_codes;
 }
@@ -695,52 +753,19 @@ extern "C" int bdx_config_describe(const bdx_config *cfg, int pass, char *buf, i
 extern "C" int bdx_pack_reads4(const bdx_config *cfg, const uint8_t *seq, int64_t n_bytes, uint8_t *packed)
 {
     if (!cfg || n_bytes < 0 || (n_bytes > 0 && (!seq || !packed))) return fail(BDX_ERR_INVALID, "bad argument");
-    if (!cfg->n_codes) return fail(BDX_ERR_INVALID, "more than 15 distinct barcode bytes: no 4-bit packed input for this config");
+    if (!cfg->n_codes) return fail(BDX_ERR_INVALID, kNoPackedInput);
     bdx_pack4_bytes(cfg->code_of, seq, n_bytes, packed);
     return BDX_OK;
 }
 
-static int ensure_packed_buffers(bdx_stream *s, bool host)
-{
-    CU(cudaSetDevice(s->device));
-    const size_t cap = (size_t)std::max<int64_t>(s->max_bytes, 16) / 2 + 32;
-    for (Slot &sl : s->slot) {
-        if (!sl.d_packed) CU(cudaMalloc(&sl.d_packed, cap));
-        if (host && !sl.h_packed) CU(cudaHostAlloc(&sl.h_packed, cap, cudaHostAllocDefault));
-        if (host && !sl.h_off) CU(cudaHostAlloc(&sl.h_off, ((size_t)s->max_reads + 1) * 4, cudaHostAllocDefault));
-    }
-    return BDX_OK;
-}
-
-static int submit_packed(bdx_stream *s, const uint8_t *packed, const int32_t *offsets, int32_t n, uint64_t tag, bool pinned)
-{
-    if (!s || (n > 0 && (!packed || !offsets))) return fail(BDX_ERR_INVALID, "null argument");
-    if (!s->cfg->n_codes) return fail(BDX_ERR_INVALID, "more than 15 distinct barcode bytes: no 4-bit packed input for this config");
-    if (s->max_reads <= 0) return fail(BDX_ERR_STATE, "stream has no staging (max_reads = 0)");
-    if (s->acquired) return fail(BDX_ERR_STATE, "bdx_acquire pending; call bdx_commit");
-    if (s->in_flight >= BDX_MAX_IN_FLIGHT) return fail(BDX_ERR_STATE, "BDX_MAX_IN_FLIGHT batches already in flight; call bdx_fetch");
-    int rc = check_batch(s, offsets, n);
-    if (rc) return rc;
-    if ((rc = ensure_packed_buffers(s, !pinned))) return rc;
-    Slot &sl = s->slot[s->head];
-    sl.n = n;
-    sl.tag = tag;
-    if (pinned) return launch_slot(s, sl, packed, offsets, true);
-    if (n) {
-        memcpy(sl.h_off, offsets, ((size_t)n + 1) * 4);
-        memcpy(sl.h_packed, packed, ((size_t)offsets[n] + 1) / 2);
-    }
-    return launch_slot(s, sl, sl.h_packed, sl.h_off, true);
-}
-
 extern "C" int bdx_submit_packed4(bdx_stream *s, const uint8_t *packed, const int32_t *offsets, int32_t n, uint64_t tag)
 {
-    return submit_packed(s, packed, offsets, n, tag, false);
+    return submit_batch(s, {packed, offsets, nullptr, false, true, false}, n, tag);
 }
 
 extern "C" int bdx_submit_packed4_pinned(bdx_stream *s, const uint8_t *packed, const int32_t *offsets, int32_t n, uint64_t tag)
 {
-    return submit_packed(s, packed, offsets, n, tag, true);
+    return submit_batch(s, {packed, offsets, nullptr, false, true, true}, n, tag);
 }
 
 // ---- search-window input (windows.cu) ----
@@ -786,75 +811,25 @@ extern "C" int bdx_window_reads(const bdx_config *cfg, const uint8_t *seq, const
     return BDX_OK;
 }
 
-static int ensure_window_buffers(bdx_stream *s, bool packed, bool host)
-{
-    int rc = packed ? ensure_packed_buffers(s, host) : host ? ensure_host_staging(s) : BDX_OK;
-    if (rc) return rc;
-    CU(cudaSetDevice(s->device));
-    for (Slot &sl : s->slot) {
-        if (!packed && !sl.d_win) CU(cudaMalloc(&sl.d_win, (size_t)std::max<int64_t>(s->max_bytes, 16)));
-        if (!sl.d_win_off) CU(cudaMalloc(&sl.d_win_off, ((size_t)s->max_reads + 1) * 4));
-        if (host && !sl.h_win_off) CU(cudaHostAlloc(&sl.h_win_off, ((size_t)s->max_reads + 1) * 4, cudaHostAllocDefault));
-    }
-    return BDX_OK;
-}
-
-static int submit_windows(bdx_stream *s, const uint8_t *win, const int32_t *win_off, const int32_t *offsets, int32_t n,
-                          int packed, uint64_t tag, bool pinned)
-{
-    if (!s || (n > 0 && (!offsets || !win_off))) return fail(BDX_ERR_INVALID, "null argument");
-    if (packed && !s->cfg->n_codes) return fail(BDX_ERR_INVALID, "more than 15 distinct barcode bytes: no 4-bit packed input for this config");
-    if (s->max_reads <= 0) return fail(BDX_ERR_STATE, "stream has no staging (max_reads = 0)");
-    if (s->acquired) return fail(BDX_ERR_STATE, "bdx_acquire pending; call bdx_commit");
-    if (s->in_flight >= BDX_MAX_IN_FLIGHT) return fail(BDX_ERR_STATE, "BDX_MAX_IN_FLIGHT batches already in flight; call bdx_fetch");
-    int rc = check_batch(s, offsets, n);
-    if (rc) return rc;
-    // the device trusts win_off: every read's window length is checked against the rule here
-    if (n && win_off[0] != 0) return fail(BDX_ERR_INVALID, "win_offsets[0] must be 0");
-    const DevParams &P = s->tab->P;
-    int32_t last_n = -1, len = 0;
-    for (int32_t i = 0; i < n; i++) {
-        int sp[4];
-        if (offsets[i + 1] - offsets[i] != last_n) len = read_windows(P, last_n = offsets[i + 1] - offsets[i], sp);
-        if (win_off[i + 1] - win_off[i] != len)
-            return fail(BDX_ERR_INVALID, "win_offsets do not match the search windows of the read lengths (first bad read: " +
-                                         std::to_string(i) + ")");
-    }
-    if (n && win_off[n] > 0 && !win) return fail(BDX_ERR_INVALID, "null argument");
-    if ((rc = ensure_window_buffers(s, packed != 0, !pinned))) return rc;
-    Slot &sl = s->slot[s->head];
-    sl.n = n;
-    sl.tag = tag;
-    if (pinned) return launch_slot(s, sl, win, offsets, packed != 0, win_off);
-    uint8_t *const h_in = packed ? sl.h_packed : sl.h_seq;
-    if (n) {
-        memcpy(sl.h_off, offsets, ((size_t)n + 1) * 4);
-        memcpy(sl.h_win_off, win_off, ((size_t)n + 1) * 4);
-        if (win_off[n]) memcpy(h_in, win, packed ? ((size_t)win_off[n] + 1) / 2 : (size_t)win_off[n]);
-    }
-    return launch_slot(s, sl, h_in, sl.h_off, packed != 0, sl.h_win_off);
-}
-
 extern "C" int bdx_submit_windows(bdx_stream *s, const uint8_t *win, const int32_t *win_offsets, const int32_t *offsets,
                                   int32_t n_reads, int packed4, uint64_t tag)
 {
-    return submit_windows(s, win, win_offsets, offsets, n_reads, packed4, tag, false);
+    return submit_batch(s, {win, offsets, win_offsets, true, packed4 != 0, false}, n_reads, tag);
 }
 
 extern "C" int bdx_submit_windows_pinned(bdx_stream *s, const uint8_t *win, const int32_t *win_offsets,
                                          const int32_t *offsets, int32_t n_reads, int packed4, uint64_t tag)
 {
-    return submit_windows(s, win, win_offsets, offsets, n_reads, packed4, tag, true);
+    return submit_batch(s, {win, offsets, win_offsets, true, packed4 != 0, true}, n_reads, tag);
 }
 
 extern "C" int bdx_acquire(bdx_stream *s, uint8_t **seq, int32_t **offsets)
 {
     if (!s || !seq || !offsets) return fail(BDX_ERR_INVALID, "null argument");
-    if (s->max_reads <= 0) return fail(BDX_ERR_STATE, "stream has no staging (max_reads = 0)");
-    if (s->acquired) return fail(BDX_ERR_STATE, "already acquired");
-    if (s->in_flight >= BDX_MAX_IN_FLIGHT) return fail(BDX_ERR_STATE, "BDX_MAX_IN_FLIGHT batches already in flight; call bdx_fetch");
-    int rc = ensure_host_staging(s);
+    int rc = check_stream(s, "already acquired");
     if (rc) return rc;
+    CU(cudaSetDevice(s->device));
+    if ((rc = ensure_input_buffers(s, false, false, true))) return rc;
     Slot &sl = s->slot[s->head];
     *seq = sl.h_seq;
     *offsets = sl.h_off;
@@ -866,13 +841,23 @@ extern "C" int bdx_commit(bdx_stream *s, int32_t n, uint64_t tag)
 {
     if (!s) return fail(BDX_ERR_INVALID, "null stream");
     if (!s->acquired) return fail(BDX_ERR_STATE, "bdx_commit without bdx_acquire");
-    Slot &sl = s->slot[s->head];
-    int rc = check_batch(s, sl.h_off, n);
-    if (rc) return rc;
-    s->acquired = false;
-    sl.n = n;
-    sl.tag = tag;
-    return launch_slot(s, sl, sl.h_seq, sl.h_off);
+    const Slot &sl = s->slot[s->head];
+    return stage_batch(s, {sl.h_seq, sl.h_off, nullptr, false, false, true}, n, tag);
+}
+
+// Waits for the oldest batch in flight and takes it off the ring; its results stay in the slot's pinned staging
+// until a later submit reuses the slot.
+static int pop_oldest(bdx_stream *s, uint64_t *tag, int32_t *n_reads, Slot *&out)
+{
+    Slot &sl = s->slot[s->tail];
+    CU(cudaEventSynchronize(sl.ev_done));
+    if (tag) *tag = sl.tag;
+    if (n_reads) *n_reads = sl.n;
+    sl.busy = false;
+    s->tail = (s->tail + 1) % BDX_MAX_IN_FLIGHT;
+    s->in_flight--;
+    out = &sl;
+    return BDX_OK;
 }
 
 extern "C" int bdx_fetch(bdx_stream *s, uint64_t *tag, int32_t *n_reads, bdx_result *results,
@@ -881,15 +866,10 @@ extern "C" int bdx_fetch(bdx_stream *s, uint64_t *tag, int32_t *n_reads, bdx_res
     if (!s) return fail(BDX_ERR_INVALID, "null stream");
     if (s->in_flight == 0) return fail(BDX_ERR_STATE, "nothing in flight");
     if (details && !s->details) return fail(BDX_ERR_STATE, "details not enabled on this stream");
-    Slot &sl = s->slot[s->tail];
-    CU(cudaEventSynchronize(sl.ev_done));
-    if (tag) *tag = sl.tag;
-    if (n_reads) *n_reads = sl.n;
-    if (results && sl.n) memcpy(results, sl.h_res, (size_t)sl.n * sizeof(bdx_result));
-    if (details && sl.n) memcpy(details, sl.h_det, (size_t)sl.n * 2 * sizeof(bdx_pass_detail));
-    sl.busy = false;
-    s->tail = (s->tail + 1) % BDX_MAX_IN_FLIGHT;
-    s->in_flight--;
+    Slot *sl = nullptr;
+    if (int rc = pop_oldest(s, tag, n_reads, sl)) return rc;
+    if (results && sl->n) memcpy(results, sl->h_res, (size_t)sl->n * sizeof(bdx_result));
+    if (details && sl->n) memcpy(details, sl->h_det, (size_t)sl->n * 2 * sizeof(bdx_pass_detail));
     return BDX_OK;
 }
 
@@ -900,15 +880,10 @@ extern "C" int bdx_fetch_view(bdx_stream *s, uint64_t *tag, int32_t *n_reads, co
 {
     if (!s) return fail(BDX_ERR_INVALID, "null stream");
     if (s->in_flight == 0) return fail(BDX_ERR_STATE, "nothing in flight");
-    Slot &sl = s->slot[s->tail];
-    CU(cudaEventSynchronize(sl.ev_done));
-    if (tag) *tag = sl.tag;
-    if (n_reads) *n_reads = sl.n;
-    if (results) *results = sl.h_res;
-    if (details) *details = s->details ? sl.h_det : nullptr;
-    sl.busy = false;
-    s->tail = (s->tail + 1) % BDX_MAX_IN_FLIGHT;
-    s->in_flight--;
+    Slot *sl = nullptr;
+    if (int rc = pop_oldest(s, tag, n_reads, sl)) return rc;
+    if (results) *results = sl->h_res;
+    if (details) *details = s->details ? sl->h_det : nullptr;
     return BDX_OK;
 }
 
@@ -979,28 +954,33 @@ extern "C" int bdx_stream_profile_read(bdx_stream *s, double *filter_ms, int32_t
     return BDX_OK;
 }
 
+// the 12 counters of bdx_stream::d_counters once the compute stream has drained; reset: zero them afterwards
+static int read_counters(bdx_stream *s, unsigned long long (&h)[12], int reset)
+{
+    CU(cudaSetDevice(s->device));
+    CU(cudaStreamSynchronize(s->st_comp));
+    CU(cudaMemcpy(h, s->d_counters, sizeof(h), cudaMemcpyDeviceToHost));
+    if (reset) CU(cudaMemset(s->d_counters, 0, sizeof(h)));
+    return BDX_OK;
+}
+
 extern "C" int bdx_stream_path_counters(bdx_stream *s, int64_t *prefilter_reads, int64_t *seed_reads,
                                         int64_t *automaton_reads, int reset)
 {
     if (!s) return fail(BDX_ERR_INVALID, "null stream");
-    CU(cudaSetDevice(s->device));
-    CU(cudaStreamSynchronize(s->st_comp));
     unsigned long long h[12];
-    CU(cudaMemcpy(h, s->d_counters, sizeof(h), cudaMemcpyDeviceToHost));
+    if (int rc = read_counters(s, h, reset)) return rc;
     if (prefilter_reads) *prefilter_reads = (int64_t)h[0];
     if (seed_reads) *seed_reads = (int64_t)h[2];
     if (automaton_reads) *automaton_reads = (int64_t)h[1];
-    if (reset) CU(cudaMemset(s->d_counters, 0, sizeof(h)));
     return BDX_OK;
 }
 
 extern "C" int bdx_stream_work_counters(bdx_stream *s, int64_t out[12], int reset)
 {
     if (!s || !out) return fail(BDX_ERR_INVALID, "null argument");
-    CU(cudaSetDevice(s->device));
-    CU(cudaStreamSynchronize(s->st_comp));
     unsigned long long h[12];
-    CU(cudaMemcpy(h, s->d_counters, sizeof(h), cudaMemcpyDeviceToHost));
+    if (int rc = read_counters(s, h, reset)) return rc;
     out[0] = (int64_t)h[0];
     out[1] = (int64_t)h[2];
     out[2] = (int64_t)h[1];
@@ -1008,7 +988,6 @@ extern "C" int bdx_stream_work_counters(bdx_stream *s, int64_t out[12], int rese
     out[4] = (int64_t)h[4];
     for (int k = 5; k < 9; k++) out[k] = (int64_t)h[k];
     out[9] = out[10] = out[11] = 0;
-    if (reset) CU(cudaMemset(s->d_counters, 0, sizeof(h)));
     return BDX_OK;
 }
 

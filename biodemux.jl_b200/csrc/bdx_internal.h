@@ -197,6 +197,9 @@ struct Scratch {
 // current device; raises the kernel's dynamic shared-memory limit on first use.  Cached per (device, kernel,
 // threads, smem): the two runtime queries cost microseconds each, which adds up for 4000-read batches.
 cudaError_t blocks_per_sm_cached(const void *kern, int threads, size_t smem, int *per_sm);
+// Grid of `kern` for `groups` units of work (blocks' worth of reads): as many blocks as are resident on the device's
+// `sm_count` SMs at once, fewer when there is less work, at least one.  Blocks loop over the groups past the grid.
+cudaError_t resident_grid(const void *kern, int threads, size_t smem, long long groups, int sm_count, int *blocks);
 
 // dynamic shared memory of each kernel's launch, from its file's layout arithmetic (the pass plan, plan.cu, holds
 // them against its budgets)

@@ -689,11 +689,9 @@ cudaError_t launch_prefilter(const DevParams &P, int pass, const uint8_t *seq, c
     const DevSet &S = P.set[pass];
     const size_t smem = prefilter_smem_bytes(S);
     auto kern = P.algo == BDX_EXACT ? k_prefilter<1> : (P.algo == BDX_HAMMING ? k_prefilter<2> : k_prefilter<0>);
-    int per_sm = 0;
-    cudaError_t e = blocks_per_sm_cached((const void *)kern, kPfThreads, smem, &per_sm);
+    int blocks = 0;
+    cudaError_t e = resident_grid((const void *)kern, kPfThreads, smem, (n + kPfThreads - 1) / kPfThreads, sm_count, &blocks);
     if (e != cudaSuccess) return e;
-    const int groups = (n + kPfThreads - 1) / kPfThreads;
-    const int blocks = std::min(groups, sm_count * per_sm);
     e = cudaMemsetAsync(sc.n_work, 0, sizeof(int), st);
     if (e != cudaSuccess) return e;
     kern<<<blocks, kPfThreads, smem, st>>>(P, pass, seq, off, n, sc.pass[pass], sc.pass[0], sc.worklist, sc.n_work,
@@ -717,16 +715,13 @@ static cudaError_t launch_wgv(const DevParams &P, int pass, const uint8_t *seq, 
 {
     const size_t smem = filter_smem_bytes(P.set[pass]);
     auto kern = k_filter<W, G, CODING, PAIR>;
-    int per_sm = 0;
-    cudaError_t e = blocks_per_sm_cached((const void *)kern, kFilterWarps * 32, smem, &per_sm);
-    if (e != cudaSuccess) return e;
     // persistent grid: a whole number of resident blocks per SM, capped by the work
-    long long blocks = (long long)sm_count * per_sm;
-    const long long need = ((long long)n + kFilterWarps - 1) / kFilterWarps;
-    if (blocks > need) blocks = need;
-    if (blocks < 1) blocks = 1;
-    kern<<<(unsigned)blocks, kFilterWarps * 32, smem, st>>>(P, pass, seq, off, n, sc.pass[pass], sc.pass[0],
-                                                            sc.cand, sc.cand_cnt, counters, wl, n_wl, sc.wl_full, sc.n_lit + 1);
+    int blocks = 0;
+    const cudaError_t e = resident_grid((const void *)kern, kFilterWarps * 32, smem,
+                                        ((long long)n + kFilterWarps - 1) / kFilterWarps, sm_count, &blocks);
+    if (e != cudaSuccess) return e;
+    kern<<<blocks, kFilterWarps * 32, smem, st>>>(P, pass, seq, off, n, sc.pass[pass], sc.pass[0],
+                                                  sc.cand, sc.cand_cnt, counters, wl, n_wl, sc.wl_full, sc.n_lit + 1);
     return cudaGetLastError();
 }
 

@@ -211,11 +211,10 @@ cudaError_t launch_hamming_scan(const DevParams &P, int pass, const uint8_t *seq
 {
     const DevSet &S = P.set[pass];
     const size_t smem = hamming_scan_smem(S);
-    int per_sm = 0;
-    cudaError_t e = blocks_per_sm_cached((const void *)k_hamming_scan, kHpThreads, smem, &per_sm);
+    int blocks = 0;
+    cudaError_t e = resident_grid((const void *)k_hamming_scan, kHpThreads, smem, (n + kHpThreads - 1) / kHpThreads,
+                                  sm_count, &blocks);
     if (e != cudaSuccess) return e;
-    const int groups = (n + kHpThreads - 1) / kHpThreads;
-    const int blocks = std::max(1, std::min(groups, sm_count * per_sm));
     k_hamming_scan<<<blocks, kHpThreads, smem, st>>>(P, pass, seq, off, n, sc.pass[pass], sc.pass[0], sc.cand, sc.cand_cnt);
     return cudaGetLastError();
 }

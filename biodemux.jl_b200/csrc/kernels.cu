@@ -51,6 +51,15 @@ cudaError_t blocks_per_sm_cached(const void *kern, int threads, size_t smem, int
     return cudaSuccess;
 }
 
+cudaError_t resident_grid(const void *kern, int threads, size_t smem, long long groups, int sm_count, int *blocks)
+{
+    int per_sm = 0;
+    const cudaError_t e = blocks_per_sm_cached(kern, threads, smem, &per_sm);
+    if (e != cudaSuccess) return e;
+    *blocks = (int)std::max<long long>(1, std::min<long long>(groups, (long long)sm_count * per_sm));
+    return cudaSuccess;
+}
+
 // ---------------------------------------------------------------------------
 // k_literal: one thread per read walks barcodes in file order under the running
 // threshold -- the body of find_best_matching_bc (classification.jl:632-728)

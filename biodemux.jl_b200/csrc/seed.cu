@@ -366,11 +366,10 @@ cudaError_t launch_seed(const DevParams &P, int pass, int level, const uint8_t *
     const bool tab = seed_tab_in_smem(S, L);
     const size_t smem = seed_smem(S, L, tab);
     auto kern = S.words == 1 ? (tab ? k_seed<true, 1> : k_seed<false, 1>) : (tab ? k_seed<true, 2> : k_seed<false, 2>);
-    int per_sm = 0;
-    cudaError_t e = blocks_per_sm_cached((const void *)kern, kSeedThreads, smem, &per_sm);
+    int blocks = 0;     // groups of n reads: an upper bound, the worklist is <= n
+    cudaError_t e = resident_grid((const void *)kern, kSeedThreads, smem, (n + kSeedThreads - 1) / kSeedThreads, sm_count,
+                                  &blocks);
     if (e != cudaSuccess) return e;
-    const int groups = (n + kSeedThreads - 1) / kSeedThreads;     // upper bound: the worklist is <= n
-    const int blocks = std::max(1, std::min(groups, sm_count * per_sm));
     e = cudaMemsetAsync(n_out, 0, sizeof(int), st);
     if (e != cudaSuccess) return e;
     kern<<<blocks, kSeedThreads, smem, st>>>(P, pass, level, seq, off, n, sc.pass[pass], sc.pass[0], wl_in, n_in, wl_out, n_out,

@@ -278,11 +278,10 @@ cudaError_t launch_seed_deep(const DevParams &P, int pass, const uint8_t *seq, c
     const DevSet &S = P.set[pass];
     const size_t smem = deep_smem(S);
     auto kern = S.words == 1 ? k_seed_deep<1> : k_seed_deep<2>;
-    int per_sm = 0;
-    cudaError_t e = blocks_per_sm_cached((const void *)kern, kSeedThreads, smem, &per_sm);
+    int blocks = 0;
+    cudaError_t e = resident_grid((const void *)kern, kSeedThreads, smem, (n + kSeedThreads - 1) / kSeedThreads, sm_count,
+                                  &blocks);
     if (e != cudaSuccess) return e;
-    const int groups = (n + kSeedThreads - 1) / kSeedThreads;
-    const int blocks = std::max(1, std::min(groups, sm_count * per_sm));
     e = cudaMemsetAsync(n_out, 0, sizeof(int), st);
     if (e != cudaSuccess) return e;
     kern<<<blocks, kSeedThreads, smem, st>>>(P, pass, seq, off, sc.pass[pass], sc.pass[0], wl_in, n_in, wl_out, n_out, counters,

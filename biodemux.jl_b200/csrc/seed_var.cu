@@ -734,11 +734,10 @@ cudaError_t launch_seed_var(const DevParams &P, int pass, int level, const uint8
     const SeedVar &V = S.sv[level];
     const SvLaunch L = sv_launch_params(S, V);
     auto kern = S.words == 1 ? k_seed_var<1> : k_seed_var<2>;
-    int per_sm = 0;
-    cudaError_t e = blocks_per_sm_cached((const void *)kern, kSvThreads, L.smem, &per_sm);
+    int blocks = 0;
+    cudaError_t e = resident_grid((const void *)kern, kSvThreads, L.smem, (n + V.group_reads - 1) / V.group_reads,
+                                  sm_count, &blocks);
     if (e != cudaSuccess) return e;
-    const int groups = (n + V.group_reads - 1) / V.group_reads;
-    const int blocks = std::max(1, std::min(groups, sm_count * per_sm));
     e = cudaMemsetAsync(n_out, 0, sizeof(int), st);
     if (e != cudaSuccess) return e;
     kern<<<blocks, kSvThreads, L.smem, st>>>(P, pass, level, seq, off, n, sc.pass[pass], sc.pass[0], wl_in, n_in, wl_out, n_out,
